@@ -2,6 +2,7 @@
 """bench.py — k-mer recruitment read-bases/s on B200 (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cenx|cen6|stream] [--scale S]
+                    [--dump-outputs DIR]
 
 Workloads (config.workload), all drawn from genomes made by the reference's own simulate_tandem_repeat.py
 (tests/golden/genomes/, oracle/make_genomes.py) with reads from centroflye_b200.synth:
@@ -23,6 +24,11 @@ Workloads (config.workload), all drawn from genomes made by the reference's own 
 `value` times a step with inputs resident in HBM; `e2e` times the same call from pinned host buffers (H2D inside) to
 host-resident results (D2H inside); `e2e_cli` is the drop-in command line from a report file on disk to the two output
 files.  --scale shrinks the array multiplicity (parity / smoke use); 1.0 is the configuration the metric is quoted on.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned (cenx / cen6: rare k-mers, clouds,
+edges, recruited k-mers, counters; stream: the rare k-mers and count table of the last batch) in a canonical order as
+float64 .npy files, arrays beyond 12 MB as a fixed, seeded sample of their rows (DIR/manifest.json says which).  The
+inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import contextlib
@@ -274,6 +280,41 @@ def sum_over_ranks(xs, world, device):
     return [int(x) for x in t.tolist()]
 
 
+# ---- --dump-outputs: what the timed path returned in its last step, for output-by-output comparison of two builds ----
+DUMP_BYTES_PER_ARRAY = 12 << 20  # five arrays of that size at most per run, so a dump stays under 64 MB
+DUMP_SEED = 20261020
+
+
+def sorted_rows(a):
+    """Rows of a 2-D integer array in lexicographic order (the device returns edges and table slots unordered)."""
+    return a[np.lexsort(a.T[::-1])] if a.shape[0] else a
+
+
+def dump_outputs(dirname, arrays, rank=0, world=1):
+    """arrays: name -> integer numpy array in a canonical order.  Written as float64 (exact for the integers here:
+    2-bit k-mer codes of k <= 26, ids, counts), each one cut to DUMP_BYTES_PER_ARRAY by a fixed, seeded choice of rows
+    that depends only on the number of rows, so equal outputs give equal files.  manifest.json records the full shapes
+    and which rows were kept.  At several ranks every rank writes its own shard as <name>_rank<r>.npy."""
+    os.makedirs(dirname, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    manifest = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        out = a.astype(np.float64)
+        row_bytes = max(out[:1].nbytes, 8)
+        entry = {"shape": list(a.shape), "source_dtype": str(a.dtype), "rows": "all"}
+        if out.nbytes > DUMP_BYTES_PER_ARRAY:
+            keep = DUMP_BYTES_PER_ARRAY // row_bytes
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(a.shape[0], size=keep, replace=False))
+            out = out[rows]
+            entry["rows"] = (f"{keep} of {a.shape[0]}: np.sort(np.random.default_rng({DUMP_SEED}).choice({a.shape[0]}, "
+                             f"size={keep}, replace=False))")
+        np.save(os.path.join(dirname, f"{name}{suffix}.npy"), out)
+        manifest[name] = entry
+    with open(os.path.join(dirname, f"manifest{suffix}.json"), "w") as f:
+        json.dump(manifest, f, indent=1)
+
+
 # ---- parity leg: a down-scaled instance of the same kind at THIS world size against the C oracle ------------------
 def parity_check(eng, world, rank, config):
     """Sharded (or single-GPU) recruitment on a ~1-Mbase instance == oracle/c on the whole read set: rare set, clouds
@@ -408,6 +449,16 @@ def run_recruit(args):
                 stage_ms.setdefault(name, []).append(ms)
             eng.events = None
     launches = (eng.launch_count() - launches0) / max(args.steps, 1)
+    if args.dump_outputs:
+        index, csr, dres = res
+        dump_outputs(args.dump_outputs, {
+            "rare_kmers": index.sorted_keys.cpu().numpy().view(np.uint64),
+            "cloud_unit_ptr": csr.unit_ptr.cpu().numpy()[: csr.n_units + 1],
+            "cloud_ids": csr.ids.cpu().numpy()[: csr.n_entries].view(np.uint32),
+            "edges": sorted_rows(dres.edges.cpu().numpy().view(np.uint32).reshape(-1, 4)),
+            "unique_kmers": np.sort(dres.selected.cpu().numpy().view(np.uint32)),
+            "counts": np.array([dres.n_increments, dres.n_candidates, dres.n_pair_candidates], dtype=np.int64)},
+            rank, world)
     ms = max_over_ranks(float(np.mean(step_ms)), world, eng.device)
     last = res[2]
     n_edges_total, = sum_over_ranks([int(last.edges.shape[0])], world, eng.device)
@@ -640,7 +691,7 @@ def run_stream(args):
             prev = h
             bases += batch.n_bases
             kmers += int(batch.n_bases - batch.n_reads * (k - 1))
-        eng.docfreq_stream_finish(prev)
+        last = eng.docfreq_stream_finish(prev)
         b.record()
         barrier()
         step_ms = [a.elapsed_time(b) / max(args.steps, 1)] * args.steps
@@ -650,6 +701,14 @@ def run_stream(args):
         if getattr(eng, "stream_fallbacks", 0):
             raise SystemExit("stage A fell back to the single-kernel form inside the timed region")
     launches = (eng.launch_count() - launches0) / max(args.steps, 1)
+    if args.dump_outputs:  # the last batch's rare keys and its whole count table (key, n_reads, n_multi)
+        rare, table = last
+        keys, n_reads, n_multi = (x.cpu().numpy().view(np.uint32 if x.element_size() == 4 else np.uint64)
+                                  for x in eng.table_select(table, 0, 0xFFFFFFFF, 0xFFFFFFFF, with_counts=True))
+        dump_outputs(args.dump_outputs, {
+            "rare_kmers": np.sort(rare.cpu().numpy().view(np.uint64)),
+            "count_table": sorted_rows(np.stack([keys, n_reads.astype(np.uint64), n_multi.astype(np.uint64)], axis=1))},
+            rank, world)
     # end to end: the batch's packed reads from pinned host memory, the rare keys and the table's size back
     e2e_ms, h2d, d2h = [], 0, 0
     for i in range(1 + max(2, min(args.steps, 3))):
@@ -768,7 +827,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-check", dest="check", action="store_false", help="skip the parity leg")
     ap.add_argument("--stream-batches", type=int, default=2, help="distinct batches per GPU kept resident (stream)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path returns: use it with --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,14 +1,5 @@
-"""Helper of test_read_module.py: the public names of the drop-in read_kmer_cloud module and, where /root/reference
-exists, of the reference module (imported with oracle/bio_shim standing in for Biopython)."""
+"""Helper of test_read_module.py: the names the drop-in read_kmer_cloud module binds, with its public ones."""
 import importlib
-import importlib.util
-import os
-import sys
-import warnings
-
-from conftest import ROOT
-
-REF = "/root/reference/scripts"
 
 
 def _public(mod):
@@ -20,20 +11,4 @@ def load_names():
     ours_mod = importlib.import_module("centroflye_b200.read_kmer_cloud")
     ours = {n: getattr(ours_mod, n) for n in vars(ours_mod)}
     ours["__public__"] = _public(ours_mod)
-    ref = None
-    if os.path.exists(os.path.join(REF, "read_kmer_cloud.py")):
-        saved = list(sys.path)
-        sys.path[:0] = [os.path.join(ROOT, "oracle", "bio_shim"), REF]
-        try:
-            with warnings.catch_warnings():
-                warnings.simplefilter("ignore")
-                spec = importlib.util.spec_from_file_location("reference_read_kmer_cloud", os.path.join(REF, "read_kmer_cloud.py"))
-                mod = importlib.util.module_from_spec(spec)
-                spec.loader.exec_module(mod)
-            ref = {n: getattr(mod, n) for n in vars(mod)}
-            ref["__public__"] = _public(mod)
-        finally:
-            sys.path[:] = saved
-            for name in ("ncrf_parser", "utils", "utils.bio", "utils.os_utils"):
-                sys.modules.pop(name, None)
-    return ours, ref
+    return ours

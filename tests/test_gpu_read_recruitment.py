@@ -1,21 +1,25 @@
 """Row f rank 4, second half: the read recruitment pre-filter (scripts/read_recruitment/rr.cpp) on the device.
 
-* against the REFERENCE BINARY itself -- oracle/_ref/rr, compiled by oracle/build_rr_ref.sh from rr.cpp and the edlib /
-  kseq sources vendored in the reference tree, with the reference's own flags: same command line, byte-identical output
-  file, for several thresholds, FASTA / FASTQ / gzip input;
+* against the output file the REFERENCE BINARY writes for the same command line -- rr.cpp's rule on exact infix edit
+  distances, stored as kept read names, size and SHA-256 in tests/golden/rr/outputs.json by oracle/make_rr_golden.py,
+  which also checks it against the binary when given one: byte-identical output file, for several thresholds,
+  FASTA / FASTQ / gzip input;
 * exact infix edit distances on both strands against a plain dynamic-programming restatement of edlib's HW mode, for
   unit lengths on every side of the 64-bit word boundaries and of the kernel's template sizes (incl. DXZ1 and D6Z1)."""
 import gzip
+import hashlib
+import json
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
-from conftest import ROOT
+from conftest import GOLDEN
 
 pytestmark = pytest.mark.gpu
-RR_REF = os.path.join(ROOT, "oracle", "_ref", "rr")
+RR_GOLDEN = os.path.join(GOLDEN, "rr", "outputs.json")
+FORMATS = ["fasta", "fastq", "fasta.gz"]
+THRESHOLDS = (0, 100, 350, 700, -1)
 
 
 def _rnd(rng, n):
@@ -62,15 +66,13 @@ def _read_set(rng, unit):
     return reads
 
 
-@pytest.mark.parametrize("fmt", ["fasta", "fastq", "fasta.gz"])
-def test_rr_output_equals_reference_binary(tmp_path, fmt):
-    if not os.path.exists(RR_REF):
-        pytest.skip("oracle/_ref/rr is not built (bash oracle/build_rr_ref.sh in the build container)")
-    from centroflye_b200 import read_recruitment as rr, synth
+def write_inputs(tmp_dir, fmt):
+    """The unit (DXZ1) and the seeded read set of one input format as files -> (unit_fn, read_fn, reads, read text)."""
+    from centroflye_b200 import synth
     rng = np.random.default_rng({"fasta": 1, "fastq": 2, "fasta.gz": 3}[fmt])
     unit = synth.load_genome("cenx_dxz1_m1500_s1")[3]
     reads = _read_set(rng, unit)
-    unit_fn, read_fn = str(tmp_path / "unit.fasta"), str(tmp_path / ("reads." + fmt))
+    unit_fn, read_fn = os.path.join(tmp_dir, "unit.fasta"), os.path.join(tmp_dir, "reads." + fmt)
     with open(unit_fn, "w") as f:
         f.write(">DXZ1 rc\n" + "\n".join(unit[i:i + 70] for i in range(0, len(unit), 70)) + "\n")
     if fmt == "fastq":
@@ -83,14 +85,26 @@ def test_rr_output_equals_reference_binary(tmp_path, fmt):
     else:
         with open(read_fn, "w") as f:
             f.write(text)
+    return unit_fn, read_fn, reads, text
+
+
+@pytest.mark.parametrize("fmt", FORMATS)
+def test_rr_output_equals_reference_binary(tmp_path, fmt):
+    from centroflye_b200 import read_recruitment as rr
+    with open(RR_GOLDEN) as f:
+        golden = json.load(f)[fmt]
+    unit_fn, read_fn, reads, text = write_inputs(str(tmp_path), fmt)
+    assert hashlib.sha256(text.encode()).hexdigest() == golden["reads_sha256"], \
+        "the seeded read set is not the one the golden outputs were made from"
     kept_counts = []
-    for threshold in (0, 100, 350, 700, -1):
-        want_fn, got_fn = str(tmp_path / f"want{threshold}.fasta"), str(tmp_path / f"got{threshold}.fasta")
-        subprocess.check_call([RR_REF, unit_fn, read_fn, want_fn, str(threshold)])
+    for threshold in THRESHOLDS:
+        want = golden["outputs"][str(threshold)]
+        got_fn = str(tmp_path / f"got{threshold}.fasta")
         assert rr.main([unit_fn, read_fn, got_fn, str(threshold)]) == 0
-        want, got = open(want_fn, "rb").read(), open(got_fn, "rb").read()
-        assert got == want
-        kept_counts.append(want.count(b">"))
+        got = open(got_fn, "rb").read()
+        assert [ln[1:].decode() for ln in got.split(b"\n") if ln.startswith(b">")] == want["kept"]
+        assert len(got) == want["bytes"] and hashlib.sha256(got).hexdigest() == want["sha256"]
+        kept_counts.append(len(want["kept"]))
     assert kept_counts[0] >= 2 and kept_counts[0] < kept_counts[2] < kept_counts[4] == len(reads)
 
 

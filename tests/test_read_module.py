@@ -1,14 +1,13 @@
 """scripts/read.py (SURVEY.md §8 a10) and the never-called get_all_kmers of scripts/read_kmer_cloud.py:57-63: the
-drop-in modules against known answers worked out from the reference's source -- and, in the build container where
-/root/reference exists, against the reference classes themselves."""
-import importlib.util
+drop-in modules against known answers worked out from the reference's source, and against what the reference classes
+and module answered (tests/golden/reference_modules.json)."""
+import json
 import os
 
 import pytest
 
-from conftest import ROOT  # noqa: F401
+from conftest import GOLDEN
 
-REF = "/root/reference/scripts"
 SIMLORD_ID = "Read_17_length=8742bp_startpos=104652_chromosome=chrX_strand=+_numberOfErrors=1205_totalErrorProb=0.1378_passes=3.0_passesLeft=3_passesRight=2_cutPosition=4027_mult=1.5"
 
 
@@ -18,13 +17,8 @@ def _ours():
 
 
 def _reference():
-    path = os.path.join(REF, "read.py")
-    if not os.path.exists(path):
-        return None
-    spec = importlib.util.spec_from_file_location("reference_read", path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod.Read
+    with open(os.path.join(GOLDEN, "reference_modules.json")) as f:
+        return json.load(f)
 
 
 def test_read_plain():
@@ -55,26 +49,23 @@ def test_read_from_biopy():
 
 
 def test_read_equals_reference_class():
-    ref = _reference()
-    if ref is None:
-        pytest.skip("/root/reference is not on this box")
-    for args in (("r1", "ACGTACGT", False), (SIMLORD_ID, "ACGT", True), ("r2", None, False)):
-        a, b = _ours()(*args), ref(*args)
-        assert vars(a) == vars(b)
-        if args[1] is not None:
-            assert len(a) == len(b) and a[1:3] == b[1:3]
+    cases = _reference()["read"]
+    assert [tuple(c["args"]) for c in cases] == [("r1", "ACGTACGT", False), (SIMLORD_ID, "ACGT", True), ("r2", None, False)]
+    for c in cases:
+        a = _ours()(*c["args"])
+        assert vars(a) == c["vars"]
+        if c["args"][1] is not None:
+            assert len(a) == c["len"] and a[1:3] == c["seq_1_3"]
 
 
 def test_get_all_kmers_behaves_like_the_reference():
     from scripts_shim_check import load_names
-    ours, ref = load_names()
+    ours = load_names()
+    ref = _reference()["read_kmer_cloud"]
     assert "get_all_kmers" in ours
-    assert ours["get_all_kmers"]({}) == []
+    assert ours["get_all_kmers"]({}) == ref["get_all_kmers"]["{}"] == []
+    assert ref["get_all_kmers"]["{'r': object()}"] == "AttributeError"
     with pytest.raises(AttributeError):
         ours["get_all_kmers"]({"r": object()})
-    if ref is not None:
-        assert ref["get_all_kmers"]({}) == []
-        with pytest.raises(AttributeError):
-            ref["get_all_kmers"]({"r": object()})
-        missing = {n for n in ref["__public__"] if n not in ours["__public__"]}
-        assert not missing, f"names the reference module binds and the drop-in does not: {missing}"
+    missing = {n for n in ref["public"] if n not in ours["__public__"]}
+    assert not missing, f"names the reference module binds and the drop-in does not: {missing}"
