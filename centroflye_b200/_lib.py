@@ -41,6 +41,10 @@ SIGNATURES = {
     "cfk_rr_max_symbols": (_int, []),
     "cfk_rr_words": (_int, [_i32]),
     "cfk_rr_filter": (_int, [_p, _p, _p, _p, _i64, _p, _p, _i32, _i32, _i32, _p, _p, _p]),
+    "cfk_seq_scan": (_int, [_p, _i64, _i32, _p, _i64, _p, _i64, _p]),  # host pointers
+    "cfk_rr_gather": (_int, [_p, _p, _i64, _p, _i64, _p]),
+    "cfk_rr_keep_sizes": (_int, [_p, _p, _p, _i64, _p, _p]),
+    "cfk_rr_emit": (_int, [_p, _p, _p, _p, _i64, _i64, _p, _p]),
     "cfk_placer_best_blocks": (_int, []),
     "cfk_placer_add_read": (_int, [_p, _p, _i64, _i32, _i64, _i64, _u32, _p, _p, _i64, _p, _p, _i64, _p, _p]),
     "cfk_placer_initial_pairs": (_int, [_p, _i64, _p, _p, _i64, _p, _p]),

@@ -106,6 +106,95 @@ int rr_launch(const RrArgs& A, cudaStream_t st) {
   return NW;
 }
 
+// ---- streaming form (read_recruitment.recruit_file): raw file text in, output file text out ----------------------
+// Both copy kernels are driven by the destination: one thread writes 16 consecutive output bytes with one 16-byte store
+// and finds its source by a binary search over the sorted destination offsets, so 80-column FASTA lines and megabase
+// single-line reads cost the same per byte.
+constexpr int COPY_THREADS = 256;
+
+// last i in [0, n) with key[i * stride] <= q (keys ascending, key[0] <= q)
+__device__ __forceinline__ int64_t last_at_or_below(const int64_t* key, int64_t stride, int64_t n, int64_t q) {
+  int64_t lo = 0, hi = n;
+  while (hi - lo > 1) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (key[mid * stride] <= q) lo = mid;
+    else hi = mid;
+  }
+  return lo;
+}
+
+__device__ __forceinline__ uint4 pack16(const uint8_t* b) {
+  uint32_t w[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+    w[i] = (uint32_t)b[4 * i] | ((uint32_t)b[4 * i + 1] << 8) | ((uint32_t)b[4 * i + 2] << 16) | ((uint32_t)b[4 * i + 3] << 24);
+  return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+// text[q] = the sequence byte that piece p places at q, 0 between records.  piece = [n][3] (source offset in raw,
+// length, destination offset), destinations ascending and non-overlapping.
+__global__ void __launch_bounds__(COPY_THREADS) rr_gather_kernel(const uint8_t* __restrict__ raw, const int64_t* __restrict__ piece,
+                                                                 int64_t n_pieces, uint8_t* __restrict__ text, int64_t text_bytes) {
+  const int64_t q0 = ((int64_t)blockIdx.x * COPY_THREADS + threadIdx.x) * 16;
+  if (q0 >= text_bytes) return;
+  uint8_t b[16];
+  int64_t p = (n_pieces > 0 && piece[2] <= q0) ? last_at_or_below(piece + 2, 3, n_pieces, q0) : 0;
+  int64_t src = 0, dst = INT64_MAX, end = INT64_MAX;
+  if (p < n_pieces) src = piece[3 * p], end = (dst = piece[3 * p + 2]) + piece[3 * p + 1];
+#pragma unroll
+  for (int k = 0; k < 16; ++k) {
+    const int64_t q = q0 + k;
+    while (q >= end && ++p < n_pieces) src = piece[3 * p], end = (dst = piece[3 * p + 2]) + piece[3 * p + 1];
+    b[k] = (q >= dst && q < end) ? raw[src + (q - dst)] : 0;
+  }
+  reinterpret_cast<uint4*>(text)[q0 >> 4] = pack16(b);
+}
+
+// sizes[r] = bytes of ">name\nsequence\n" when record r is kept, else 0.  A record is kept when any of its segments
+// seg_keep[seg_ptr[r] .. seg_ptr[r + 1]) hit; seg_keep == NULL keeps every record.
+__global__ void rr_keep_sizes_kernel(const uint8_t* __restrict__ seg_keep, const int64_t* __restrict__ seg_ptr,
+                                     const int64_t* __restrict__ rec, int64_t n, int32_t* __restrict__ sizes) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  bool keep = seg_keep == nullptr;
+  if (!keep)
+    for (int64_t s = seg_ptr[r]; s < seg_ptr[r + 1] && !keep; ++s) keep = seg_keep[s] != 0;
+  sizes[r] = keep ? (int32_t)(rec[4 * r + 1] + rec[4 * r + 2] + 3) : 0;
+}
+
+// out[out_off[r] ..] = ">" name "\n" sequence "\n" of record r (rec = [n][4]: name offset in raw, name length, sequence
+// length, sequence offset in text); out_off = exclusive scan of the sizes, out_off[n] = total.
+__global__ void __launch_bounds__(COPY_THREADS) rr_emit_kernel(const uint8_t* __restrict__ raw, const uint8_t* __restrict__ text,
+                                                               const int64_t* __restrict__ rec, const int64_t* __restrict__ out_off,
+                                                               int64_t n, int64_t max_bytes, uint8_t* __restrict__ out) {
+  const int64_t total = min(out_off[n], max_bytes);
+  const int64_t q0 = ((int64_t)blockIdx.x * COPY_THREADS + threadIdx.x) * 16;
+  if (q0 >= total) return;
+  int64_t r = last_at_or_below(out_off, 1, n + 1, q0);
+  int64_t lo = out_off[r], hi = out_off[r + 1];
+  uint8_t b[16];
+#pragma unroll
+  for (int k = 0; k < 16; ++k) {
+    const int64_t q = q0 + k;
+    if (q >= total) {
+      b[k] = 0;
+      continue;
+    }
+    while (q >= hi) lo = hi, hi = out_off[++r + 1];
+    const int64_t at = q - lo, nl = rec[4 * r + 1];
+    uint8_t c = '\n';
+    if (at == 0) c = '>';
+    else if (at <= nl) c = raw[rec[4 * r] + at - 1];
+    else if (at > nl + 1 && q < hi - 1) c = text[rec[4 * r + 3] + at - nl - 2];
+    b[k] = c;
+  }
+  if (q0 + 16 <= total) {
+    reinterpret_cast<uint4*>(out)[q0 >> 4] = pack16(b);
+  } else {
+    for (int k = 0; q0 + k < total; ++k) out[q0 + k] = b[k];
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -140,6 +229,39 @@ int cfk_rr_filter(const uint8_t* text, const int64_t* read_off, const int64_t* r
     default: rr_launch<52>(A, st); break;
   }
   CFK_CHECK_LAUNCH("rr_filter_kernel", 1);
+  return CFK_OK;
+}
+
+int cfk_rr_gather(const uint8_t* raw, const int64_t* pieces, int64_t n_pieces, uint8_t* text, int64_t text_bytes,
+                  cfk_stream_t stream) {
+  if (n_pieces < 0 || text_bytes < 0 || (text_bytes & 15) != 0 || ((uintptr_t)text & 15u) != 0)
+    return fail(CFK_ERR_INVALID, "cfk_rr_gather: bad sizes, or text not 16-byte aligned");
+  if (text_bytes == 0) return CFK_OK;
+  rr_gather_kernel<<<(unsigned)blocks_for(text_bytes / 16, COPY_THREADS), COPY_THREADS, 0, (cudaStream_t)stream>>>(
+      raw, pieces, n_pieces, text, text_bytes);
+  CFK_CHECK_LAUNCH("rr_gather_kernel", 1);
+  return CFK_OK;
+}
+
+int cfk_rr_keep_sizes(const uint8_t* seg_keep, const int64_t* seg_ptr, const int64_t* records, int64_t n_records,
+                      int32_t* sizes, cfk_stream_t stream) {
+  if (n_records < 0 || (seg_keep == nullptr) != (seg_ptr == nullptr))
+    return fail(CFK_ERR_INVALID, "cfk_rr_keep_sizes: n_records < 0, or only one of seg_keep / seg_ptr given");
+  if (n_records == 0) return CFK_OK;
+  rr_keep_sizes_kernel<<<(unsigned)blocks_for(n_records, 256), 256, 0, (cudaStream_t)stream>>>(seg_keep, seg_ptr, records,
+                                                                                                n_records, sizes);
+  CFK_CHECK_LAUNCH("rr_keep_sizes_kernel", 1);
+  return CFK_OK;
+}
+
+int cfk_rr_emit(const uint8_t* raw, const uint8_t* text, const int64_t* records, const int64_t* out_off, int64_t n_records,
+                int64_t max_bytes, uint8_t* out, cfk_stream_t stream) {
+  if (n_records < 0 || max_bytes < 0 || ((uintptr_t)out & 15u) != 0)
+    return fail(CFK_ERR_INVALID, "cfk_rr_emit: bad sizes, or out not 16-byte aligned");
+  if (n_records == 0 || max_bytes == 0) return CFK_OK;
+  rr_emit_kernel<<<(unsigned)blocks_for((max_bytes + 15) / 16, COPY_THREADS), COPY_THREADS, 0, (cudaStream_t)stream>>>(
+      raw, text, records, out_off, n_records, max_bytes, out);
+  CFK_CHECK_LAUNCH("rr_emit_kernel", 1);
   return CFK_OK;
 }
 

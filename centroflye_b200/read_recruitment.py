@@ -3,11 +3,20 @@ device: same command line (``rr unit.fasta reads.fasta[.gz] output.fasta edit_di
 
 rr.cpp:73-90 aligns the unit and its reverse complement against every read with edlib in HW mode (the whole unit
 against any infix of the read, k = threshold) and copies the read to the output when either alignment exists.  Here the
-two alignments of every read are bit-parallel scans on the GPU (csrc/rr_filter.cu, cfk_rr_filter); the host parses the
-FASTA / FASTQ (plain or gzip, like kseq) and writes ``>name\\nsequence\\n`` for the kept reads in input order.
+two alignments of every read are bit-parallel scans on the GPU (csrc/rr_filter.cu, cfk_rr_filter).
+
+The command line streams (recruit_file): the read file goes through in chunks of a fixed size -- a reader thread reads
+or inflates it, a native scanner (csrc/seq_scan.cpp, cfk_seq_scan) finds the records of a chunk, the device gathers
+the sequences, filters them and assembles ``>name\\nsequence\\n`` of the kept reads in input order, and a writer thread
+appends that to the output.  Host and device memory follow the chunk size, not the input size.  read_sequences() and
+recruit() are the in-memory form of the same computation, and the specification the streaming form is tested against.
 """
 import gzip
+import os
+import queue
 import sys
+import threading
+import time
 
 import numpy as np
 
@@ -132,6 +141,367 @@ def recruit(unit, seqs, threshold, exact=False, engine=None):
     return (keep, dist) if exact else keep
 
 
+CHUNK_BYTES = 64 << 20  # read-file bytes per streaming step (recruit_file); main() uses this
+_BLOCK_BYTES = 8 << 20   # the reader thread's unit of readinto / inflate; four blocks are read ahead
+# scanner table sizes: a record slot (32 bytes) per 128 chunk bytes, a piece slot (24 bytes) per 64; a chunk whose
+# records need more is processed in parts
+_REC_BYTES_PER_SLOT, _PIECE_BYTES_PER_SLOT = 128, 64
+
+
+def _open_binary(path):
+    """The read file as bytes, inflated when it starts with the gzip magic (like read_sequences)."""
+    with open(path, "rb") as f:
+        magic = f.read(2)
+    return gzip.open(path, "rb") if magic == b"\x1f\x8b" else open(path, "rb")
+
+
+class _Fallback(Exception):
+    """The chunk is outside what the streaming form reproduces byte for byte (a byte >= 0x80, which str semantics
+    treat differently, or a record too large for the int32 output sizes): recruit_file runs the in-memory path."""
+
+
+class _BlockReader:
+    """Reads (or inflates) the file block by block on a thread of its own; readinto and zlib release the GIL."""
+
+    def __init__(self, path, block, depth=4):
+        self.f = _open_binary(path)
+        self.block, self.seconds = block, 0.0
+        self.free, self.full = queue.Queue(), queue.Queue()
+        for _ in range(depth):
+            self.free.put(np.empty(block, dtype=np.uint8))
+        self.thread = threading.Thread(target=self._run, name="rr-reader", daemon=True)
+        self.thread.start()
+
+    def _run(self):
+        try:
+            while True:
+                buf = self.free.get()
+                if buf is None:
+                    return
+                t0, n, view = time.perf_counter(), 0, memoryview(buf)
+                while n < buf.size:
+                    k = self.f.readinto(view[n:])
+                    if not k:
+                        break
+                    n += k
+                self.seconds += time.perf_counter() - t0
+                self.full.put((buf, n))
+                if n < buf.size:
+                    return
+        except BaseException as e:  # noqa: BLE001 -- handed to the consumer, which raises it
+            self.full.put(e)
+
+    def get(self):
+        item = self.full.get()
+        if isinstance(item, BaseException):
+            raise item
+        return item
+
+    def close(self):
+        self.free.put(None)
+        self.thread.join()
+        self.f.close()
+
+
+def _grown(store, key, nbytes, make):
+    """store[key], replaced by make(size) when it holds fewer than nbytes bytes (sizes are multiples of 16, and exact
+    otherwise: the pinned host allocator rounds up to a power of two, and chunk sizes usually are one)."""
+    buf = store.get(key)
+    if buf is None or buf.numel() < nbytes:
+        buf = store[key] = make(max(int(nbytes) + 15 & ~15, 1 << 12))
+    return buf
+
+
+def _scan_chunks(read_fn, chunk_bytes, host, stats):
+    """Chunks of the read file cut at record boundaries by cfk_seq_scan: yields (slot, raw, records, pieces, text_bytes)
+    where raw (uint8 tensor) holds the chunk's text, records int64[n, 4] and pieces int64[m, 3] are the scanner's tables
+    (numpy views of tensors in `host`, made by host["alloc"]).  Two slots alternate: what is yielded stays valid until
+    the next-but-one chunk is asked for.  A chunk without a complete record is doubled until it has one, so an
+    ultra-long read fits any chunk size."""
+    alloc = lambda key, nbytes: _grown(host, key, nbytes, host["alloc"])  # noqa: E731
+    reader = _BlockReader(read_fn, max(1 << 16, min(chunk_bytes, _BLOCK_BYTES)))
+    out = np.zeros(5, dtype=np.int64)
+    carry, eof, slot, table_scale = np.zeros(0, dtype=np.uint8), False, 0, 1
+    blk, at, k = None, 0, 0  # the reader's block being taken apart: blk[at:k] is not in a chunk yet
+    try:
+        while True:
+            n, target = carry.size, max(chunk_bytes, carry.size)
+            raw = alloc((slot, "raw"), target)
+            raw.numpy()[:n] = carry
+            while True:
+                t0 = time.perf_counter()
+                while n < target and not (eof and blk is None):
+                    if blk is None:
+                        blk, k = reader.get()
+                        at, eof = 0, k < blk.size
+                    if raw.numel() < target:
+                        old = raw
+                        raw = alloc((slot, "raw"), target)
+                        raw[:n] = old[:n]
+                    take = min(k - at, target - n)
+                    raw.numpy()[n:n + take] = blk[at:at + take]
+                    n, at = n + take, at + take
+                    if at == k:
+                        reader.free.put(blk)
+                        blk = None
+                end = eof and blk is None
+                t1 = time.perf_counter()
+                max_rec = table_scale * max(64, n // _REC_BYTES_PER_SLOT)
+                max_piece = table_scale * max(64, n // _PIECE_BYTES_PER_SLOT)
+                rec = alloc((slot, "rec"), 32 * max_rec).numpy().view(np.int64)
+                piece = alloc((slot, "piece"), 24 * max_piece).numpy().view(np.int64)
+                buf = raw.numpy()
+                _lib.call("cfk_seq_scan", buf.ctypes.data, n, int(end), rec.ctypes.data, max_rec, piece.ctypes.data,
+                          max_piece, out.ctypes.data)
+                stats["assemble_s"] += t1 - t0
+                stats["scan_s"] += time.perf_counter() - t1
+                n_rec, n_piece, consumed, text_bytes, flags = out.tolist()
+                if flags & _SCAN_NOT_ASCII:
+                    raise _Fallback("a byte >= 0x80 in the read file")
+                if n_rec:
+                    break
+                if flags & _SCAN_FULL:
+                    table_scale *= 2
+                elif end:
+                    return
+                else:
+                    target = 2 * n
+            yield slot, raw[:n], rec[:4 * n_rec].reshape(-1, 4), piece[:3 * n_piece].reshape(-1, 3), text_bytes
+            if end and consumed == n:
+                return
+            carry, slot = buf[consumed:n], slot ^ 1
+    finally:
+        stats["read_s"] += reader.seconds
+        reader.close()
+
+
+_SCAN_NOT_ASCII, _SCAN_FULL = 1, 2  # cfk_seq_scan flags (include/cfk.h)
+
+
+def scan_sequences(path, chunk_bytes=CHUNK_BYTES):
+    """(name, sequence) of every record, as read_sequences(path) yields them, through the native scanner and the
+    chunking of recruit_file, on the host alone.  Raises _Fallback where recruit_file hands over to read_sequences."""
+    import torch
+    host = {"alloc": lambda n: torch.empty(n, dtype=torch.uint8)}
+    stats = {"assemble_s": 0.0, "scan_s": 0.0, "read_s": 0.0}
+    for _, raw, rec, piece, _ in _scan_chunks(path, chunk_bytes, host, stats):
+        buf, p = raw.numpy(), 0
+        for name_off, name_len, seq_len, seq_dst in rec.tolist():
+            parts = []
+            while p < len(piece) and piece[p, 2] < seq_dst + seq_len:
+                parts.append(buf[piece[p, 0]:piece[p, 0] + piece[p, 1]].tobytes())
+                p += 1
+            yield buf[name_off:name_off + name_len].tobytes().decode(), b"".join(parts).decode()
+
+
+def _write_in_memory(unit, read_fn, path, threshold):
+    """The whole read set as Python strings, one recruit() call, one write: the form every input can take."""
+    records = list(read_sequences(read_fn))
+    keep = recruit(unit, [seq for _, seq in records], threshold) if records else np.zeros(0, dtype=bool)
+    with open(path, "w") as f:
+        f.write("".join(f">{name}\n{seq}\n" for (name, seq), k in zip(records, keep.tolist()) if k))
+
+
+def recruit_file(unit, read_fn, output_fn, threshold, chunk_bytes=CHUNK_BYTES, engine=None, stats=None):
+    """rr's whole run, from the read file to the output file: ``>name\\nsequence\\n`` of every read of read_fn (FASTA /
+    FASTQ, plain or gzip) that holds the unit or its reverse complement within `threshold` edits (threshold < 0: every
+    read), in input order -- the bytes the in-memory path (read_sequences + recruit) writes, streamed in chunks of
+    about chunk_bytes.  The output appears under output_fn only when the run has finished (it is written to a temporary
+    file beside it, then renamed).  An input without records gives an empty file and touches neither the device nor the
+    unit; otherwise an invalid unit raises before any output exists.  A chunk with a byte >= 0x80 hands the whole run to
+    the in-memory path.  stats: None, or a dict that receives seconds per host stage, device seconds per stage
+    (CUDA events, "device_s") and counts."""
+    threshold = int(threshold)
+    out_dir, base = os.path.split(os.path.abspath(output_fn))
+    i = 0
+    while True:
+        tmp = os.path.join(out_dir, f".{base}.{os.getpid()}.{i}.part")
+        try:
+            f = open(tmp, "xb")
+            break
+        except FileExistsError:
+            i += 1
+    st = {key: 0.0 for key in ("read_s", "assemble_s", "scan_s", "plan_s", "wait_s", "write_s")}
+    st.update(chunks=0, records=0, bases=0, out_bytes=0, fallback=None, device_s=None if stats is None else {})
+    try:
+        try:
+            with f:
+                _stream(unit, read_fn, f, threshold, chunk_bytes, engine, st)
+        except _Fallback as e:
+            st["fallback"] = str(e)
+            _write_in_memory(unit, read_fn, tmp, threshold)
+        os.replace(tmp, output_fn)
+    except BaseException:
+        if os.path.exists(tmp):
+            os.remove(tmp)
+        raise
+    if stats is not None:
+        stats.update(st)
+    return 0
+
+
+def _stream(unit, read_fn, f, threshold, chunk_bytes, engine, st):
+    """recruit_file's pipeline.  While the device works on chunk i, the reader thread reads ahead, this thread scans
+    chunk i + 1, and the writer thread writes chunk i - 1.  Every device step of a chunk is on one stream, so one set
+    of device buffers serves all chunks; host buffers come in two slots (see _scan_chunks) plus two output buffers."""
+    import torch
+    host = {"alloc": lambda n: torch.empty(n, dtype=torch.uint8)}  # pageable until the first record is seen
+    dev, out_host = {}, {}
+    device_s, events = st["device_s"], []
+    eng = d_peq = d_sym = writer = None
+    writer_q, free_out, writer_err = queue.Queue(), queue.Queue(), []
+
+    def mark():
+        if device_s is None:
+            return None
+        e = torch.cuda.Event(enable_timing=True)
+        e.record()
+        return e
+
+    def write_loop():
+        while True:
+            item = writer_q.get()
+            if item is None:
+                return
+            done, key, nbytes = item
+            try:
+                done.synchronize()
+                t0 = time.perf_counter()
+                f.write(memoryview(out_host[key].numpy()[:nbytes]))
+                st["write_s"] += time.perf_counter() - t0
+            except BaseException as e:  # noqa: BLE001 -- raised by the main thread at its next hand-over
+                writer_err.append(e)
+            free_out.put(key)
+
+    def start_device():
+        nonlocal eng, d_peq, d_sym, writer
+        from .engine import default_engine
+        eng = engine or default_engine()
+        peq, sym_of, _ = build_masks(unit)  # raises on an invalid unit, before any output
+        d_peq, d_sym = eng._to_dev(peq.reshape(-1).view(np.int64)), eng._to_dev(sym_of)
+        host["alloc"] = lambda n: torch.empty(n, dtype=torch.uint8, pin_memory=True)
+        for key in (0, 1):
+            free_out.put(key)
+        writer = threading.Thread(target=write_loop, name="rr-writer", daemon=True)
+        writer.start()
+
+    def dbuf(key, nbytes, dtype=torch.uint8):
+        t = _grown(dev, key, nbytes, lambda n: torch.empty(n, dtype=torch.uint8, device=eng.device))
+        return t.view(dtype)
+
+    def launch(slot, raw, rec, piece, text_bytes):
+        p = eng._p
+        t0 = time.perf_counter()
+        R, P, n = rec.shape[0], piece.shape[0], raw.numel()
+        seq_len = rec[:, 2]
+        sizes = rec[:, 1] + seq_len + 3
+        if int(sizes.max()) >= 1 << 31:
+            raise _Fallback("a record of 2 GiB or more")
+        upper = int(sizes.sum())
+        st["records"] += R
+        st["bases"] += int(seq_len.sum())
+        # segments as recruit() plans them; threshold < 0 keeps every read without a filter run.  Host layout, int64:
+        # seg_off[S] | seg_len[S] | seg_ptr[R + 1] (first segment of each record) | order[S] (int32 in the first half)
+        S = 0
+        if threshold >= 0:
+            overlap = len(unit) + threshold
+            n_seg = np.maximum(1, -(-np.maximum(seq_len - overlap, 1) // SEGMENT))
+            S = int(n_seg.sum())
+            seg_read = np.repeat(np.arange(R, dtype=np.int64), n_seg)
+            j = np.arange(S, dtype=np.int64) - np.repeat(np.cumsum(n_seg) - n_seg, n_seg)
+            nb = 8 * (3 * S + R + 1)
+            hs = _grown(host, (slot, "seg"), nb, host["alloc"])
+            seg = hs.numpy()[:nb].view(np.int64)
+            seg_lens = seg[S:2 * S]
+            seg[:S] = rec[seg_read, 3] + j * SEGMENT
+            seg_lens[:] = np.minimum(SEGMENT + overlap, seq_len[seg_read] - j * SEGMENT)
+            seg[2 * S] = 0
+            np.cumsum(n_seg, out=seg[2 * S + 1:2 * S + R + 1])
+            seg[2 * S + R + 1:].view(np.int32)[:S] = np.argsort(-seg_lens, kind="stable")
+        st["plan_s"] += time.perf_counter() - t0
+        a = mark()
+        d_raw = dbuf("raw", n + 16)
+        d_raw[:n].copy_(raw, non_blocking=True)
+        d_rec = dbuf("rec", 32 * R, torch.int64)
+        d_rec[:4 * R].copy_(torch.from_numpy(rec.reshape(-1)), non_blocking=True)
+        d_piece = dbuf("piece", 24 * P + 8, torch.int64)
+        if P:
+            d_piece[:3 * P].copy_(torch.from_numpy(piece.reshape(-1)), non_blocking=True)
+        if S:
+            d_seg = dbuf("seg", nb)
+            d_seg[:nb].copy_(hs[:nb], non_blocking=True)
+        b = mark()
+        stream = eng._stream()
+        d_text = dbuf("text", text_bytes + 16)
+        _lib.call("cfk_rr_gather", p(d_raw), p(d_piece), P, p(d_text), text_bytes, stream)
+        c = mark()
+        d_keep = seg_ptr = None
+        if S:
+            d_keep = dbuf("keep", S)
+            d_keep[:S].zero_()
+            base = d_seg.data_ptr()
+            seg_ptr = base + 16 * S
+            _lib.call("cfk_rr_filter", p(d_text), base, base + 8 * S, base + 8 * (2 * S + R + 1), S, p(d_peq), p(d_sym),
+                      len(unit), threshold, 0, None, p(d_keep), stream)
+        d = mark()
+        d_sizes = dbuf("sizes", 4 * R, torch.int32)
+        d_off = dbuf("off", 8 * (R + 1), torch.int64)
+        d_scratch = dbuf("scratch", 8 * int(eng.lib.cfk_scan_scratch_elems(R)))
+        d_out = dbuf("out", upper + 16)
+        _lib.call("cfk_rr_keep_sizes", p(d_keep), seg_ptr, p(d_rec), R, p(d_sizes), stream)
+        _lib.call("cfk_exclusive_scan", p(d_sizes), p(d_off), R, p(d_scratch), stream)
+        _lib.call("cfk_rr_emit", p(d_raw), p(d_text), p(d_rec), p(d_off), R, upper, p(d_out), stream)
+        if device_s is not None:
+            events.extend((("h2d", a, b), ("gather", b, c), ("filter", c, d), ("emit", d, mark())))
+        st["chunks"] += 1
+        return d_off[R], d_out
+
+    def finish(d_total, d_out):
+        t0 = time.perf_counter()
+        total = int(d_total.item())  # the chunk's one size read-back
+        key = free_out.get()
+        st["wait_s"] += time.perf_counter() - t0
+        if writer_err:
+            raise writer_err[0]
+        h = _grown(out_host, key, total, host["alloc"])
+        a = mark()
+        if total:
+            h[:total].copy_(d_out[:total], non_blocking=True)
+        done = torch.cuda.Event()
+        done.record()
+        if device_s is not None:
+            events.append(("d2h", a, mark()))
+        st["out_bytes"] += total
+        writer_q.put((done, key, total))
+
+    chunks = _scan_chunks(read_fn, chunk_bytes, host, st)
+    pending = None
+    try:
+        for slot, raw, rec, piece, text_bytes in chunks:  # scanning chunk i overlaps the device's work on chunk i - 1
+            if pending is not None:
+                finish(*pending)
+            first = eng is None
+            if first:
+                start_device()
+            pending = launch(slot, raw, rec, piece, text_bytes)
+            if first:  # chunk 0 was scanned into pageable memory (copied synchronously): later chunks use pinned buffers
+                for name in ("raw", "rec", "piece"):
+                    host.pop((slot, name))
+        if pending is not None:
+            finish(*pending)
+    finally:
+        chunks.close()
+        if writer is not None:
+            writer_q.put(None)
+            writer.join()
+    if writer_err:
+        raise writer_err[0]
+    if device_s is not None:
+        torch.cuda.synchronize()
+        for name, a, b in events:
+            device_s[name] = device_s.get(name, 0.0) + a.elapsed_time(b) / 1e3
+
+
 def main(argv=None):
     argv = sys.argv[1:] if argv is None else list(argv)
     if len(argv) != 4 or argv[0] == "-h":
@@ -143,10 +513,7 @@ def main(argv=None):
     except ValueError:
         threshold = 0  # std::atoi
     unit = next(read_sequences(unit_fn))[1]
-    records = list(read_sequences(read_fn))
-    keep = recruit(unit, [seq for _, seq in records], threshold) if records else np.zeros(0, dtype=bool)
-    with open(output_fn, "w") as f:
-        f.write("".join(f">{name}\n{seq}\n" for (name, seq), k in zip(records, keep.tolist()) if k))
+    recruit_file(unit, read_fn, output_fn, threshold)
     return 0
 
 

@@ -193,6 +193,42 @@ int cfk_rr_filter(const uint8_t* text, const int64_t* read_off, const int64_t* r
                   const uint64_t* peq, const uint8_t* sym_of, int32_t m, int32_t threshold, int32_t exact, int32_t* out_dist,
                   uint8_t* out_keep, cfk_stream_t stream);
 
+/* ---- streaming read recruitment: read file text in, output file text out ---------------------------------------
+ * cfk_seq_scan (HOST code) finds the records of one chunk of FASTA / FASTQ text exactly as read_sequences() yields them
+ * (centroflye_b200/read_recruitment.py:29-55, the restatement of rr.cpp's kseq_read loop): "\n", "\r\n" and a lone "\r"
+ * end a line; lines before a header ('>' or '@') are skipped; the name is the header after its first byte up to the
+ * first whitespace (str.isspace on ASCII), after leading whitespace; sequence lines, each stripped of whitespace at
+ * both ends, run until a line starting with '>', '@' or '+'; after '+' whole lines are skipped while fewer quality
+ * characters than bases have been.  It writes
+ *   records_h [n][4]   name offset in buf_h, name length, sequence length, sequence offset in the packed text (every
+ *                      sequence on a 16-byte boundary, text_bytes in all), for every complete record;
+ *   pieces_h  [n][3]   source offset in buf_h, length, destination offset in the packed text, per non-empty stripped
+ *                      sequence line of those records, in order;
+ *   out_h     [5]      n_records, n_pieces, consumed, text_bytes, flags.
+ * `consumed` is where the first incomplete record (or unfinished line) begins: the caller carries buf_h[consumed:] into
+ * the next chunk.  Without at_eof a record ending with the chunk is incomplete, and so is a '\r' as its last byte.  The
+ * scan stops before a record that does not fit max_records / max_pieces (flag CFK_SCAN_FULL).  A byte >= 0x80 anywhere
+ * in the chunk sets CFK_SCAN_NOT_ASCII and nothing else: str semantics differ from byte semantics there.
+ *
+ * The device part, on the chunk copied to the device as it is (raw):
+ *   cfk_rr_gather      text[pieces[p][2] + i] = raw[pieces[p][0] + i]; 0 elsewhere; text 16-byte aligned, text_bytes a
+ *                      multiple of 16 -> the text cfk_rr_filter reads;
+ *   cfk_rr_keep_sizes  sizes[r] = bytes of ">name\nsequence\n" if any of the segments seg_keep[seg_ptr[r] ..
+ *                      seg_ptr[r + 1]) of record r hit (seg_keep = cfk_rr_filter's out_keep over segments), else 0;
+ *                      seg_keep = seg_ptr = NULL keeps every record -> out_off by cfk_exclusive_scan;
+ *   cfk_rr_emit        out[out_off[r] ..] = ">name\nsequence\n" of every kept record, names from raw, sequences from
+ *                      text; bytes at or beyond max_bytes are not written (launch size: max_bytes / 16 threads). */
+#define CFK_SCAN_NOT_ASCII 1
+#define CFK_SCAN_FULL 2
+int cfk_seq_scan(const uint8_t* buf_h, int64_t len, int32_t at_eof, int64_t* records_h, int64_t max_records,
+                 int64_t* pieces_h, int64_t max_pieces, int64_t* out_h);
+int cfk_rr_gather(const uint8_t* raw, const int64_t* pieces, int64_t n_pieces, uint8_t* text, int64_t text_bytes,
+                  cfk_stream_t stream);
+int cfk_rr_keep_sizes(const uint8_t* seg_keep, const int64_t* seg_ptr, const int64_t* records, int64_t n_records,
+                      int32_t* sizes, cfk_stream_t stream);
+int cfk_rr_emit(const uint8_t* raw, const uint8_t* text, const int64_t* records, const int64_t* out_off, int64_t n_records,
+                int64_t max_bytes, uint8_t* out, cfk_stream_t stream);
+
 /* ---- read_placer scoring on the cloud CSR (SURVEY.md §8f rank 2) --------------------------------
  * Replaces the data structures of ReadPlacer.add_reads, scripts/read_placer.py:42-94, and of CloudContig.add_read /
  * update_mapping_scores, scripts/cloud_contig.py:26-41,87-95; the greedy loop (one read per iteration) stays on the
