@@ -22,28 +22,42 @@ using namespace cfk;
 constexpr int RR_THREADS = 128;
 constexpr int RR_MAX_SYMBOLS = 8;  // distinct bytes of the unit (ACGT in practice) + slot 0 = "not in the unit"
 
+// One unit of a launch: where its match masks and symbol table are, its length and threshold.
+struct RrUnit {
+  int64_t peq_off;            // first word of the unit's [2][RR_MAX_SYMBOLS][NW] block in RrArgs::peq
+  int64_t keep_off;           // index * n_reads: the unit's row of out_keep
+  int32_t index;              // the unit's row of sym_of [U][256]
+  int32_t m;                  // unit length
+  int32_t threshold;          // < 0: no limit (edlib's k = -1)
+  int32_t pad;
+};
+constexpr int RR_UNITS_PER_LAUNCH = 64;  // blockIdx.y < this; a word class with more units takes several launches
+
 struct RrArgs {
   const uint8_t* text;        // all reads, every read starts on a 16-byte boundary
   const int64_t* read_off;    // byte offset of read r
   const int64_t* read_len;
   const int32_t* order;       // items are dealt longest read first
   int64_t n_reads;
-  const uint64_t* peq;        // [2 strands][RR_MAX_SYMBOLS][NW]
-  const uint8_t* sym_of;      // [256] byte -> symbol slot (0 = not in the unit)
-  int32_t m;                  // unit length
-  int32_t threshold;          // < 0: no limit (edlib's k = -1)
+  const uint64_t* peq;        // per unit [2 strands][RR_MAX_SYMBOLS][NW], at RrUnit::peq_off
+  const uint8_t* sym_of;      // per unit [256] byte -> symbol slot (0 = not in the unit)
   int32_t exact;              // != 0: never stop early, out_dist holds the exact infix distance
-  int32_t* out_dist;          // [2 * n_reads] (read, strand), or NULL
-  uint8_t* out_keep;          // [n_reads]
+  int32_t* out_dist;          // [U][2 * n_reads] (read, strand), or NULL
+  uint8_t* out_keep;          // [U][n_reads]
+  RrUnit unit[RR_UNITS_PER_LAUNCH];  // blockIdx.y selects one (read from the parameter space: __grid_constant__)
 };
 
 template <int NW>
-__global__ void __launch_bounds__(RR_THREADS) rr_filter_kernel(const RrArgs A) {
+__global__ void __launch_bounds__(RR_THREADS) rr_filter_kernel(const __grid_constant__ RrArgs A) {
   __shared__ uint64_t s_peq[2 * RR_MAX_SYMBOLS * NW];
   __shared__ uint8_t s_sym[256];
-  for (int i = threadIdx.x; i < 2 * RR_MAX_SYMBOLS * NW; i += RR_THREADS) s_peq[i] = A.peq[i];
-  for (int i = threadIdx.x; i < 256; i += RR_THREADS) s_sym[i] = A.sym_of[i];
+  const RrUnit& U = A.unit[blockIdx.y];
+  const uint64_t* g_peq = A.peq + U.peq_off;
+  const uint8_t* g_sym = A.sym_of + 256 * (int64_t)U.index;
+  for (int i = threadIdx.x; i < 2 * RR_MAX_SYMBOLS * NW; i += RR_THREADS) s_peq[i] = g_peq[i];
+  for (int i = threadIdx.x; i < 256; i += RR_THREADS) s_sym[i] = g_sym[i];
   __syncthreads();
+  const int32_t m = U.m;
   const int64_t item = (int64_t)blockIdx.x * RR_THREADS + threadIdx.x;
   if (item >= 2 * A.n_reads) return;
   const int64_t r = A.order[item >> 1];
@@ -51,15 +65,15 @@ __global__ void __launch_bounds__(RR_THREADS) rr_filter_kernel(const RrArgs A) {
   const uint64_t* peq = s_peq + strand * RR_MAX_SYMBOLS * NW;
   const int64_t n = A.read_len[r];
   const uint4* text = reinterpret_cast<const uint4*>(A.text + A.read_off[r]);
-  const int last_bit = (A.m - 1) & 63;
+  const int last_bit = (m - 1) & 63;
   uint64_t Pv[NW], Mv[NW];
 #pragma unroll
   for (int j = 0; j < NW; ++j) {
     Pv[j] = ~0ull;
     Mv[j] = 0ull;
   }
-  int score = A.m, best = A.m;
-  const bool limited = A.threshold >= 0 && !A.exact;
+  int score = m, best = m;
+  const int stop = A.exact ? -1 : U.threshold;  // best >= 0: a negative value never stops the scan
   for (int64_t t0 = 0; t0 < n; t0 += 16) {
     const uint4 chunk = __ldg(text + (t0 >> 4));
     const int cnt = (int)min((int64_t)16, n - t0);
@@ -93,17 +107,25 @@ __global__ void __launch_bounds__(RR_THREADS) rr_filter_kernel(const RrArgs A) {
         best = min(best, score);
       }
     }
-    if (limited && best <= A.threshold) break;
+    if (best <= stop) break;
   }
-  if (A.out_dist != nullptr) A.out_dist[2 * r + strand] = best;
-  if (A.threshold < 0 || best <= A.threshold) A.out_keep[r] = 1;
+  const int64_t at = U.keep_off + r;
+  if (A.out_dist != nullptr) A.out_dist[2 * at + strand] = best;
+  if (U.threshold < 0 || best <= U.threshold) A.out_keep[at] = 1;
 }
 
-template <int NW>
-int rr_launch(const RrArgs& A, cudaStream_t st) {
-  const int64_t items = 2 * A.n_reads;
-  rr_filter_kernel<NW><<<(unsigned)blocks_for(items, RR_THREADS), RR_THREADS, 0, st>>>(A);
-  return NW;
+// A.unit[0 .. n_units) all have cfk_rr_words(m) == nw.
+int rr_launch(int nw, const RrArgs& A, int n_units, cudaStream_t st) {
+  const dim3 grid((unsigned)blocks_for(2 * A.n_reads, RR_THREADS), (unsigned)n_units);
+  switch (nw) {
+    case 4: rr_filter_kernel<4><<<grid, RR_THREADS, 0, st>>>(A); break;
+    case 9: rr_filter_kernel<9><<<grid, RR_THREADS, 0, st>>>(A); break;
+    case 17: rr_filter_kernel<17><<<grid, RR_THREADS, 0, st>>>(A); break;
+    case 33: rr_filter_kernel<33><<<grid, RR_THREADS, 0, st>>>(A); break;
+    default: rr_filter_kernel<52><<<grid, RR_THREADS, 0, st>>>(A); break;
+  }
+  CFK_CHECK_LAUNCH("rr_filter_kernel", 1);
+  return CFK_OK;
 }
 
 // ---- streaming form (read_recruitment.recruit_file): raw file text in, output file text out ----------------------
@@ -219,16 +241,40 @@ int cfk_rr_filter(const uint8_t* text, const int64_t* read_off, const int64_t* r
   if (n_reads < 0 || n_reads >= (1ll << 30)) return fail(CFK_ERR_INVALID, "cfk_rr_filter: bad sizes");
   if (((uintptr_t)text & 15u) != 0) return fail(CFK_ERR_INVALID, "cfk_rr_filter: text must be 16-byte aligned");
   if (n_reads == 0) return CFK_OK;
-  RrArgs A{text, read_off, read_len, order, n_reads, peq, sym_of, m, threshold, exact, out_dist, out_keep};
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (nw) {
-    case 4: rr_launch<4>(A, st); break;
-    case 9: rr_launch<9>(A, st); break;
-    case 17: rr_launch<17>(A, st); break;
-    case 33: rr_launch<33>(A, st); break;
-    default: rr_launch<52>(A, st); break;
+  RrArgs A{text, read_off, read_len, order, n_reads, peq, sym_of, exact, out_dist, out_keep, {}};
+  A.unit[0] = RrUnit{0, 0, 0, m, threshold, 0};
+  return rr_launch(nw, A, 1, (cudaStream_t)stream);
+}
+
+int cfk_rr_filter_units(const uint8_t* text, const int64_t* seg_off, const int64_t* seg_len, const int32_t* order, int64_t n_seg,
+                        int32_t n_units, const uint64_t* peq, const uint8_t* sym_of, const int32_t* unit_m,
+                        const int32_t* unit_threshold, uint8_t* out_keep, cfk_stream_t stream) {
+  if (n_seg < 0 || n_seg >= (1ll << 30) || n_units < 0 || (n_units > 0 && (unit_m == nullptr || unit_threshold == nullptr)))
+    return fail(CFK_ERR_INVALID, "cfk_rr_filter_units: bad sizes");
+  if (((uintptr_t)text & 15u) != 0) return fail(CFK_ERR_INVALID, "cfk_rr_filter_units: text must be 16-byte aligned");
+  for (int32_t u = 0; u < n_units; ++u)
+    if (cfk_rr_words(unit_m[u]) < 0) return fail(CFK_ERR_INVALID, "cfk_rr_filter_units: every unit must have 1..3328 bases");
+  if (n_seg == 0 || n_units == 0) return CFK_OK;
+  // one launch per word class present (several when a class has more than RR_UNITS_PER_LAUNCH units), all on `stream`
+  const cudaStream_t st = (cudaStream_t)stream;
+  for (int nw : {4, 9, 17, 33, 52}) {
+    RrArgs A{text, seg_off, seg_len, order, n_seg, peq, sym_of, 0, nullptr, out_keep, {}};
+    int n = 0;
+    int64_t off = 0;
+    for (int32_t u = 0; u < n_units; ++u) {
+      const int w = cfk_rr_words(unit_m[u]);
+      if (w == nw) {
+        A.unit[n++] = RrUnit{off, u * n_seg, u, unit_m[u], unit_threshold[u], 0};
+        if (n == RR_UNITS_PER_LAUNCH) {
+          if (const int rc = rr_launch(nw, A, n, st)) return rc;
+          n = 0;
+        }
+      }
+      off += 2 * RR_MAX_SYMBOLS * w;
+    }
+    if (n > 0)
+      if (const int rc = rr_launch(nw, A, n, st)) return rc;
   }
-  CFK_CHECK_LAUNCH("rr_filter_kernel", 1);
   return CFK_OK;
 }
 

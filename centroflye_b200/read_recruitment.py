@@ -8,7 +8,10 @@ two alignments of every read are bit-parallel scans on the GPU (csrc/rr_filter.c
 The command line streams (recruit_file): the read file goes through in chunks of a fixed size -- a reader thread reads
 or inflates it, a native scanner (csrc/seq_scan.cpp, cfk_seq_scan) finds the records of a chunk, the device gathers
 the sequences, filters them and assembles ``>name\\nsequence\\n`` of the kept reads in input order, and a writer thread
-appends that to the output.  Host and device memory follow the chunk size, not the input size.  read_sequences() and
+appends that to the output.  Host and device memory follow the chunk size, not the input size.  recruit_file_units is
+the same pipeline for several (unit, output, threshold) jobs: the file is read and scanned once, one filter launch per
+word class covers every unit, and each output gets the bytes recruit_file writes for that job alone (recruit_file is
+its one-job case; main_units / scripts/rr_multi.py is its command line).  read_sequences() and
 recruit() are the in-memory form of the same computation, and the specification the streaming form is tested against.
 """
 import gzip
@@ -296,10 +299,21 @@ def scan_sequences(path, chunk_bytes=CHUNK_BYTES):
 
 def _write_in_memory(unit, read_fn, path, threshold):
     """The whole read set as Python strings, one recruit() call, one write: the form every input can take."""
+    _write_in_memory_jobs(read_fn, [(unit, path, threshold)])
+
+
+def _write_in_memory_jobs(read_fn, jobs):
+    """_write_in_memory for every (unit, path, threshold) of jobs, reading the file once.  Every unit is checked before
+    the first output is written."""
     records = list(read_sequences(read_fn))
-    keep = recruit(unit, [seq for _, seq in records], threshold) if records else np.zeros(0, dtype=bool)
-    with open(path, "w") as f:
-        f.write("".join(f">{name}\n{seq}\n" for (name, seq), k in zip(records, keep.tolist()) if k))
+    if records:
+        for unit, _, _ in jobs:
+            build_masks(unit)
+    seqs = [seq for _, seq in records]
+    for unit, path, threshold in jobs:
+        keep = recruit(unit, seqs, threshold) if records else np.zeros(0, dtype=bool)
+        with open(path, "w") as f:
+            f.write("".join(f">{name}\n{seq}\n" for (name, seq), k in zip(records, keep.tolist()) if k))
 
 
 def recruit_file(unit, read_fn, output_fn, threshold, chunk_bytes=CHUNK_BYTES, engine=None, stats=None):
@@ -311,45 +325,89 @@ def recruit_file(unit, read_fn, output_fn, threshold, chunk_bytes=CHUNK_BYTES, e
     unit; otherwise an invalid unit raises before any output exists.  A chunk with a byte >= 0x80 hands the whole run to
     the in-memory path.  stats: None, or a dict that receives seconds per host stage, device seconds per stage
     (CUDA events, "device_s") and counts."""
-    threshold = int(threshold)
+    return recruit_file_units([(unit, output_fn, threshold)], read_fn, chunk_bytes, engine, stats)
+
+
+def _part_file(output_fn):
+    """A new temporary file beside output_fn -> (path, binary file object)."""
     out_dir, base = os.path.split(os.path.abspath(output_fn))
     i = 0
     while True:
         tmp = os.path.join(out_dir, f".{base}.{os.getpid()}.{i}.part")
         try:
-            f = open(tmp, "xb")
-            break
+            return tmp, open(tmp, "xb")
         except FileExistsError:
             i += 1
+
+
+def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stats=None):
+    """recruit_file for every job (unit, output_fn, threshold) of `jobs` in one pass over read_fn: the file is read,
+    inflated and scanned once, the device filters every chunk for all units in one launch per unit word class, and
+    each output file gets the bytes recruit_file writes for that job alone.  All outputs appear together when the run
+    has finished; on an error none is created or modified.  An input without records gives empty files and checks no
+    unit; otherwise every unit is checked, with recruit_file's errors, before any output exists.  A byte >= 0x80 hands
+    the whole run to the in-memory path (the file is read once, then recruit() per job).  Raises ValueError for no jobs,
+    or for two jobs with the same output file.  Host and device memory follow chunk_bytes times the number of jobs.
+    stats: as in recruit_file, plus "job_out_bytes" (output bytes per job)."""
+    jobs = [(unit, output_fn, int(threshold)) for unit, output_fn, threshold in jobs]
+    if not jobs:
+        raise ValueError("recruit_file_units: no jobs")
+    real = [os.path.realpath(output_fn) for _, output_fn, _ in jobs]
+    if len(set(real)) != len(real):
+        raise ValueError("recruit_file_units: two jobs write the same output file")
     st = {key: 0.0 for key in ("read_s", "assemble_s", "scan_s", "plan_s", "wait_s", "write_s")}
-    st.update(chunks=0, records=0, bases=0, out_bytes=0, fallback=None, device_s=None if stats is None else {})
+    st.update(chunks=0, records=0, bases=0, out_bytes=0, job_out_bytes=[0] * len(jobs), fallback=None,
+              device_s=None if stats is None else {})
+    tmps, files = [], []
     try:
+        for _, output_fn, _ in jobs:
+            tmp, f = _part_file(output_fn)
+            tmps.append(tmp)
+            files.append(f)
         try:
-            with f:
-                _stream(unit, read_fn, f, threshold, chunk_bytes, engine, st)
+            try:
+                _stream([(unit, threshold) for unit, _, threshold in jobs], read_fn, files, chunk_bytes, engine, st)
+            finally:
+                for f in files:
+                    f.close()
         except _Fallback as e:
             st["fallback"] = str(e)
-            _write_in_memory(unit, read_fn, tmp, threshold)
-        os.replace(tmp, output_fn)
+            _write_in_memory_jobs(read_fn, [(unit, tmp, threshold) for (unit, _, threshold), tmp in zip(jobs, tmps)])
+        for tmp, (_, output_fn, _) in zip(tmps, jobs):
+            os.replace(tmp, output_fn)
     except BaseException:
-        if os.path.exists(tmp):
-            os.remove(tmp)
+        for f in files:
+            f.close()
+        for tmp in tmps:
+            if os.path.exists(tmp):
+                os.remove(tmp)
         raise
     if stats is not None:
         stats.update(st)
     return 0
 
 
-def _stream(unit, read_fn, f, threshold, chunk_bytes, engine, st):
-    """recruit_file's pipeline.  While the device works on chunk i, the reader thread reads ahead, this thread scans
-    chunk i + 1, and the writer thread writes chunk i - 1.  Every device step of a chunk is on one stream, so one set
-    of device buffers serves all chunks; host buffers come in two slots (see _scan_chunks) plus two output buffers."""
+def _stream(jobs, read_fn, files, chunk_bytes, engine, st):
+    """recruit_file_units' pipeline: jobs = [(unit, threshold)], files[j] receives job j's output.  While the device
+    works on chunk i, the reader thread reads ahead, this thread scans chunk i + 1, and the writer thread writes chunk
+    i - 1.  Every device step of a chunk is on one stream, so one set of device buffers serves all chunks; host buffers
+    come in two slots (see _scan_chunks) plus two output buffers per job."""
     import torch
     host = {"alloc": lambda n: torch.empty(n, dtype=torch.uint8)}  # pageable until the first record is seen
     dev, out_host = {}, {}
     device_s, events = st["device_s"], []
     eng = d_peq = d_sym = writer = None
-    writer_q, free_out, writer_err = queue.Queue(), queue.Queue(), []
+    writer_q, free_out, writer_err = queue.Queue(), [queue.Queue() for _ in jobs], []
+    # the jobs that run the filter (threshold >= 0; the others keep every read), and their units' rows in d_peq / d_sym
+    filtered = [j for j, (_, threshold) in enumerate(jobs) if threshold >= 0]
+    row = {j: i for i, j in enumerate(filtered)}
+    unit_m = np.array([len(jobs[j][0]) for j in filtered], dtype=np.int32)
+    unit_threshold = np.array([jobs[j][1] for j in filtered], dtype=np.int32)
+    # One segment plan serves every unit.  A hit within t edits spans at most |unit| + t read bases, so it lies wholly
+    # inside some segment whenever the segments overlap by at least that much; and a segment is an infix of its read,
+    # so a hit inside a segment is a hit in the read.  Overlapping by the largest |unit| + t of all jobs therefore
+    # decides every read as recruit()'s plan for each job alone does.
+    overlap = max((len(jobs[j][0]) + jobs[j][1] for j in filtered), default=0)
 
     def mark():
         if device_s is None:
@@ -363,25 +421,28 @@ def _stream(unit, read_fn, f, threshold, chunk_bytes, engine, st):
             item = writer_q.get()
             if item is None:
                 return
-            done, key, nbytes = item
+            done, j, key, nbytes = item
             try:
                 done.synchronize()
                 t0 = time.perf_counter()
-                f.write(memoryview(out_host[key].numpy()[:nbytes]))
+                files[j].write(memoryview(out_host[j, key].numpy()[:nbytes]))
                 st["write_s"] += time.perf_counter() - t0
             except BaseException as e:  # noqa: BLE001 -- raised by the main thread at its next hand-over
                 writer_err.append(e)
-            free_out.put(key)
+            free_out[j].put(key)
 
     def start_device():
         nonlocal eng, d_peq, d_sym, writer
         from .engine import default_engine
         eng = engine or default_engine()
-        peq, sym_of, _ = build_masks(unit)  # raises on an invalid unit, before any output
-        d_peq, d_sym = eng._to_dev(peq.reshape(-1).view(np.int64)), eng._to_dev(sym_of)
+        masks = [build_masks(unit) for unit, _ in jobs]  # raises on an invalid unit, before any output
+        if filtered:
+            d_peq = eng._to_dev(np.concatenate([masks[j][0].reshape(-1) for j in filtered]).view(np.int64))
+            d_sym = eng._to_dev(np.concatenate([masks[j][1] for j in filtered]))
         host["alloc"] = lambda n: torch.empty(n, dtype=torch.uint8, pin_memory=True)
-        for key in (0, 1):
-            free_out.put(key)
+        for q in free_out:
+            for key in (0, 1):
+                q.put(key)
         writer = threading.Thread(target=write_loop, name="rr-writer", daemon=True)
         writer.start()
 
@@ -400,11 +461,11 @@ def _stream(unit, read_fn, f, threshold, chunk_bytes, engine, st):
         upper = int(sizes.sum())
         st["records"] += R
         st["bases"] += int(seq_len.sum())
-        # segments as recruit() plans them; threshold < 0 keeps every read without a filter run.  Host layout, int64:
-        # seg_off[S] | seg_len[S] | seg_ptr[R + 1] (first segment of each record) | order[S] (int32 in the first half)
+        # segments as recruit() plans them (with the overlap above); when no job has threshold >= 0 no filter runs.
+        # Host layout, int64: seg_off[S] | seg_len[S] | seg_ptr[R + 1] (first segment of each record) | order[S] (int32
+        # in the first half)
         S = 0
-        if threshold >= 0:
-            overlap = len(unit) + threshold
+        if filtered:
             n_seg = np.maximum(1, -(-np.maximum(seq_len - overlap, 1) // SEGMENT))
             S = int(n_seg.sum())
             seg_read = np.repeat(np.arange(R, dtype=np.int64), n_seg)
@@ -437,42 +498,52 @@ def _stream(unit, read_fn, f, threshold, chunk_bytes, engine, st):
         c = mark()
         d_keep = seg_ptr = None
         if S:
-            d_keep = dbuf("keep", S)
-            d_keep[:S].zero_()
+            d_keep = dbuf("keep", len(filtered) * S)  # [unit][segment]
+            d_keep[:len(filtered) * S].zero_()
             base = d_seg.data_ptr()
             seg_ptr = base + 16 * S
-            _lib.call("cfk_rr_filter", p(d_text), base, base + 8 * S, base + 8 * (2 * S + R + 1), S, p(d_peq), p(d_sym),
-                      len(unit), threshold, 0, None, p(d_keep), stream)
+            _lib.call("cfk_rr_filter_units", p(d_text), base, base + 8 * S, base + 8 * (2 * S + R + 1), S, len(filtered),
+                      p(d_peq), p(d_sym), unit_m.ctypes.data, unit_threshold.ctypes.data, p(d_keep), stream)
         d = mark()
         d_sizes = dbuf("sizes", 4 * R, torch.int32)
         d_off = dbuf("off", 8 * (R + 1), torch.int64)
         d_scratch = dbuf("scratch", 8 * int(eng.lib.cfk_scan_scratch_elems(R)))
-        d_out = dbuf("out", upper + 16)
-        _lib.call("cfk_rr_keep_sizes", p(d_keep), seg_ptr, p(d_rec), R, p(d_sizes), stream)
-        _lib.call("cfk_exclusive_scan", p(d_sizes), p(d_off), R, p(d_scratch), stream)
-        _lib.call("cfk_rr_emit", p(d_raw), p(d_text), p(d_rec), p(d_off), R, upper, p(d_out), stream)
+        d_totals = dbuf("totals", 8 * len(jobs), torch.int64)
+        d_outs = []
+        for j in range(len(jobs)):  # sizes, offsets and scan scratch are reused: the job's emit has read them by then
+            d_out = dbuf(("out", j), upper + 16)
+            seg_keep = None if j not in row else p(d_keep) + row[j] * S
+            _lib.call("cfk_rr_keep_sizes", seg_keep, None if seg_keep is None else seg_ptr, p(d_rec), R, p(d_sizes), stream)
+            _lib.call("cfk_exclusive_scan", p(d_sizes), p(d_off), R, p(d_scratch), stream)
+            _lib.call("cfk_rr_emit", p(d_raw), p(d_text), p(d_rec), p(d_off), R, upper, p(d_out), stream)
+            d_totals[j:j + 1].copy_(d_off[R:R + 1])
+            d_outs.append(d_out)
         if device_s is not None:
             events.extend((("h2d", a, b), ("gather", b, c), ("filter", c, d), ("emit", d, mark())))
         st["chunks"] += 1
-        return d_off[R], d_out
+        return d_totals[:len(jobs)], d_outs
 
-    def finish(d_total, d_out):
+    def finish(d_totals, d_outs):
         t0 = time.perf_counter()
-        total = int(d_total.item())  # the chunk's one size read-back
-        key = free_out.get()
+        totals = d_totals.tolist()  # the chunk's one size read-back
         st["wait_s"] += time.perf_counter() - t0
-        if writer_err:
-            raise writer_err[0]
-        h = _grown(out_host, key, total, host["alloc"])
-        a = mark()
-        if total:
-            h[:total].copy_(d_out[:total], non_blocking=True)
-        done = torch.cuda.Event()
-        done.record()
-        if device_s is not None:
-            events.append(("d2h", a, mark()))
-        st["out_bytes"] += total
-        writer_q.put((done, key, total))
+        for j, (total, d_out) in enumerate(zip(totals, d_outs)):
+            t0 = time.perf_counter()
+            key = free_out[j].get()
+            st["wait_s"] += time.perf_counter() - t0
+            if writer_err:
+                raise writer_err[0]
+            h = _grown(out_host, (j, key), total, host["alloc"])
+            a = mark()
+            if total:
+                h[:total].copy_(d_out[:total], non_blocking=True)
+            done = torch.cuda.Event()
+            done.record()
+            if device_s is not None:
+                events.append(("d2h", a, mark()))
+            st["out_bytes"] += total
+            st["job_out_bytes"][j] += total
+            writer_q.put((done, j, key, total))
 
     chunks = _scan_chunks(read_fn, chunk_bytes, host, st)
     pending = None
@@ -514,6 +585,28 @@ def main(argv=None):
         threshold = 0  # std::atoi
     unit = next(read_sequences(unit_fn))[1]
     recruit_file(unit, read_fn, output_fn, threshold)
+    return 0
+
+
+UNITS_USAGE = "Usage: rr_multi.py reads.fasta[.gz|.fastq] unit1.fasta output1.fasta threshold1 [unit2.fasta output2.fasta threshold2 ...]"
+
+
+def main_units(argv=None):
+    """``rr_multi.py reads unit1 output1 threshold1 [unit2 output2 threshold2 ...]``: what one rr run per triple writes,
+    from one pass over the read file (recruit_file_units).  Each unit is the first record of its file; thresholds are
+    read as main() reads them.  Wrong argument count: the usage on stderr, status 2."""
+    argv = sys.argv[1:] if argv is None else list(argv)
+    if len(argv) < 4 or (len(argv) - 1) % 3:
+        print(UNITS_USAGE, file=sys.stderr)
+        return 2
+    jobs = []
+    for unit_fn, output_fn, text in zip(argv[1::3], argv[2::3], argv[3::3]):
+        try:
+            threshold = int(text)
+        except ValueError:
+            threshold = 0  # std::atoi, as in main()
+        jobs.append((next(read_sequences(unit_fn))[1], output_fn, threshold))
+    recruit_file_units(jobs, argv[0])
     return 0
 
 

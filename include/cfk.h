@@ -193,6 +193,20 @@ int cfk_rr_filter(const uint8_t* text, const int64_t* read_off, const int64_t* r
                   const uint64_t* peq, const uint8_t* sym_of, int32_t m, int32_t threshold, int32_t exact, int32_t* out_dist,
                   uint8_t* out_keep, cfk_stream_t stream);
 
+/* cfk_rr_filter for U units at once over the same reads (read_recruitment.recruit_file_units): out_keep[u * n_seg + r]
+ * = 1 iff unit u, or its reverse complement, occurs in read r within unit_threshold[u] edits (< 0: no limit).
+ *   peq             each unit's [2][cfk_rr_max_symbols()][cfk_rr_words(unit_m[u])] block (cfk_rr_filter's layout), the
+ *                   blocks of units 0 .. U-1 one after another
+ *   sym_of          [U][256], one symbol table per unit
+ *   unit_m, unit_threshold   HOST int32[U]; they are passed to the kernels by value
+ *   out_keep        [U][n_seg], zeroed by the caller
+ * Every unit_m is checked (1..3328) before anything is launched.  One launch per word class present (more for a
+ * class of more than 64 units), all on `stream`.  The scan of a strand stops early as in cfk_rr_filter (no exact
+ * distances). */
+int cfk_rr_filter_units(const uint8_t* text, const int64_t* seg_off, const int64_t* seg_len, const int32_t* order, int64_t n_seg,
+                        int32_t n_units, const uint64_t* peq, const uint8_t* sym_of, const int32_t* unit_m,
+                        const int32_t* unit_threshold, uint8_t* out_keep, cfk_stream_t stream);
+
 /* ---- streaming read recruitment: read file text in, output file text out ---------------------------------------
  * cfk_seq_scan (HOST code) finds the records of one chunk of FASTA / FASTQ text exactly as read_sequences() yields them
  * (centroflye_b200/read_recruitment.py:29-55, the restatement of rr.cpp's kseq_read loop): "\n", "\r\n" and a lone "\r"

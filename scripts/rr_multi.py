@@ -1,0 +1,11 @@
+"""rr for several units in one pass over the read file: `python rr_multi.py reads.fasta[.gz|.fastq] unit1.fasta
+output1.fasta threshold1 [unit2.fasta output2.fasta threshold2 ...]` writes, for every triple, the file that
+`rr unit.fasta reads output.fasta threshold` writes, reading and scanning the read file once."""
+import os
+import sys
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+from centroflye_b200.read_recruitment import main_units  # noqa: E402
+
+if __name__ == "__main__":
+    sys.exit(main_units())
