@@ -21,9 +21,15 @@ namespace {
 
 using namespace cfk;
 
-__device__ __forceinline__ int64_t pl_upsert(uint64_t* keys, int64_t cap, uint64_t key) {
+// The score tables of placer_update_kernel report a full table through counters[1], and the host repeats the call
+// with 4x larger ones.  One thread walks every occurrence of its pair's k-mer serially, so a full table must not cost
+// it a scan of the whole table per occurrence: probing there stops after PL_MAX_PROBES slots, which reports the table
+// as full (a repeat with larger tables gives the same scores), and a thread stops once any thread reported it.
+constexpr int64_t PL_MAX_PROBES = 1 << 12;
+
+__device__ __forceinline__ int64_t pl_upsert(uint64_t* keys, int64_t cap, uint64_t key, int64_t max_probes) {
   int64_t slot = home_slot(mix64(key), cap);
-  for (int64_t probes = 0; probes < cap; ++probes) {
+  for (int64_t probes = 0; probes < max_probes; ++probes) {
     const uint64_t cur = ((volatile uint64_t*)keys)[slot];
     if (cur == key) return slot;
     if (cur == EMPTY) {
@@ -52,7 +58,7 @@ __global__ void placer_add_read_kernel(const int64_t* __restrict__ unit_ptr, con
   }
   const uint32_t id = ids[e];
   const uint64_t p = (uint64_t)(position + lo);
-  const int64_t slot = pl_upsert(contig_keys, cap, (p << 32) | id);
+  const int64_t slot = pl_upsert(contig_keys, cap, (p << 32) | id, cap);
   if (slot < 0) {
     counters[1] = 1;
     return;
@@ -95,17 +101,25 @@ __global__ void placer_update_kernel(const uint2* __restrict__ pairs, const int6
     const uint2 pr = pairs[i];
     const int64_t cc_pos = pr.y;
     for (int64_t o = occ_ptr[pr.x]; o < occ_ptr[pr.x + 1]; ++o) {
+      if (((volatile int64_t*)counters)[1]) return;  // a table is full: the host discards this call's scores
       const int64_t g = occ[o];
       const int64_t r = unit_read[g];
       if (!read_sel[r]) continue;
       const int64_t pos = g - read_first_unit[r];
       if (cc_pos < pos) continue;
-      const uint64_t off = (uint64_t)(cc_pos - pos);
-      // set of (read, offset, position): read < 2^24, offset < 2^24, position < 2^16 (checked on the host)
-      const uint64_t k1 = ((uint64_t)r << 40) | (off << 16) | (uint64_t)pos;
+      const uint64_t off = (uint64_t)(cc_pos - pos);  // < 2^32: contig positions are (checked in cfk_placer_add_read)
+      // (read, offset) first: read < 2^24 (checked on the host), so the key is exact
+      const int64_t s2 = pl_upsert(m2_keys, cap2, ((uint64_t)r << 32) | off, min(cap2, PL_MAX_PROBES));
+      if (s2 < 0) {
+        counters[1] = 1;
+        continue;
+      }
+      // set of (read, offset, position), keyed by the (read, offset) slot, which never moves within a call:
+      // slot < cap2 < 2^48, position < 2^16 (checked on the host), so the key is exact for any offset
+      const uint64_t k1 = ((uint64_t)s2 << 16) | (uint64_t)pos;
       int64_t slot = home_slot(mix64(k1), cap1);
       bool fresh = false, placed = false;
-      for (int64_t probes = 0; probes < cap1 && !placed; ++probes) {
+      for (int64_t probes = 0, max_probes = min(cap1, PL_MAX_PROBES); probes < max_probes && !placed; ++probes) {
         const uint64_t cur = ((volatile uint64_t*)m1_keys)[slot];
         if (cur == k1) placed = true;
         else if (cur == EMPTY) {
@@ -116,8 +130,7 @@ __global__ void placer_update_kernel(const uint2* __restrict__ pairs, const int6
         }
         if (!placed && ++slot == cap1) slot = 0;
       }
-      const int64_t s2 = placed ? pl_upsert(m2_keys, cap2, ((uint64_t)r << 32) | off) : -1;
-      if (s2 < 0) {
+      if (!placed) {
         counters[1] = 1;
         continue;
       }
@@ -202,7 +215,7 @@ int cfk_placer_update(const uint32_t* pairs, const int64_t* pair_counters, int64
                       const uint32_t* occ, const int32_t* unit_read, const int64_t* read_first_unit, const uint8_t* read_sel,
                       uint64_t* m1_keys, int64_t cap1, uint64_t* m2_keys, uint64_t* m2_val, int64_t cap2, int64_t* counters,
                       cfk_stream_t stream) {
-  if (cap1 < 1 || cap2 < 1 || max_pairs < 0) return fail(CFK_ERR_INVALID, "cfk_placer_update: bad sizes");
+  if (cap1 < 1 || cap2 < 1 || cap2 >= (1ll << 48) || max_pairs < 0) return fail(CFK_ERR_INVALID, "cfk_placer_update: bad sizes");
   if (max_pairs == 0) return CFK_OK;
   const int64_t grid = blocks_for(max_pairs, 128) < 148 * 16 ? blocks_for(max_pairs, 128) : 148 * 16;
   placer_update_kernel<<<(unsigned)grid, 128, 0, (cudaStream_t)stream>>>((const uint2*)pairs, pair_counters, max_pairs, occ_ptr,

@@ -20,7 +20,10 @@ Reference lines followed (relative to /root/reference/scripts):
   dist_counts          distance_based_kmer_recruitment.py:85-128
   filter_edges         distance_based_kmer_recruitment.py:131-149
   result_files         distance_based_kmer_recruitment.py:152-171
+  PlacerModel          read_placer.py:35-94 + cloud_contig.py:26-41,87-95, as centroflye_b200/read_placer.py
+                       and csrc/placer.cu document them (checked against read_positions_<tag>.csv)
 """
+import heapq
 import itertools
 import math
 import re
@@ -126,3 +129,121 @@ def result_files(selected, edges):
     kmers_txt = "".join(kmer + "\n" for kmer in sorted(selected))
     edge_lines = sorted(f"{d} {a} {b} {c}\n" for d, a, b, c in edges)
     return kmers_txt, edge_lines
+
+
+class PlacerContig:
+    """cloud_contig.CloudContig as the placer uses it: (position, k-mer) counters, every position each k-mer was
+    added at, and the k-mers that reached min_cloud_kmer_freq at some position (0 counts as 1)."""
+
+    def __init__(self, min_cloud_kmer_freq):
+        self.min_freq = max(1, min_cloud_kmer_freq)
+        self.cnt = Counter()                # (position, kmer) -> count
+        self.positions = defaultdict(set)   # kmer -> positions it was added at
+        self.freq = set()
+        self.read_positions = {}
+        self.coverage = defaultdict(int)
+        self.max_pos = 0
+        self._last = -1                     # last position any unit was added at
+
+    def add_read(self, clouds, r_id, position):
+        """Adds one read; returns the (kmer, position) pairs whose count reached min_freq just now."""
+        self.read_positions[r_id] = position
+        new = []
+        for i, cloud in enumerate(clouds):
+            p = position + i
+            self.coverage[p] += 1
+            for kmer in cloud:
+                self.cnt[(p, kmer)] += 1
+                self.positions[kmer].add(p)
+                if self.cnt[(p, kmer)] == self.min_freq:
+                    self.freq.add(kmer)
+                    new.append((kmer, p))
+        if len(clouds):
+            self._last = max(self._last, position + len(clouds) - 1)
+        self.max_pos = max(self._last, 0)
+        return new
+
+
+class PlacerModel:
+    """ReadPlacer's greedy loop over plain dicts and sets of k-mer strings.  ``clouds`` maps r_id -> list of unit
+    clouds.  ``lines`` is what read_positions.csv holds after the calls so far; ``decided`` counts, per pick, which
+    level of the selection rule separated the winner from the best other candidate: "alone" (no other candidate),
+    "score" (distinct positions, total), "offset" (the larger offset) or "r_id" (the smaller r_id string)."""
+
+    def __init__(self, min_cloud_kmer_freq):
+        self.contig = PlacerContig(min_cloud_kmer_freq)
+        self.lines = []
+        self.decided = Counter()
+        self.scores = {}   # (r_id, offset) -> [distinct positions, total] of the last add_reads call
+
+    def add_prefix_reads(self, prefix_reads, clouds):
+        self.lines = []    # the file is rewritten
+        for r_id in prefix_reads:
+            self.contig.add_read(clouds[r_id], r_id, 0)
+            self.lines.append(f"{r_id} 0")
+
+    @staticmethod
+    def _passes(distinct, total, min_unit, min_inters, min_prop):
+        return distinct >= min_unit and total >= min_inters and total >= min_prop * distinct
+
+    def add_reads(self, reads, clouds, min_unit, min_inters, min_prop=3):
+        kmers2pos = defaultdict(list)
+        for r_id in reads:
+            for pos, cloud in enumerate(clouds[r_id]):
+                for kmer in cloud:
+                    kmers2pos[kmer].append((r_id, pos))
+        seen = set()       # (r_id, offset, position in read)
+        scores = self.scores = {}
+        # candidates of unused reads, largest first; an entry is stale once its scores have moved on
+        heap = []
+        unused = set(reads)
+        pairs = [(kmer, p) for kmer in self.contig.freq for p in self.contig.positions[kmer]]
+        while unused:
+            touched = set()
+            for kmer, cc_pos in pairs:
+                for r_id, pos in kmers2pos.get(kmer, ()):
+                    if cc_pos < pos:
+                        continue
+                    off = cc_pos - pos
+                    sc = scores.setdefault((r_id, off), [0, 0])
+                    if (r_id, off, pos) not in seen:
+                        seen.add((r_id, off, pos))
+                        sc[0] += 1
+                    sc[1] += 1
+                    touched.add((r_id, off))
+            for r_id, off in touched:
+                d, t = scores[(r_id, off)]
+                if r_id in unused and self._passes(d, t, min_unit, min_inters, min_prop):
+                    heapq.heappush(heap, (-d, -t, -off, r_id))
+            best = self._pop(heap, scores, unused)
+            if best is None:
+                self.lines += [f"{r_id} None" for r_id in reads if r_id in unused]
+                return
+            runner_up = self._pop(heap, scores, unused)
+            if runner_up is None:
+                self.decided["alone"] += 1
+            else:
+                heapq.heappush(heap, runner_up)
+                level = "score" if runner_up[:2] != best[:2] else "offset" if runner_up[2] != best[2] else "r_id"
+                self.decided[level] += 1
+            d, t, off, r_id = -best[0], -best[1], -best[2], best[3]
+            self.lines.append(f"{r_id} {off} {d} {t}")
+            unused.discard(r_id)
+            pairs = self.contig.add_read(clouds[r_id], r_id, off)
+
+    @staticmethod
+    def _pop(heap, scores, unused):
+        while heap:
+            e = heapq.heappop(heap)
+            if e[3] in unused and scores[(e[3], -e[2])] == [-e[0], -e[1]]:
+                return e
+        return None
+
+
+def place_reads(prefix, internal, suffix, clouds, min_cloud_kmer_freq, min_unit, min_inters, min_prop=3):
+    """ReadPlacer.run after classification: prefix reads, then internal reads, then suffix reads."""
+    model = PlacerModel(min_cloud_kmer_freq)
+    model.add_prefix_reads(prefix, clouds)
+    model.add_reads(internal, clouds, min_unit, min_inters, min_prop)
+    model.add_reads(suffix, clouds, min_unit, min_inters, min_prop)
+    return model
