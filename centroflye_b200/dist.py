@@ -21,8 +21,8 @@ import os
 
 import numpy as np
 
-from . import _lib
 from ._lib import CfkError
+from .engine import stream_counters
 
 U32_MAX = 0xFFFFFFFF
 _GOLDEN = np.uint64(0x9E3779B97F4A7C15)
@@ -225,52 +225,38 @@ class ShardedRecruiter:
             return eng._empty(0, t.int64)[:0]
         n_parts, part_cap = eng.stream_plan(self.n_kmers_total, self.reads.n_reads, n_ranks=W,
                                             n_kmers_local=self.n_kmers_local)
-        per = n_parts // W
-        for attempt in range(3):
+        for launches in (1, 2, 3):
             records, cursors, ecounters = eng.emit_records(self.reads, self.k, n_parts, part_cap)
             with eng._stage("exchange_pack"):
                 counts = cursors.clamp(max=part_cap)
                 offsets, _ = padded_run_offsets(counts, W, eng.exclusive_scan)
-                send = eng._empty(self.n_kmers_local + RUN_ALIGN * W, t.int64)  # records <= k-mer occurrences
-                _lib.call("cfk_records_pack", eng._p(records), part_cap, eng._p(counts), eng._p(offsets), n_parts,
-                          eng._p(send), eng._stream())
+                send = eng.pack_records(records, part_cap, counts, offsets,
+                                        self.n_kmers_local + RUN_ALIGN * W)  # records <= k-mer occurrences
             with eng._stage("exchange_docfreq"):
                 recv, recv_counts, flags, n_sent = exchange_records(send, counts, W, self.group,
                                                                     flags=eng.emit_stats(cursors, ecounters))
             self.bytes_exchanged += 8 * n_sent + 4 * n_parts
-            if flags[1]:
-                raise CfkError("stage A: per-read k-mer set overflowed (internal error)")
-            if not flags[0]:
+            s = stream_counters(emit=flags)  # all-reduced: every rank takes the same branch
+            if not s.emit_overflow:
                 break
-            biggest = int(cursors.max().item())  # some rank ran out of room: all ranks go again with what they measured
-            eng.part_cap_seen[n_parts] = max(eng.part_cap_seen.get(n_parts, 0), biggest)
-            part_cap = max(part_cap, int(biggest * 1.05) + 256)
+            part_cap = eng.grow_part_cap(n_parts, s.biggest_part, launches)  # some rank ran out of room: all go again
             del records, send, recv
-        else:
-            raise CfkError("stage A: partition buffers overflowed three times (internal error)")
         roff, _ = padded_run_offsets(recv_counts, W, eng.exclusive_scan)
-        band = (lo, hi, max_nonuniq)
-        out = eng.finish_count(lambda counters: eng.count_records(recv, recv_counts, per, 1, self.k, band, n_src=W,
-                                                                  offsets=roff, counters=counters, group=eng.stream_group),
-                               band, False)
+        h = eng.docfreq_count_launch(recv, recv_counts, n_parts // W, 1, self.k, (lo, hi, max_nonuniq), n_src=W,
+                                     offsets=roff)
+        out = eng.docfreq_stream_finish(h)
         ok = t.tensor([0 if out is None else 1], dtype=t.int64, device=eng.device)
         self.dist.all_reduce(ok, op=self.dist.ReduceOp.MIN, group=self.group)
         if int(ok.item()) == 0:
             return None
-        mine, c = out
-        eng._adapt_stream_group(int(c[5]), per, int(c[6]))
         with eng._stage("exchange_rare"):
             # every rank sorts its own keys; the gathered runs (distinct keys: a k-mer has one owner) are merged by rank
-            mine = eng.sort_keys(mine.contiguous().clone()) if mine.numel() > 1 else mine.contiguous()
+            mine = eng.sort_keys(out[0].clone()) if out[0].numel() > 1 else out[0].contiguous()
             allk, counts = all_gather_v(mine, self.group)
             self.bytes_exchanged += 8 * int(mine.numel())
             if allk.numel() == 0:
                 return allk
-            run_ptr = eng._to_dev(np.concatenate([[0], np.cumsum(np.asarray(counts, dtype=np.int64))]))
-            merged = eng._empty(int(allk.numel()), t.int64)
-            _lib.call("cfk_merge_sorted_runs", eng._p(allk.contiguous()), eng._p(run_ptr), W, int(allk.numel()),
-                      eng._p(merged), eng._stream())
-        return merged[: int(allk.numel())]
+            return eng.merge_sorted_runs(allk, counts)
 
     def global_rare_keys(self, table, lo, hi, max_nonuniq):
         """Local table -> sorted rare keys of the WHOLE read set (identical on every rank).

@@ -13,6 +13,7 @@ There is no CPU fallback: constructing an Engine without CUDA or without libcfk.
 import contextlib
 import math
 import os
+from collections import namedtuple
 from dataclasses import dataclass
 
 import numpy as np
@@ -60,6 +61,23 @@ class DocFreqTable:
     slots: object       # int64[2 * cap]: per slot (key as uint64 bits, -1 = empty ; n_reads | n_multi << 32)
     cap: int
     dense: bool = False  # True: every slot is occupied and in no particular order (two-phase stage A): scans only
+
+
+StreamCounters = namedtuple("StreamCounters", "unfit n_rare n_distinct n_retried emit_overflow biggest_part")
+
+
+def stream_counters(c=(), emit=()):
+    """Host int64 values of two-phase stage A -> StreamCounters; the only code that knows where each value sits.
+    c = the counters of cfk_docfreq_count_parts (include/cfk.h: a partition did not fit, internal error, -, -, rare
+    k-mers found, distinct k-mers, units retried), optionally followed by Engine.emit_stats (the one readback of a
+    launch); emit = emit_stats alone (the sharded path's all-reduced phase-1 flags).  Internal errors raise."""
+    unfit, internal, _, _, n_rare, n_distinct, n_retried, _, *tail = [int(x) for x in c] or [0] * 8
+    emit_overflow, emit_internal, biggest_part = tail or [int(x) for x in emit] or [0, 0, 0]
+    if internal:
+        raise CfkError("stage A: phase 2 reported an internal error")
+    if emit_internal:
+        raise CfkError("stage A: per-read k-mer set overflowed (internal error)")
+    return StreamCounters(unfit, n_rare, n_distinct, n_retried, emit_overflow, biggest_part)
 
 
 @dataclass
@@ -118,6 +136,7 @@ class Engine:
         self.part_slack = 1.25  # records per partition buffer / expected records per partition (stream mode)
         self.stream_group = 1   # partitions per phase-2 unit; adapted after every call (_adapt_stream_group)
         self.part_cap_seen = {}  # n_parts -> largest partition (records) phase 1 produced so far
+        self.stream_fallbacks = 0  # two-phase calls that handed stage A to the single-kernel form
         self._stat_pool, self._stat_next = [], 0  # pinned result slots of docfreq_stream_launch
         self.events = None  # set to a list to collect (stage, start_event, end_event) per C-ABI call group
         self._host_pool = {}  # name -> pinned uint8 buffer for results (to_host)
@@ -364,7 +383,7 @@ class Engine:
         return records, cursors, counters
 
     def count_records(self, records, cursors, n_parts, part_cap, k, band=None, with_counts=False, dense=None,
-                      n_src=1, src_stride=0, offsets=None, counters=None, group=1):
+                      n_src=1, src_stride=0, offsets=None, group=1):
         """Phase 2 over n_parts partitions -> (rare_keys, rare_nreads, rare_nmulti, counters, max_rare); the rare
         outputs are None without a band.  `dense` (int64[2 * max_dense]) receives the whole table when given."""
         t = self.torch
@@ -374,7 +393,7 @@ class Engine:
         rare = self._empty(max_rare, t.int64) if band is not None else None
         rare_nr = self._empty(max_rare, t.int32) if band is not None and with_counts else None
         rare_nm = self._empty(max_rare, t.int32) if band is not None and with_counts else None
-        counters = self._counters() if counters is None else counters
+        counters = self._counters()
         with self._stage("docfreq_count"):
             _lib.call("cfk_docfreq_count_parts", self._p(records), part_cap, self._p(cursors), self._p(offsets), n_parts,
                       n_src, src_stride, int(group), int(k), int(lo), int(min(hi, U32_MAX)), int(min(mn, U32_MAX)),
@@ -392,38 +411,18 @@ class Engine:
             group = max(1, min(group, self.stream_group // 2))
         self.stream_group = group
 
-    def finish_count(self, run_count, band, with_counts, extra=None):
-        """Runs phase 2 (run_count(counters) -> the tuple of count_records) until its rare output fits; ONE host sync
-        per run brings its counters (and `extra`, a small int64 device tensor, appended).  Returns (rare outputs, host
-        counters + extra) or None when a partition did not fit phase 2 at all."""
-        t = self.torch
-        counters = self._counters()
-        while True:
-            rare, rare_nr, rare_nm, counters, max_rare = run_count(counters)
-            c = (counters if extra is None else t.cat([counters, extra])).cpu()
-            if int(c[1]):
-                raise CfkError("stage A: shared-memory set overflowed (internal error)")
-            if extra is not None and int(c[8]):
-                return "emit-overflow", c  # phase 1 ran out of room: these results are void
-            if int(c[0]):
-                self.stream_fallbacks = getattr(self, "stream_fallbacks", 0) + 1
-                return None
-            n_rare = int(c[4])
-            if band is None or n_rare <= max_rare:
-                break
-            self.select_hint[("stream", bool(with_counts))] = n_rare + 1024  # the size is now known: phase 2 again
-            counters = self._counters()
-        if band is None:
-            return None, c
-        self.select_hint[("stream", bool(with_counts))] = max(max_rare, int(n_rare * 1.05) + 1024)
-        if with_counts:
-            return (rare[:n_rare], rare_nr[:n_rare], rare_nm[:n_rare]), c
-        return rare[:n_rare], c
-
     def emit_stats(self, cursors, counters):
         """int64[3] device tensor: phase 1's overflow flag, its internal-error flag, its largest partition."""
         t = self.torch
         return t.stack([counters[0], counters[1], cursors.max().to(t.int64)])
+
+    def grow_part_cap(self, n_parts, biggest, launches):
+        """Phase 1 overflowed on its `launches`-th launch and needed `biggest` records in its largest partition -> the
+        part_cap to launch it again with.  Later plans start from the largest size seen (stream_plan)."""
+        if launches >= 3:
+            raise CfkError("stage A: partition buffers overflowed three times (internal error)")
+        self.part_cap_seen[n_parts] = max(self.part_cap_seen.get(n_parts, 0), biggest)
+        return int(biggest * 1.05) + 256
 
     def docfreq_stream(self, reads, k, band=None, with_counts=False, want_table=False, table_buf=None):
         """Two-phase stage A on one GPU -> (rare, table) or None when phase 2 could not hold a partition (more than
@@ -432,86 +431,91 @@ class Engine:
         count tensors when with_counts); table = the dense DocFreqTable when want_table.  One host sync at the end
         (two when the table is wanted and no table_buf -- int64[2 * slots], at least one slot per k-mer occurrence --
         is given: its size then comes from phase 1)."""
-        t = self.torch
-        total_k = max(reads.n_bases - reads.n_reads * (k - 1), 0)
-        n_parts, part_cap = self.stream_plan(total_k, reads.n_reads)
-        for attempt in range(3):
-            records, cursors, ecounters = self.emit_records(reads, k, n_parts, part_cap)
-            dense = table_buf if want_table else None
-            if want_table and dense is None:
-                n_rec = int(cursors.clamp(max=part_cap).sum(dtype=t.int64).item())  # distinct k-mers <= records
-                dense = self._empty(2 * max(n_rec, 1), t.int64)
-            out = self.finish_count(lambda counters: self.count_records(records, cursors, n_parts, part_cap, k, band,
-                                                                        with_counts, dense, counters=counters,
-                                                                        group=self.stream_group),
-                                    band, with_counts, extra=self.emit_stats(cursors, ecounters))
-            if out is None:
-                return None
-            rare, c = out
-            if int(c[9]):
-                raise CfkError("stage A: per-read k-mer set overflowed (internal error)")
-            biggest = int(c[10])
-            self.part_cap_seen[n_parts] = max(self.part_cap_seen.get(n_parts, 0), biggest)
-            if not (isinstance(rare, str) and rare == "emit-overflow"):
-                break
-            del records  # a partition buffer was too small: once more with the size phase 1 measured
-            part_cap = int(biggest * 1.05) + 256
-        else:
-            raise CfkError("stage A: partition buffers overflowed three times (internal error)")
-        self._adapt_stream_group(int(c[5]), n_parts, int(c[6]))
-        table = None
-        if want_table:
-            n = int(c[5])
-            table = DocFreqTable(slots=dense[:2 * n], cap=n, dense=True)
-        return rare, table
+        return self.docfreq_stream_finish(self._stream_launch(reads, k, band, with_counts, want_table, table_buf))
 
-    # -- the same two kernels without a host round trip per batch (streams of independent batches)
     def docfreq_stream_launch(self, reads, k, band=None, with_counts=False, table_buf=None):
         """Enqueue both phases of stage A for one batch and return a handle; nothing is read back yet, so the next
         batch can be enqueued behind it.  docfreq_stream_finish(handle) waits for THIS batch's counters only."""
+        return self._stream_launch(reads, k, band, with_counts, table_buf is not None, table_buf)
+
+    def _stream_launch(self, reads, k, band, with_counts, want_table, table_buf):
+        n_parts, part_cap = self.stream_plan(max(reads.n_bases - reads.n_reads * (k - 1), 0), reads.n_reads)
+        h = dict(reads=reads, k=k, band=band, with_counts=with_counts, want_table=want_table,
+                 table_buf=table_buf if want_table else None, n_parts=n_parts, n_src=1, offsets=None, launches=0)
+        return self._stream_emit(h, part_cap)
+
+    def _stream_emit(self, h, part_cap):
+        """Phase 1 of a handle (again after an overflow, with a larger part_cap), then its phase 2."""
+        h.update(records=None, dense=None, rare=None)  # a repeat lets go of the buffers that were too small first
+        records, cursors, counters = self.emit_records(h["reads"], h["k"], h["n_parts"], part_cap)
+        dense = h["table_buf"]
+        if h["want_table"] and dense is None:
+            n_rec = int(cursors.clamp(max=part_cap).sum(dtype=self.torch.int64).item())  # distinct k-mers <= records
+            dense = self._empty(2 * max(n_rec, 1), self.torch.int64)
+        h.update(records=records, cursors=cursors, part_cap=part_cap, dense=dense,
+                 emit=self.emit_stats(cursors, counters), launches=h["launches"] + 1)
+        return self._stream_count(h)
+
+    def docfreq_count_launch(self, records, cursors, n_parts, part_cap, k, band, n_src=1, offsets=None):
+        """Phase 2 alone, on records the multi-GPU exchange delivered -> a handle for docfreq_stream_finish."""
+        return self._stream_count(dict(records=records, cursors=cursors, n_parts=n_parts, part_cap=part_cap, k=k,
+                                       band=band, with_counts=False, dense=None, n_src=n_src, offsets=offsets, emit=None))
+
+    def _stream_count(self, h):
+        """Phase 2 on the records the handle keeps; its counters (+ phase 1's emit_stats, if it ran) go home."""
+        rare, rare_nr, rare_nm, counters, h["max_rare"] = self.count_records(
+            h["records"], h["cursors"], h["n_parts"], h["part_cap"], h["k"], h["band"], h["with_counts"], h["dense"],
+            n_src=h["n_src"], offsets=h["offsets"], group=self.stream_group)
+        h["rare"] = (rare, rare_nr, rare_nm)
+        self._readback(h, counters if h["emit"] is None else self.torch.cat([counters, h["emit"]]))
+        return h
+
+    def _readback(self, h, stats):
+        """stats (<= 16 int64 on the device) -> h["host"], pinned, once h["done"] (an event) has completed."""
         t = self.torch
-        total_k = max(reads.n_bases - reads.n_reads * (k - 1), 0)
-        n_parts, part_cap = self.stream_plan(total_k, reads.n_reads)
-        records, cursors, ecounters = self.emit_records(reads, k, n_parts, part_cap)
-        counters = self._counters()
-        rare, rare_nr, rare_nm, counters, max_rare = self.count_records(
-            records, cursors, n_parts, part_cap, k, band, with_counts, table_buf, counters=counters, group=self.stream_group)
-        stats = t.cat([counters, self.emit_stats(cursors, ecounters)])
-        if not self._stat_pool:  # page-locking costs far more than the copy: a small ring of pinned slots
-            self._stat_pool = [t.empty(16, dtype=t.int64, pin_memory=True) for _ in range(8)]
-        host = self._stat_pool[self._stat_next % len(self._stat_pool)][: stats.numel()]
-        self._stat_next += 1
-        host.copy_(stats, non_blocking=True)
-        done = t.cuda.Event()
-        done.record(t.cuda.current_stream(self.device))
-        return dict(reads=reads, k=k, band=band, with_counts=with_counts, table_buf=table_buf, n_parts=n_parts,
-                    rare=(rare, rare_nr, rare_nm), max_rare=max_rare, host=host, done=done, keep=(records, cursors))
+        if "host" not in h:  # one slot of a small pinned ring per handle (page-locking costs far more than the copy)
+            self._stat_pool = self._stat_pool or [t.empty(16, dtype=t.int64, pin_memory=True) for _ in range(8)]
+            h["host"] = self._stat_pool[self._stat_next % len(self._stat_pool)][: stats.numel()]
+            self._stat_next += 1
+        h["host"].copy_(stats, non_blocking=True)
+        h["done"] = t.cuda.Event()
+        h["done"].record(t.cuda.current_stream(self.device))
 
     def docfreq_stream_finish(self, h):
-        """-> (rare, table) of a launched batch, like docfreq_stream.  A batch whose buffers turned out too small (its
-        first of a kind, usually) is simply done again through the synchronous path."""
-        h["done"].synchronize()
-        c = h["host"]
-        if int(c[1]) or int(c[9]):
-            raise CfkError("stage A: shared-memory set overflowed (internal error)")
-        self.part_cap_seen[h["n_parts"]] = max(self.part_cap_seen.get(h["n_parts"], 0), int(c[10]))
-        n_rare = int(c[4])
-        if int(c[8]) or int(c[0]) or (h["band"] is not None and n_rare > h["max_rare"]):
-            if h["band"] is not None and n_rare > h["max_rare"]:
-                self.select_hint[("stream", bool(h["with_counts"]))] = n_rare + 1024
-            return self.docfreq_stream(h["reads"], h["k"], band=h["band"], with_counts=h["with_counts"],
-                                       want_table=h["table_buf"] is not None, table_buf=h["table_buf"])
-        self._adapt_stream_group(int(c[5]), h["n_parts"], int(c[6]))
-        table = None
-        if h["table_buf"] is not None:
-            n = int(c[5])
-            table = DocFreqTable(slots=h["table_buf"][:2 * n], cap=n, dense=True)
+        """-> (rare, table) of a launched batch, like docfreq_stream.  Waits for this batch's counters only.  A phase 1
+        that ran out of partition buffer is launched again with the size it measured (three launches in all at most);
+        a rare output that was too small gets phase 2 again, on the records the handle keeps."""
+        while True:
+            h["done"].synchronize()
+            s = stream_counters(h["host"])
+            if s.emit_overflow:  # what phase 2 reported is void
+                self._stream_emit(h, self.grow_part_cap(h["n_parts"], s.biggest_part, h["launches"]))
+            elif s.unfit:
+                self.stream_fallbacks += 1
+                return None
+            elif h["band"] is not None and s.n_rare > h["max_rare"]:
+                self.select_hint[("stream", bool(h["with_counts"]))] = s.n_rare + 1024  # the size is now known
+                self._stream_count(h)
+            else:
+                break
+        if h["emit"] is not None:
+            self.part_cap_seen[h["n_parts"]] = max(self.part_cap_seen.get(h["n_parts"], 0), s.biggest_part)
+        self._adapt_stream_group(s.n_distinct, h["n_parts"], s.n_retried)
+        n = s.n_distinct
+        table = None if h["dense"] is None else DocFreqTable(slots=h["dense"][:2 * n], cap=n, dense=True)
         if h["band"] is None:
             return None, table
-        rare, rare_nr, rare_nm = h["rare"]
-        if h["with_counts"]:
-            return (rare[:n_rare], rare_nr[:n_rare], rare_nm[:n_rare]), table
-        return rare[:n_rare], table
+        self.select_hint[("stream", bool(h["with_counts"]))] = max(h["max_rare"], int(s.n_rare * 1.05) + 1024)
+        rare = tuple(x[:s.n_rare] for x in h["rare"] if x is not None)
+        return (rare if h["with_counts"] else rare[0]), table
+
+    def pack_records(self, records, part_cap, counts, offsets, n_out):
+        """Phase 1's partition buffers -> int64[n_out] holding partition p's counts[p] records from offsets[p] on
+        (cfk_records_pack)."""
+        out = self._empty(n_out, self.torch.int64)
+        _lib.call("cfk_records_pack", self._p(records), part_cap, self._p(counts), self._p(offsets), int(counts.numel()),
+                  self._p(out), self._stream())
+        return out
 
     def count_total(self, reads, batch, k, canonical=False):
         """Total occurrences of every k-mer over all reads (no per-read de-duplication) -> DocFreqTable whose n_reads
@@ -601,6 +605,15 @@ class Engine:
         keys = keys.contiguous()
         _lib.call("cfk_sort_u64", self._p(keys), int(keys.numel()), self._stream())
         return keys
+
+    def merge_sorted_runs(self, keys, counts):
+        """Back-to-back sorted runs of distinct keys, counts[r] keys in run r -> one sorted tensor (cfk_merge_sorted_runs)."""
+        n = int(keys.numel())
+        run_ptr = self._to_dev(np.concatenate([[0], np.cumsum(np.asarray(counts, dtype=np.int64))]))
+        merged = self._empty(n, self.torch.int64)
+        _lib.call("cfk_merge_sorted_runs", self._p(keys.contiguous()), self._p(run_ptr), len(counts), n, self._p(merged),
+                  self._stream())
+        return merged[:n]
 
     def build_index(self, keys, presorted=False):
         t = self.torch

@@ -33,6 +33,24 @@ def _dataset():
     return unit, reads, batch_from_synth
 
 
+KEY_BITS = np.uint64((1 << 62) - 1)
+
+
+def _records_np(batch, k):
+    """What cfk_docfreq_emit produces, restated: one record per distinct k-mer of a read, bit 63 = seen twice in it."""
+    from oracle import c_oracle
+    codes = c_oracle.unpacked_codes(batch)
+    recs = []
+    for r in range(batch.n_reads):
+        seq = codes[int(batch.read_off[r]): int(batch.read_off[r]) + int(batch.read_len[r])].astype(np.uint64)
+        km = np.zeros(seq.size - k + 1, dtype=np.uint64)
+        for j in range(k):
+            km = (km << np.uint64(2)) | seq[j: seq.size - k + 1 + j]
+        u, c = np.unique(km, return_counts=True)
+        recs.append(u | ((c > 1).astype(np.uint64) << np.uint64(63)))
+    return np.concatenate(recs)
+
+
 def _worker(rank, world, port, out_dir):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -81,17 +99,8 @@ def _worker(rank, world, port, out_dir):
         # what cfk_docfreq_emit produces is restated with numpy (one record per distinct k-mer of a read, bit 63 = seen
         # twice in that read, partition = hash range); the exchange itself is the product code (cdist.exchange_records)
         n_parts = 6 * world
-        my_codes = c_oracle.unpacked_codes(my_batch)
-        recs = []
-        for r in range(my_batch.n_reads):
-            seq = my_codes[int(my_batch.read_off[r]): int(my_batch.read_off[r]) + int(my_batch.read_len[r])].astype(np.uint64)
-            km = np.zeros(seq.size - k + 1, dtype=np.uint64)
-            for j in range(k):
-                km = (km << np.uint64(2)) | seq[j: seq.size - k + 1 + j]
-            u, c = np.unique(km, return_counts=True)
-            recs.append(u | ((c > 1).astype(np.uint64) << np.uint64(63)))
-        recs = np.concatenate(recs)
-        key_bits = np.uint64((1 << 62) - 1)
+        recs = _records_np(my_batch, k)
+        key_bits = KEY_BITS
         part = (cdist.mix64_np(recs & key_bits) % np.uint64(n_parts)).astype(np.int64)
         by_part = np.argsort(part, kind="stable")
         counts = torch.from_numpy(np.bincount(part, minlength=n_parts).astype(np.int32))
@@ -223,6 +232,117 @@ def _worker(rank, world, port, out_dir):
 @pytest.mark.parametrize("world", [2, 3])
 def test_sharded_exchange(tmp_path, world):
     mp.spawn(_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
+    assert all(os.path.exists(tmp_path / f"ok{r}") for r in range(world))
+
+
+def _stage_a_engine(recs, calls, unfit=False):
+    """An Engine whose device steps of two-phase stage A are restated with numpy on CPU tensors; stream_plan,
+    _adapt_stream_group, grow_part_cap and docfreq_stream_finish are the product's.  calls receives the part_cap of every
+    phase-1 launch; unfit: phase 2 reports a partition that did not fit."""
+    import types
+    from centroflye_b200.dist import mix64_np
+    from centroflye_b200.engine import Engine
+    eng = object.__new__(Engine)
+    eng.torch, eng.device, eng.events = torch, torch.device("cpu"), None
+    eng.lib = types.SimpleNamespace(cfk_docfreq_part_target=lambda: 20000, cfk_docfreq_part_distinct=lambda: 6144)
+    eng.part_slack, eng.stream_group, eng.part_cap_seen, eng.select_hint, eng.stream_fallbacks = 1.25, 1, {}, {}, 0
+
+    def emit_records(reads, k, n_parts, part_cap):  # cfk_docfreq_emit: records[p * part_cap + i], i < cursors[p]
+        calls.append(part_cap)
+        part = (mix64_np(recs & KEY_BITS) % np.uint64(n_parts)).astype(np.int64)
+        need = np.bincount(part, minlength=n_parts)
+        records = np.full(n_parts * part_cap, -1, dtype=np.int64)
+        for p in range(n_parts):
+            mine = recs[part == p][:part_cap].view(np.int64)
+            records[p * part_cap: p * part_cap + mine.size] = mine
+        counters = torch.zeros(8, dtype=torch.int64)
+        counters[0] = int(need.max() > part_cap)
+        return torch.from_numpy(records), torch.from_numpy(need.astype(np.int32)), counters
+
+    def pack_records(records, part_cap, counts, offsets, n_out):  # cfk_records_pack
+        out = torch.full((n_out,), -1, dtype=torch.int64)
+        for p, (c, o) in enumerate(zip(counts.tolist(), offsets.tolist())):
+            out[o: o + c] = records[p * part_cap: p * part_cap + c]
+        return out
+
+    def count_records(records, cursors, n_parts, part_cap, k, band=None, with_counts=False, dense=None, n_src=1,
+                      src_stride=0, offsets=None, group=1):  # cfk_docfreq_count_parts over the runs of every source
+        got = np.concatenate([records[o: o + c].numpy() for c, o in zip(cursors.tolist(), offsets.tolist())])
+        got = got.view(np.uint64)
+        keys, inv = np.unique(got & KEY_BITS, return_inverse=True)
+        nr = np.bincount(inv, minlength=keys.size)
+        nm = np.bincount(inv, weights=(got >> np.uint64(63)).astype(np.float64), minlength=keys.size)
+        lo, hi, mn = band
+        rare = keys[(nm <= mn) & (nr >= lo) & (nr <= hi)].view(np.int64)
+        max_rare = int(eng.select_hint.get(("stream", False), 1 << 20))
+        out = torch.zeros(max(max_rare, 1), dtype=torch.int64)
+        out[: min(rare.size, max_rare)] = torch.from_numpy(rare[:max_rare])
+        counters = torch.tensor([int(unfit), 0, 0, 0, rare.size, keys.size, 0, 0], dtype=torch.int64)
+        return out, None, None, counters, max_rare
+
+    def readback(h, stats):  # the pinned copy and its event
+        h["host"], h["done"] = stats.clone(), types.SimpleNamespace(synchronize=lambda: None)
+
+    eng.emit_records, eng.pack_records, eng.count_records, eng._readback = emit_records, pack_records, count_records, readback
+    eng.exclusive_scan = lambda c: torch.cat([torch.zeros(1, dtype=torch.int64), torch.cumsum(c.to(torch.int64), 0)])
+    eng.sort_keys = lambda keys: torch.from_numpy(np.sort(keys.numpy().view(np.uint64)).view(np.int64))
+    eng.merge_sorted_runs = lambda keys, counts: eng.sort_keys(keys)  # cfk_merge_sorted_runs: runs of distinct keys
+    return eng
+
+
+def _rare_stream_worker(rank, world, port, out_dir):
+    """ShardedRecruiter.global_rare_stream itself, its device steps restated (_stage_a_engine): the same rare set on
+    every rank, also after one rank's phase 1 overflowed; all ranks fall back together when one rank's phase 2 cannot."""
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    try:
+        import types
+        from centroflye_b200 import dist as cdist
+        from oracle import c_oracle
+        unit, reads, batch_from_synth = _dataset()
+        k, lo, hi, max_nonuniq = 15, 3, 12, 2
+        whole_batch, _ = batch_from_synth(reads, len(unit))
+        gk, gr, gm = c_oracle.docfreq(c_oracle.unpacked_codes(whole_batch), whole_batch, k)
+        want_rare = gk[(gm <= max_nonuniq) & (gr >= lo) & (gr <= hi)]
+        my_batch, _ = batch_from_synth(reads[rank::world], len(unit))
+        recs = _records_np(my_batch, k)
+        n_local = int(np.maximum(my_batch.read_len - k + 1, 0).sum())
+        n_total = torch.tensor([n_local])
+        dist.all_reduce(n_total)
+        for case in ("plain", "emit_overflow", "unfit"):
+            calls = []
+            eng = _stage_a_engine(recs, calls, unfit=case == "unfit" and rank == world - 1)
+            if case == "emit_overflow" and rank == 1:  # this rank's first partition buffers are far too small
+                plan = eng.stream_plan
+                eng.stream_plan = lambda *a, **kw: (plan(*a, **kw)[0], 64)
+            sr = object.__new__(cdist.ShardedRecruiter)
+            sr.eng, sr.torch, sr.dist, sr.world, sr.rank, sr.group, sr.k = eng, torch, dist, world, rank, None, k
+            sr.reads, sr.n_kmers_local, sr.n_kmers_total = types.SimpleNamespace(n_reads=my_batch.n_reads), n_local, int(n_total)
+            sr.bytes_exchanged = 0
+            got = sr.global_rare_stream(lo, hi, max_nonuniq)
+            n_parts = eng.stream_plan(int(n_total), my_batch.n_reads, n_ranks=world, n_kmers_local=n_local)[0]
+            assert n_parts >= 2 * world
+            if case == "unfit":
+                assert got is None and len(calls) == 1 and eng.stream_fallbacks == int(rank == world - 1)
+                continue
+            assert np.array_equal(got.numpy().view(np.uint64), want_rare) and want_rare.size > 50
+            assert eng.stream_fallbacks == 0
+            if case == "plain":
+                assert len(calls) == 1 and eng.part_cap_seen == {}
+            else:  # every rank went again, with the largest partition of all ranks, and remembers it
+                part = (cdist.mix64_np(recs & KEY_BITS) % np.uint64(n_parts)).astype(np.int64)
+                biggest = torch.tensor([int(np.bincount(part, minlength=n_parts).max())])
+                dist.all_reduce(biggest, op=dist.ReduceOp.MAX)
+                assert len(calls) == 2 and calls[1] == int(int(biggest) * 1.05) + 256
+                assert eng.part_cap_seen == {n_parts: int(biggest)}
+        open(os.path.join(out_dir, f"ok{rank}"), "w").write("ok")
+    finally:
+        dist.destroy_process_group()
+
+
+@pytest.mark.parametrize("world", [2, 3])
+def test_sharded_rare_stream(tmp_path, world):
+    mp.spawn(_rare_stream_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
     assert all(os.path.exists(tmp_path / f"ok{r}") for r in range(world))
 
 

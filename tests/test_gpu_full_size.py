@@ -102,7 +102,7 @@ def test_cen6_noisy_reads_match_oracle():
     k = P["k"]
     index, csr, res = eng.recruit(eng.upload_reads(batch, k), eng.upload_units(units, k), k, lo, hi, P["max_nonuniq"],
                                   P["min_d"], P["max_d"], P["min_coverage"])
-    assert getattr(eng, "stream_fallbacks", 0) == 0
+    assert eng.stream_fallbacks == 0
     want = c_oracle.recruit(batch, units, k, lo, hi, P["max_nonuniq"], P["min_d"], P["max_d"], P["min_coverage"],
                             threads=os.cpu_count() or 1)
     assert np.array_equal(index.sorted_keys.cpu().numpy().view(np.uint64), want["rare"])

@@ -375,9 +375,9 @@ def test_stream_count_splits_oversized_partitions(eng):
     try:
         for group in (1, 8):  # grouped units that do not fit are retried partition by partition, then split
             eng.stream_group = group
-            before = getattr(eng, "stream_fallbacks", 0)
+            before = eng.stream_fallbacks
             table = eng.count_docfreq(eng.upload_reads(batch, k), k)
-            assert table.dense and getattr(eng, "stream_fallbacks", 0) == before
+            assert table.dense and eng.stream_fallbacks == before
             keys, nr, nm = eng.table_select(table, 0, 0xFFFFFFFF, 0xFFFFFFFF, with_counts=True)
             keys = keys.cpu().numpy().view(np.uint64)
             order = np.argsort(keys)
@@ -525,3 +525,42 @@ def test_stream_launch_finish_equals_synchronous_call(eng):
         eng.docfreq_mode, eng.part_slack = old[0], old[2]
         eng.part_cap_seen.clear()
         eng.part_cap_seen.update(old[1])
+
+
+def test_stream_rare_output_too_small_on_both_paths(eng):
+    """A rare output too small for the band: rare_kmers and a docfreq_stream_launch / docfreq_stream_finish pair both
+    run phase 2 again on the records they keep (phase 1 once per call), return what a call with ample room returns and
+    leave a hint large enough for the next call."""
+    from centroflye_b200 import synth
+    from centroflye_b200.ingest import batch_from_synth
+    unit = synth.hor_unit(4, 60, 0.25, seed=5)
+    genome, a0, alen = synth.simulate_genome(unit, 120, 0.02, 6, flank_len=2000)
+    batch, _ = batch_from_synth(synth.simulate_reads(genome, a0, alen, unit, 20, 0.05, 7, median_len=7000, sigma=0.4,
+                                                     min_len=5200, max_len=20000), len(unit))
+    k, band, key = 19, (8, 24, 3), ("stream", False)
+    old = (eng.docfreq_mode, dict(eng.select_hint))
+    emit, emits = eng.emit_records, []
+
+    def counted(*a, **kw):
+        emits.append(1)
+        return emit(*a, **kw)
+    eng.docfreq_mode = "stream"
+    try:
+        reads = eng.upload_reads(batch, k)
+        eng.select_hint[key] = 1 << 20
+        want = np.sort(eng.rare_kmers(reads, k, *band).cpu().numpy().view(np.uint64))
+        assert want.size > 100
+        eng.emit_records = counted
+        eng.select_hint[key] = 1
+        got = eng.rare_kmers(reads, k, *band)
+        assert len(emits) == 1 and np.array_equal(np.sort(got.cpu().numpy().view(np.uint64)), want)
+        assert eng.select_hint[key] > want.size
+        eng.select_hint[key] = 1
+        got, table = eng.docfreq_stream_finish(eng.docfreq_stream_launch(reads, k, band=band))
+        assert len(emits) == 2 and table is None and np.array_equal(np.sort(got.cpu().numpy().view(np.uint64)), want)
+        assert eng.select_hint[key] > want.size
+    finally:
+        eng.__dict__.pop("emit_records", None)
+        eng.docfreq_mode = old[0]
+        eng.select_hint.clear()
+        eng.select_hint.update(old[1])

@@ -84,7 +84,7 @@ def test_sweep_point_matches_oracle(data, ctx, min_cov):
         data["uploads"] = {k: (eng.upload_reads(data["batch"], k), eng.upload_units(data["units"], k))}
     reads, dunits = data["uploads"][k]
     index, csr, res = eng.recruit(reads, dunits, k, ctx["lo"], ctx["hi"], c["max_nonuniq"], P["min_d"], P["max_d"], min_cov)
-    assert getattr(eng, "stream_fallbacks", 0) == 0
+    assert eng.stream_fallbacks == 0
     assert eng.last_pair_kernel == ("pair_candidates_kernel" if min_cov == 2 else "pair_sketch_kernel")
     keys = index.sorted_keys.cpu().numpy().view(np.uint64)
     assert np.array_equal(keys, want["rare"])

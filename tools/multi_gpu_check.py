@@ -55,7 +55,7 @@ def main():
     for _ in range(2):  # the second step runs with the adapted partition grouping / buffer sizes
         index, csr, res = rec.step(lo, hi, max_nonuniq, min_d, max_d, min_cov)
     keys = index.sorted_keys.cpu().numpy().view(np.uint64)
-    assert getattr(eng, "stream_fallbacks", 0) == 0, "the record exchange fell back"
+    assert eng.stream_fallbacks == 0, "the record exchange fell back"
     assert np.array_equal(keys, index_full.sorted_keys.cpu().numpy().view(np.uint64)), "record exchange != table exchange"
 
     whole_batch, whole_units = batch_from_synth(reads, len(unit))
