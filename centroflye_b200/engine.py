@@ -426,7 +426,7 @@ class Engine:
 
     def docfreq_stream(self, reads, k, band=None, with_counts=False, want_table=False, table_buf=None):
         """Two-phase stage A on one GPU -> (rare, table) or None when phase 2 could not hold a partition (more than
-        65535 reads sharing a k-mer, or a partition that does not fit after 64-fold splitting): the caller falls back
+        65536 reads sharing a k-mer, or a partition that does not fit after 64-fold splitting): the caller falls back
         to the single-kernel form.  rare = unordered keys inside band = (lo, hi, max_nonuniq) (a tuple with the two
         count tensors when with_counts); table = the dense DocFreqTable when want_table.  One host sync at the end
         (two when the table is wanted and no table_buf -- int64[2 * slots], at least one slot per k-mer occurrence --

@@ -129,7 +129,10 @@ int cfk_docfreq_count_resident(const uint32_t* packed, const int64_t* read_off, 
  *                            lays a rank's partitions back to back, out[offsets[p] + i], before the all-to-all).
  * cfk_docfreq_emit_plan writes n_pass[i] = passes of read order[i] (-> item_ptr by cfk_exclusive_scan).
  * cfk_docfreq_part_target() = k-mer occurrences to plan per partition (n_parts = ceil(occurrences / target)); a
- * partition may receive any number of records but must hold <= CFK_DOCFREQ_PART_DISTINCT distinct k-mers.
+ * partition may receive any number of records.  One with more distinct k-mers than a table holds
+ * (CFK_DOCFREQ_PART_DISTINCT planned, CFK_DOCFREQ_PART_DISTINCT * 4 / 3 slots) is counted again by halves of its hash
+ * range, then quarters, ... down to 64 sub-ranges; only a partition that does not fit even then sets counters[0].
+ * A k-mer may be in at most 65536 reads (more sets counters[0] too).
  * cursors[] and counters[8] are zeroed by the caller.  counters[0] != 0: a partition buffer (emit) or a
  * partition's table / 16-bit extra-read counter (count) overflowed -- results invalid, the caller falls back to
  * cfk_docfreq_count_resident; [1] != 0 internal error; [2], [3] work tickets.  The shared-memory sets claim empty
