@@ -11,7 +11,8 @@ the sequences, filters them and assembles ``>name\\nsequence\\n`` of the kept re
 appends that to the output.  Host and device memory follow the chunk size, not the input size.  recruit_file_units is
 the same pipeline for several (unit, output, threshold) jobs: the file is read and scanned once, one filter launch per
 word class covers every unit, and each output gets the bytes recruit_file writes for that job alone (recruit_file is
-its one-job case; main_units / scripts/rr_multi.py is its command line).  read_sequences() and
+its one-job case; main_units / scripts/rr_multi.py is its command line); with devices= it deals every chunk's records
+out to several GPUs in contiguous ranges, and the outputs are the same bytes.  read_sequences() and
 recruit() are the in-memory form of the same computation, and the specification the streaming form is tested against.
 """
 import gzip
@@ -340,7 +341,7 @@ def _part_file(output_fn):
             i += 1
 
 
-def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stats=None):
+def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stats=None, devices=None):
     """recruit_file for every job (unit, output_fn, threshold) of `jobs` in one pass over read_fn: the file is read,
     inflated and scanned once, the device filters every chunk for all units in one launch per unit word class, and
     each output file gets the bytes recruit_file writes for that job alone.  All outputs appear together when the run
@@ -348,16 +349,37 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
     unit; otherwise every unit is checked, with recruit_file's errors, before any output exists.  A byte >= 0x80 hands
     the whole run to the in-memory path (the file is read once, then recruit() per job).  Raises ValueError for no jobs,
     or for two jobs with the same output file.  Host and device memory follow chunk_bytes times the number of jobs.
-    stats: as in recruit_file, plus "job_out_bytes" (output bytes per job)."""
+
+    devices: None runs on one device (`engine`, or the default engine).  A list of devices (indices or torch.device;
+    repeats allowed) runs one worker per entry, each with an Engine, buffers and a thread of its own: every chunk's
+    records are dealt out in contiguous ranges of about equal bases (_split_records), each worker runs the device
+    work of its range, and every output is the workers' parts of each chunk in list order -- the same bytes.
+    stats: as in recruit_file, plus "job_out_bytes" (output bytes per job), "devices" (the number of workers) and
+    "device_s_per_device" (device seconds per stage of each worker; "device_s" is their sum)."""
     jobs = [(unit, output_fn, int(threshold)) for unit, output_fn, threshold in jobs]
     if not jobs:
         raise ValueError("recruit_file_units: no jobs")
     real = [os.path.realpath(output_fn) for _, output_fn, _ in jobs]
     if len(set(real)) != len(real):
         raise ValueError("recruit_file_units: two jobs write the same output file")
+    if devices is None:
+        def engines():
+            from .engine import default_engine
+            return [engine or default_engine()]
+        n_dev = 1
+    else:
+        devices = list(devices)
+        if not devices or engine is not None:
+            raise ValueError("recruit_file_units: devices must be a non-empty list, and excludes engine")
+
+        def engines():
+            from .engine import Engine
+            return [Engine(d) for d in devices]
+        n_dev = len(devices)
     st = {key: 0.0 for key in ("read_s", "assemble_s", "scan_s", "plan_s", "wait_s", "write_s")}
     st.update(chunks=0, records=0, bases=0, out_bytes=0, job_out_bytes=[0] * len(jobs), fallback=None,
-              device_s=None if stats is None else {})
+              devices=n_dev, device_s=None if stats is None else {},
+              device_s_per_device=None if stats is None else [{} for _ in range(n_dev)])
     tmps, files = [], []
     try:
         for _, output_fn, _ in jobs:
@@ -366,7 +388,7 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
             files.append(f)
         try:
             try:
-                _stream([(unit, threshold) for unit, _, threshold in jobs], read_fn, files, chunk_bytes, engine, st)
+                _stream([(unit, threshold) for unit, _, threshold in jobs], read_fn, files, chunk_bytes, engines, st)
             finally:
                 for f in files:
                     f.close()
@@ -387,190 +409,294 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
     return 0
 
 
-def _stream(jobs, read_fn, files, chunk_bytes, engine, st):
-    """recruit_file_units' pipeline: jobs = [(unit, threshold)], files[j] receives job j's output.  While the device
-    works on chunk i, the reader thread reads ahead, this thread scans chunk i + 1, and the writer thread writes chunk
-    i - 1.  Every device step of a chunk is on one stream, so one set of device buffers serves all chunks; host buffers
-    come in two slots (see _scan_chunks) plus two output buffers per job."""
+def _split_records(seq_len, n):
+    """The records of one chunk dealt to n devices: bounds int64[n + 1], device g takes records bounds[g] ..
+    bounds[g + 1] - 1.  The ranges are contiguous and cover every record once; none is empty unless there are fewer
+    records than devices; each holds total / n bases give or take the longest record.  A record goes to the range its
+    middle base falls in, so a range gains or loses at most half a record at either end.  A range can only be left
+    empty by a record longer than total / n; such ranges then take one record each from their neighbours, which only
+    shrinks the others."""
+    R = len(seq_len)
+    if R < n:
+        return np.minimum(np.arange(n + 1, dtype=np.int64), R)
+    ends = np.cumsum(seq_len, dtype=np.int64)
+    twice_mid = 2 * ends - seq_len
+    b = np.searchsorted(n * twice_mid, 2 * int(ends[-1]) * np.arange(n + 1, dtype=np.int64), side="left")
+    b[0], b[n] = 0, R
+    for k in range(1, n):
+        b[k] = min(max(b[k], b[k - 1] + 1), R - n + k)
+    return b.astype(np.int64)
+
+
+class _Worker:
+    """One device of recruit_file_units' pipeline: a thread (named rr-device-<index>) that runs step() on its record
+    range of every chunk handed to it through `inbox` and puts step()'s result, or the exception that ended it, on
+    `outbox`.  Its engine, device buffers, pinned host buffers and output buffers are its own and follow the size of
+    its ranges.  Every device call of a step is on the engine's stream, so one set of device buffers serves all
+    chunks.  `run` holds what every worker shares: the filter plan of the jobs and the run's error state."""
+
+    def __init__(self, index, eng, run, peq, sym_of):
+        import torch
+        self.torch, self.index, self.eng, self.run = torch, index, eng, run
+        self.host, self.dev, self.events, self.plan_s = {}, {}, [], 0.0
+        self.free_out = [queue.Queue() for _ in run.jobs]  # two output buffers per job, handed back by the writer
+        for q in self.free_out:
+            q.put(0)
+            q.put(1)
+        self.d_peq = self.d_sym = None
+        if run.filtered:
+            self.d_peq, self.d_sym = eng._to_dev(peq), eng._to_dev(sym_of)
+        self.inbox, self.outbox = queue.Queue(), queue.Queue()
+        self.thread = threading.Thread(target=self._loop, name=f"rr-device-{index}", daemon=True)
+        self.thread.start()
+
+    def _loop(self):
+        try:
+            self.eng._stream()  # makes the engine's device current for this thread
+            while True:
+                item = self.inbox.get()
+                if item is None:
+                    return
+                if not self.run.abort.is_set():
+                    self.outbox.put(self.step(*item))
+        except BaseException as e:  # noqa: BLE001 -- raised by the main thread when it collects this chunk
+            self.outbox.put(e)
+
+    def _mark(self):
+        if not self.run.timed:
+            return None
+        e = self.torch.cuda.Event(enable_timing=True)
+        e.record()
+        return e
+
+    def _hbuf(self, key, nbytes):
+        return _grown(self.host, key, nbytes, lambda n: self.torch.empty(n, dtype=self.torch.uint8, pin_memory=True))
+
+    def _dbuf(self, key, nbytes, dtype=None):
+        t = self.torch
+        buf = _grown(self.dev, key, nbytes, lambda n: t.empty(n, dtype=t.uint8, device=self.eng.device))
+        return buf.view(dtype or t.uint8)
+
+    def step(self, raw, rec, piece, text_bytes, r0, r1):
+        """The device work of records r0 .. r1 - 1 of a chunk as _scan_chunks yields it: their bytes of raw and their
+        rows of rec and piece, rebased on the host, go to the device, which gathers their sequences, filters them for
+        every unit and emits every job's output; the outputs come home into this worker's output buffers.  Returns
+        the parts for the writer, [(copy-done event, job, host buffer, bytes, free queue, key)], in job order."""
+        if r0 == r1:
+            return []
+        torch, run, p = self.torch, self.run, self.eng._p
+        t0 = time.perf_counter()
+        # the range's text is rec[r0, 3] .. the next record's (16-byte aligned, like every record's), its pieces are
+        # the ones placed there, and its raw bytes run from its first name to its last name or piece
+        t_lo = int(rec[r0, 3])
+        t_hi = int(rec[r1, 3]) if r1 < rec.shape[0] else text_bytes
+        p0, p1 = (int(x) for x in np.searchsorted(piece[:, 2], (t_lo, t_hi)))
+        lo, hi = int(rec[r0, 0]), int(rec[r1 - 1, 0] + rec[r1 - 1, 1])
+        if p1 > p0:
+            hi = max(hi, int(piece[p1 - 1, 0] + piece[p1 - 1, 1]))
+        R, P, n, text_bytes = r1 - r0, p1 - p0, hi - lo, t_hi - t_lo
+        h_rec = self._hbuf("rec", 32 * R)
+        rec = np.subtract(rec[r0:r1], np.array([lo, 0, 0, t_lo], dtype=np.int64),
+                          out=h_rec.numpy()[:32 * R].view(np.int64).reshape(R, 4))
+        h_piece = self._hbuf("piece", 24 * P)
+        np.subtract(piece[p0:p1], np.array([lo, 0, t_lo], dtype=np.int64),
+                    out=h_piece.numpy()[:24 * P].view(np.int64).reshape(P, 3))
+        seq_len = rec[:, 2]
+        upper = int((rec[:, 1] + seq_len).sum()) + 3 * R
+        # segments as recruit() plans them (with run.overlap); when no job has threshold >= 0 no filter runs.
+        # Host layout, int64: seg_off[S] | seg_len[S] | seg_ptr[R + 1] (first segment of each record) | order[S] (int32
+        # in the first half)
+        S, F = 0, len(run.filtered)
+        if F:
+            n_seg = np.maximum(1, -(-np.maximum(seq_len - run.overlap, 1) // SEGMENT))
+            S = int(n_seg.sum())
+            seg_read = np.repeat(np.arange(R, dtype=np.int64), n_seg)
+            j = np.arange(S, dtype=np.int64) - np.repeat(np.cumsum(n_seg) - n_seg, n_seg)
+            nb = 8 * (3 * S + R + 1)
+            hs = self._hbuf("seg", nb)
+            seg = hs.numpy()[:nb].view(np.int64)
+            seg_lens = seg[S:2 * S]
+            seg[:S] = rec[seg_read, 3] + j * SEGMENT
+            seg_lens[:] = np.minimum(SEGMENT + run.overlap, seq_len[seg_read] - j * SEGMENT)
+            seg[2 * S] = 0
+            np.cumsum(n_seg, out=seg[2 * S + 1:2 * S + R + 1])
+            seg[2 * S + R + 1:].view(np.int32)[:S] = np.argsort(-seg_lens, kind="stable")
+        self.plan_s += time.perf_counter() - t0
+        a = self._mark()
+        d_raw = self._dbuf("raw", n + 16)
+        d_raw[:n].copy_(raw[lo:hi], non_blocking=True)
+        d_rec = self._dbuf("rec", 32 * R)
+        d_rec[:32 * R].copy_(h_rec[:32 * R], non_blocking=True)
+        d_piece = self._dbuf("piece", 24 * P + 8)
+        if P:
+            d_piece[:24 * P].copy_(h_piece[:24 * P], non_blocking=True)
+        if S:
+            d_seg = self._dbuf("seg", nb)
+            d_seg[:nb].copy_(hs[:nb], non_blocking=True)
+        b = self._mark()
+        stream = self.eng._stream()
+        d_text = self._dbuf("text", text_bytes + 16)
+        _lib.call("cfk_rr_gather", p(d_raw), p(d_piece), P, p(d_text), text_bytes, stream)
+        c = self._mark()
+        d_keep = seg_ptr = None
+        if S:
+            d_keep = self._dbuf("keep", F * S)  # [unit][segment]
+            d_keep[:F * S].zero_()
+            base = d_seg.data_ptr()
+            seg_ptr = base + 16 * S
+            _lib.call("cfk_rr_filter_units", p(d_text), base, base + 8 * S, base + 8 * (2 * S + R + 1), S, F,
+                      p(self.d_peq), p(self.d_sym), run.unit_m.ctypes.data, run.unit_threshold.ctypes.data, p(d_keep),
+                      stream)
+        d = self._mark()
+        d_sizes = self._dbuf("sizes", 4 * R, torch.int32)
+        d_off = self._dbuf("off", 8 * (R + 1), torch.int64)
+        d_scratch = self._dbuf("scratch", 8 * int(self.eng.lib.cfk_scan_scratch_elems(R)))
+        d_totals = self._dbuf("totals", 8 * len(run.jobs), torch.int64)
+        d_outs = []
+        for j in range(len(run.jobs)):  # sizes, offsets and scan scratch are reused: the job's emit has read them by then
+            d_out = self._dbuf(("out", j), upper + 16)
+            seg_keep = None if j not in run.row else p(d_keep) + run.row[j] * S
+            _lib.call("cfk_rr_keep_sizes", seg_keep, None if seg_keep is None else seg_ptr, p(d_rec), R, p(d_sizes),
+                      stream)
+            _lib.call("cfk_exclusive_scan", p(d_sizes), p(d_off), R, p(d_scratch), stream)
+            _lib.call("cfk_rr_emit", p(d_raw), p(d_text), p(d_rec), p(d_off), R, upper, p(d_out), stream)
+            d_totals[j:j + 1].copy_(d_off[R:R + 1])
+            d_outs.append(d_out)
+        if run.timed:
+            self.events.extend((("h2d", a, b), ("gather", b, c), ("filter", c, d), ("emit", d, self._mark())))
+        totals = d_totals[:len(run.jobs)].tolist()  # the range's one size read-back
+        parts = []
+        for j, (total, d_out) in enumerate(zip(totals, d_outs)):
+            key = self.free_out[j].get()
+            if run.writer_err:
+                raise run.writer_err[0]
+            h = self._hbuf(("out", j, key), total)
+            a = self._mark()
+            if total:
+                h[:total].copy_(d_out[:total], non_blocking=True)
+            done = torch.cuda.Event()
+            done.record()
+            if run.timed:
+                self.events.append(("d2h", a, self._mark()))
+            parts.append((done, j, h, total, self.free_out[j], key))
+        return parts
+
+
+def _stream(jobs, read_fn, files, chunk_bytes, engines, st):
+    """recruit_file_units' pipeline: jobs = [(unit, threshold)], files[j] receives job j's output, engines() -> one
+    engine per worker (called once the first record is seen).  While the workers' devices work on chunk i, the reader
+    thread reads ahead, this thread scans chunk i + 1 and deals its records out, and the writer thread writes chunk
+    i - 1, every job's parts in worker order.  Host chunk buffers come in two slots (see _scan_chunks): a slot is
+    scanned into again only after every worker has finished with it."""
+    import types
+
     import torch
     host = {"alloc": lambda n: torch.empty(n, dtype=torch.uint8)}  # pageable until the first record is seen
-    dev, out_host = {}, {}
-    device_s, events = st["device_s"], []
-    eng = d_peq = d_sym = writer = None
-    writer_q, free_out, writer_err = queue.Queue(), [queue.Queue() for _ in jobs], []
     # the jobs that run the filter (threshold >= 0; the others keep every read), and their units' rows in d_peq / d_sym
     filtered = [j for j, (_, threshold) in enumerate(jobs) if threshold >= 0]
-    row = {j: i for i, j in enumerate(filtered)}
-    unit_m = np.array([len(jobs[j][0]) for j in filtered], dtype=np.int32)
-    unit_threshold = np.array([jobs[j][1] for j in filtered], dtype=np.int32)
     # One segment plan serves every unit.  A hit within t edits spans at most |unit| + t read bases, so it lies wholly
     # inside some segment whenever the segments overlap by at least that much; and a segment is an infix of its read,
     # so a hit inside a segment is a hit in the read.  Overlapping by the largest |unit| + t of all jobs therefore
-    # decides every read as recruit()'s plan for each job alone does.
-    overlap = max((len(jobs[j][0]) + jobs[j][1] for j in filtered), default=0)
-
-    def mark():
-        if device_s is None:
-            return None
-        e = torch.cuda.Event(enable_timing=True)
-        e.record()
-        return e
+    # decides every read as recruit()'s plan for each job alone does.  Segments never span records, so dealing the
+    # records of a chunk out to several devices changes no decision either.
+    run = types.SimpleNamespace(
+        jobs=jobs, filtered=filtered, row={j: i for i, j in enumerate(filtered)},
+        unit_m=np.array([len(jobs[j][0]) for j in filtered], dtype=np.int32),
+        unit_threshold=np.array([jobs[j][1] for j in filtered], dtype=np.int32),
+        overlap=max((len(jobs[j][0]) + jobs[j][1] for j in filtered), default=0),
+        timed=st["device_s"] is not None, abort=threading.Event(), writer_err=[])
+    workers, writer, writer_q = [], None, queue.Queue()
 
     def write_loop():
         while True:
             item = writer_q.get()
             if item is None:
                 return
-            done, j, key, nbytes = item
+            done, j, h, nbytes, free, key = item
             try:
                 done.synchronize()
                 t0 = time.perf_counter()
-                files[j].write(memoryview(out_host[j, key].numpy()[:nbytes]))
+                files[j].write(memoryview(h.numpy()[:nbytes]))
                 st["write_s"] += time.perf_counter() - t0
-            except BaseException as e:  # noqa: BLE001 -- raised by the main thread at its next hand-over
-                writer_err.append(e)
-            free_out[j].put(key)
+            except BaseException as e:  # noqa: BLE001 -- raised by a worker at its next hand-over
+                run.writer_err.append(e)
+            free.put(key)
 
-    def start_device():
-        nonlocal eng, d_peq, d_sym, writer
-        from .engine import default_engine
-        eng = engine or default_engine()
+    def start():
+        nonlocal writer
         masks = [build_masks(unit) for unit, _ in jobs]  # raises on an invalid unit, before any output
+        peq = sym_of = None
         if filtered:
-            d_peq = eng._to_dev(np.concatenate([masks[j][0].reshape(-1) for j in filtered]).view(np.int64))
-            d_sym = eng._to_dev(np.concatenate([masks[j][1] for j in filtered]))
+            peq = np.concatenate([masks[j][0].reshape(-1) for j in filtered]).view(np.int64)
+            sym_of = np.concatenate([masks[j][1] for j in filtered])
+        for g, eng in enumerate(engines()):
+            workers.append(_Worker(g, eng, run, peq, sym_of))
         host["alloc"] = lambda n: torch.empty(n, dtype=torch.uint8, pin_memory=True)
-        for q in free_out:
-            for key in (0, 1):
-                q.put(key)
         writer = threading.Thread(target=write_loop, name="rr-writer", daemon=True)
         writer.start()
 
-    def dbuf(key, nbytes, dtype=torch.uint8):
-        t = _grown(dev, key, nbytes, lambda n: torch.empty(n, dtype=torch.uint8, device=eng.device))
-        return t.view(dtype)
-
-    def launch(slot, raw, rec, piece, text_bytes):
-        p = eng._p
-        t0 = time.perf_counter()
-        R, P, n = rec.shape[0], piece.shape[0], raw.numel()
-        seq_len = rec[:, 2]
-        sizes = rec[:, 1] + seq_len + 3
-        if int(sizes.max()) >= 1 << 31:
-            raise _Fallback("a record of 2 GiB or more")
-        upper = int(sizes.sum())
-        st["records"] += R
-        st["bases"] += int(seq_len.sum())
-        # segments as recruit() plans them (with the overlap above); when no job has threshold >= 0 no filter runs.
-        # Host layout, int64: seg_off[S] | seg_len[S] | seg_ptr[R + 1] (first segment of each record) | order[S] (int32
-        # in the first half)
-        S = 0
-        if filtered:
-            n_seg = np.maximum(1, -(-np.maximum(seq_len - overlap, 1) // SEGMENT))
-            S = int(n_seg.sum())
-            seg_read = np.repeat(np.arange(R, dtype=np.int64), n_seg)
-            j = np.arange(S, dtype=np.int64) - np.repeat(np.cumsum(n_seg) - n_seg, n_seg)
-            nb = 8 * (3 * S + R + 1)
-            hs = _grown(host, (slot, "seg"), nb, host["alloc"])
-            seg = hs.numpy()[:nb].view(np.int64)
-            seg_lens = seg[S:2 * S]
-            seg[:S] = rec[seg_read, 3] + j * SEGMENT
-            seg_lens[:] = np.minimum(SEGMENT + overlap, seq_len[seg_read] - j * SEGMENT)
-            seg[2 * S] = 0
-            np.cumsum(n_seg, out=seg[2 * S + 1:2 * S + R + 1])
-            seg[2 * S + R + 1:].view(np.int32)[:S] = np.argsort(-seg_lens, kind="stable")
-        st["plan_s"] += time.perf_counter() - t0
-        a = mark()
-        d_raw = dbuf("raw", n + 16)
-        d_raw[:n].copy_(raw, non_blocking=True)
-        d_rec = dbuf("rec", 32 * R, torch.int64)
-        d_rec[:4 * R].copy_(torch.from_numpy(rec.reshape(-1)), non_blocking=True)
-        d_piece = dbuf("piece", 24 * P + 8, torch.int64)
-        if P:
-            d_piece[:3 * P].copy_(torch.from_numpy(piece.reshape(-1)), non_blocking=True)
-        if S:
-            d_seg = dbuf("seg", nb)
-            d_seg[:nb].copy_(hs[:nb], non_blocking=True)
-        b = mark()
-        stream = eng._stream()
-        d_text = dbuf("text", text_bytes + 16)
-        _lib.call("cfk_rr_gather", p(d_raw), p(d_piece), P, p(d_text), text_bytes, stream)
-        c = mark()
-        d_keep = seg_ptr = None
-        if S:
-            d_keep = dbuf("keep", len(filtered) * S)  # [unit][segment]
-            d_keep[:len(filtered) * S].zero_()
-            base = d_seg.data_ptr()
-            seg_ptr = base + 16 * S
-            _lib.call("cfk_rr_filter_units", p(d_text), base, base + 8 * S, base + 8 * (2 * S + R + 1), S, len(filtered),
-                      p(d_peq), p(d_sym), unit_m.ctypes.data, unit_threshold.ctypes.data, p(d_keep), stream)
-        d = mark()
-        d_sizes = dbuf("sizes", 4 * R, torch.int32)
-        d_off = dbuf("off", 8 * (R + 1), torch.int64)
-        d_scratch = dbuf("scratch", 8 * int(eng.lib.cfk_scan_scratch_elems(R)))
-        d_totals = dbuf("totals", 8 * len(jobs), torch.int64)
-        d_outs = []
-        for j in range(len(jobs)):  # sizes, offsets and scan scratch are reused: the job's emit has read them by then
-            d_out = dbuf(("out", j), upper + 16)
-            seg_keep = None if j not in row else p(d_keep) + row[j] * S
-            _lib.call("cfk_rr_keep_sizes", seg_keep, None if seg_keep is None else seg_ptr, p(d_rec), R, p(d_sizes), stream)
-            _lib.call("cfk_exclusive_scan", p(d_sizes), p(d_off), R, p(d_scratch), stream)
-            _lib.call("cfk_rr_emit", p(d_raw), p(d_text), p(d_rec), p(d_off), R, upper, p(d_out), stream)
-            d_totals[j:j + 1].copy_(d_off[R:R + 1])
-            d_outs.append(d_out)
-        if device_s is not None:
-            events.extend((("h2d", a, b), ("gather", b, c), ("filter", c, d), ("emit", d, mark())))
-        st["chunks"] += 1
-        return d_totals[:len(jobs)], d_outs
-
-    def finish(d_totals, d_outs):
-        t0 = time.perf_counter()
-        totals = d_totals.tolist()  # the chunk's one size read-back
-        st["wait_s"] += time.perf_counter() - t0
-        for j, (total, d_out) in enumerate(zip(totals, d_outs)):
+    def collect():
+        """Waits for every worker's result of the oldest chunk in flight and queues its parts for the writer."""
+        for w in workers:
             t0 = time.perf_counter()
-            key = free_out[j].get()
+            parts = w.outbox.get()
             st["wait_s"] += time.perf_counter() - t0
-            if writer_err:
-                raise writer_err[0]
-            h = _grown(out_host, (j, key), total, host["alloc"])
-            a = mark()
-            if total:
-                h[:total].copy_(d_out[:total], non_blocking=True)
-            done = torch.cuda.Event()
-            done.record()
-            if device_s is not None:
-                events.append(("d2h", a, mark()))
-            st["out_bytes"] += total
-            st["job_out_bytes"][j] += total
-            writer_q.put((done, j, key, total))
+            if isinstance(parts, BaseException):
+                raise parts
+            for part in parts:
+                _, j, _, nbytes, _, _ = part
+                st["out_bytes"] += nbytes
+                st["job_out_bytes"][j] += nbytes
+                writer_q.put(part)
 
     chunks = _scan_chunks(read_fn, chunk_bytes, host, st)
-    pending = None
+    in_flight = False
     try:
-        for slot, raw, rec, piece, text_bytes in chunks:  # scanning chunk i overlaps the device's work on chunk i - 1
-            if pending is not None:
-                finish(*pending)
-            first = eng is None
+        for slot, raw, rec, piece, text_bytes in chunks:  # scanning chunk i + 1 overlaps the devices' work on chunk i
+            first = not workers
             if first:
-                start_device()
-            pending = launch(slot, raw, rec, piece, text_bytes)
-            if first:  # chunk 0 was scanned into pageable memory (copied synchronously): later chunks use pinned buffers
+                start()
+            t0 = time.perf_counter()
+            seq_len = rec[:, 2]
+            if int((rec[:, 1] + seq_len).max()) + 3 >= 1 << 31:
+                raise _Fallback("a record of 2 GiB or more")
+            st["records"] += rec.shape[0]
+            st["bases"] += int(seq_len.sum())
+            bounds = _split_records(seq_len, len(workers)).tolist()
+            for w, r0, r1 in zip(workers, bounds[:-1], bounds[1:]):
+                w.inbox.put((raw, rec, piece, text_bytes, r0, r1))
+            st["chunks"] += 1
+            st["plan_s"] += time.perf_counter() - t0
+            if in_flight:
+                collect()
+            in_flight = True
+            if first:  # chunk 0 was scanned into pageable memory: the slot's later chunks use pinned buffers
                 for name in ("raw", "rec", "piece"):
                     host.pop((slot, name))
-        if pending is not None:
-            finish(*pending)
+        if in_flight:
+            collect()
     finally:
         chunks.close()
+        run.abort.set()  # after an error, workers skip what is queued
+        for w in workers:
+            w.inbox.put(None)
         if writer is not None:
             writer_q.put(None)
+        for w in workers:
+            w.thread.join()
+        if writer is not None:
             writer.join()
-    if writer_err:
-        raise writer_err[0]
-    if device_s is not None:
-        torch.cuda.synchronize()
-        for name, a, b in events:
-            device_s[name] = device_s.get(name, 0.0) + a.elapsed_time(b) / 1e3
+    if run.writer_err:
+        raise run.writer_err[0]
+    st["plan_s"] += sum(w.plan_s for w in workers)
+    if run.timed:
+        for w in workers:
+            torch.cuda.synchronize(w.eng.device)
+            mine = st["device_s_per_device"][w.index]
+            for name, a, b in w.events:
+                s = a.elapsed_time(b) / 1e3
+                mine[name] = mine.get(name, 0.0) + s
+                st["device_s"][name] = st["device_s"].get(name, 0.0) + s
 
 
 def main(argv=None):
@@ -588,14 +714,28 @@ def main(argv=None):
     return 0
 
 
-UNITS_USAGE = "Usage: rr_multi.py reads.fasta[.gz|.fastq] unit1.fasta output1.fasta threshold1 [unit2.fasta output2.fasta threshold2 ...]"
+UNITS_USAGE = ("Usage: rr_multi.py reads.fasta[.gz|.fastq] unit1.fasta output1.fasta threshold1 [unit2.fasta output2.fasta threshold2 ...]\n"
+               "       --gpus N (first): deal every chunk's records over cuda:0..N-1")
 
 
 def main_units(argv=None):
-    """``rr_multi.py reads unit1 output1 threshold1 [unit2 output2 threshold2 ...]``: what one rr run per triple writes,
-    from one pass over the read file (recruit_file_units).  Each unit is the first record of its file; thresholds are
-    read as main() reads them.  Wrong argument count: the usage on stderr, status 2."""
+    """``rr_multi.py [--gpus N] reads unit1 output1 threshold1 [unit2 output2 threshold2 ...]``: what one rr run per
+    triple writes, from one pass over the read file (recruit_file_units).  Each unit is the first record of its file;
+    thresholds are read as main() reads them.  --gpus N runs on cuda:0 .. N-1 (devices=); without it, on one device.
+    A wrong argument count, or an N that is not an integer from 1 to the number of visible devices: the usage on
+    stderr, status 2."""
     argv = sys.argv[1:] if argv is None else list(argv)
+    devices = None
+    if argv[:1] == ["--gpus"]:
+        import torch
+        try:
+            n = int(argv[1])
+        except (IndexError, ValueError):
+            n = 0
+        if not 1 <= n <= torch.cuda.device_count():
+            print(UNITS_USAGE, file=sys.stderr)
+            return 2
+        devices, argv = list(range(n)), argv[2:]
     if len(argv) < 4 or (len(argv) - 1) % 3:
         print(UNITS_USAGE, file=sys.stderr)
         return 2
@@ -606,7 +746,7 @@ def main_units(argv=None):
         except ValueError:
             threshold = 0  # std::atoi, as in main()
         jobs.append((next(read_sequences(unit_fn))[1], output_fn, threshold))
-    recruit_file_units(jobs, argv[0])
+    recruit_file_units(jobs, argv[0], devices=devices)
     return 0
 
 
