@@ -42,6 +42,8 @@ SIGNATURES = {
     "cfk_rr_words": (_int, [_i32]),
     "cfk_rr_filter": (_int, [_p, _p, _p, _p, _i64, _p, _p, _i32, _i32, _i32, _p, _p, _p]),
     "cfk_rr_filter_units": (_int, [_p, _p, _p, _p, _i64, _i32, _p, _p, _p, _p, _p, _p]),  # unit_m, unit_threshold: host
+    "cfk_rr_long_words": (_int, [_i32]),
+    "cfk_rr_filter_long": (_int, [_p, _p, _p, _p, _i64, _i32, _p, _p, _p, _p, _i32, _p, _p, _p]),  # unit_m, unit_threshold: host
     "cfk_seq_scan": (_int, [_p, _i64, _i32, _p, _i64, _p, _i64, _p]),  # host pointers
     "cfk_rr_gather": (_int, [_p, _p, _i64, _p, _i64, _p]),
     "cfk_rr_keep_sizes": (_int, [_p, _p, _p, _i64, _p, _p]),

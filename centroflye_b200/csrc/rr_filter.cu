@@ -128,6 +128,127 @@ int rr_launch(int nw, const RrArgs& A, int n_units, cudaStream_t st) {
   return CFK_OK;
 }
 
+// ---- units longer than 52 words: one warp per (segment, strand) ----------------------------------------------------
+// The unit's nw = ceil(m / 64) words are split over the lanes, W consecutive words per lane, so Pv / Mv of a unit of up
+// to 32 * W * 64 bases stay in registers.  The lanes form a wavefront: at step s lane L applies the block step of
+// rr_filter_kernel to its W words for text character s - L, starting from the horizontal delta that lane L - 1 produced
+// for that character at step s - 1 (lane 0 starts from 0: free start in the text).  That delta and the character's
+// symbol slot travel up the lanes in one shuffle per step, so only lane 0 reads the text.  The bottom row is bit
+// (m - 1) & 63 of word nw - 1, in lane (nw - 1) / W, which keeps score and best; a segment of n bases takes n + that lane
+// steps.  Every 16 characters of the bottom lane the warp checks best against the stop rule of rr_filter_kernel, so
+// out_dist without exact holds what rr_filter_kernel writes there.
+// Match masks are lane-minor, [2 strands][RR_MAX_SYMBOLS][W][32 lanes]: word k of every lane is one 256-byte row of
+// shared memory whatever symbol each lane holds, so a warp's load is free of bank conflicts.
+constexpr int RRW_WARPS = 8;                 // warps per block; each takes one (segment, strand)
+constexpr int RRW_THREADS = 32 * RRW_WARPS;
+constexpr int RRW_MAX_BASES = 32 * 16 * 64;  // W = 16
+
+template <int W>
+__global__ void __launch_bounds__(RRW_THREADS) rr_filter_warp_kernel(const __grid_constant__ RrArgs A) {
+  extern __shared__ uint64_t s_peq[];  // [2][RR_MAX_SYMBOLS][W][32]
+  __shared__ uint8_t s_sym[256];
+  const RrUnit& U = A.unit[blockIdx.y];
+  const uint64_t* g_peq = A.peq + U.peq_off;
+  const uint8_t* g_sym = A.sym_of + 256 * (int64_t)U.index;
+  for (int i = threadIdx.x; i < 2 * RR_MAX_SYMBOLS * W * 32; i += RRW_THREADS) s_peq[i] = g_peq[i];
+  for (int i = threadIdx.x; i < 256; i += RRW_THREADS) s_sym[i] = g_sym[i];
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int64_t item = (int64_t)blockIdx.x * RRW_WARPS + (threadIdx.x >> 5);
+  if (item >= 2 * A.n_reads) return;  // the whole warp
+  const int64_t r = A.order[item >> 1];
+  const int strand = (int)(item & 1);
+  const uint64_t* peq = s_peq + strand * RR_MAX_SYMBOLS * W * 32 + lane;
+  const int64_t n = A.read_len[r];
+  const uint4* text = reinterpret_cast<const uint4*>(A.text + A.read_off[r]);
+  const int32_t m = U.m;
+  const int nw = (m + 63) >> 6;
+  const int bottom_lane = (nw - 1) / W, bottom_k = (nw - 1) % W, last_bit = (m - 1) & 63;
+  const bool bottom = lane == bottom_lane;
+  uint64_t Pv[W], Mv[W];
+#pragma unroll
+  for (int k = 0; k < W; ++k) {
+    Pv[k] = ~0ull;
+    Mv[k] = 0ull;
+  }
+  int score = m, best = m;
+  const int stop = A.exact ? -1 : U.threshold;
+  uint4 chunk = make_uint4(0, 0, 0, 0);
+  int from_below = 1;  // (horizontal delta + 1) | symbol slot << 2, from lane - 1 at the previous step
+  const int64_t steps = n + bottom_lane;
+  for (int64_t s = 0; s < steps; ++s) {
+    const int64_t c = s - lane;  // this lane's text character
+    int sym, hin;
+    if (lane == 0) {
+      if (c < n && (c & 15) == 0) chunk = __ldg(text + (c >> 4));
+      const int q = (int)(c & 15);
+      const uint32_t word = q < 4 ? chunk.x : q < 8 ? chunk.y : q < 12 ? chunk.z : chunk.w;
+      sym = s_sym[(word >> (8 * (q & 3))) & 0xFFu];
+      hin = 0;
+    } else {
+      sym = from_below >> 2;
+      hin = (from_below & 3) - 1;
+    }
+    const bool active = c >= 0 && c < n;
+    const uint64_t* eqrow = peq + sym * (W * 32);
+    int delta = 0;
+#pragma unroll
+    for (int k = 0; k < W; ++k) {
+      uint64_t Eq = eqrow[k * 32];
+      const uint64_t pv = Pv[k], mv = Mv[k];
+      const uint64_t Xv = Eq | mv;
+      if (hin < 0) Eq |= 1ull;
+      const uint64_t Xh = (((Eq & pv) + pv) ^ pv) | Eq;
+      uint64_t Ph = mv | ~(Xh | pv);
+      uint64_t Mh = pv & Xh;
+      const int bit = (bottom && k == bottom_k) ? last_bit : 63;
+      const int hout = (int)((Ph >> bit) & 1ull) - (int)((Mh >> bit) & 1ull);
+      Ph <<= 1;
+      Mh <<= 1;
+      if (hin < 0) Mh |= 1ull;
+      else if (hin > 0) Ph |= 1ull;
+      if (active) {
+        Pv[k] = Mh | ~(Xv | Ph);
+        Mv[k] = Ph & Xv;
+      }
+      if (k == bottom_k) delta = hout;
+      hin = hout;
+    }
+    if (bottom && active) {
+      score += delta;
+      best = min(best, score);
+    }
+    from_below = __shfl_up_sync(0xFFFFFFFFu, (hin + 1) | (sym << 2), 1);
+    const int64_t done = s - bottom_lane + 1;  // characters the bottom lane has finished
+    if (done > 0 && (done & 15) == 0 && __shfl_sync(0xFFFFFFFFu, best, bottom_lane) <= stop) break;
+  }
+  if (bottom) {
+    const int64_t at = U.keep_off + r;
+    if (A.out_dist != nullptr) A.out_dist[2 * at + strand] = best;
+    if (U.threshold < 0 || best <= U.threshold) A.out_keep[at] = 1;
+  }
+}
+
+// A.unit[0 .. n_units) all have cfk_rr_long_words(m) == w.
+int rr_long_launch(int w, const RrArgs& A, int n_units, cudaStream_t st) {
+  const dim3 grid((unsigned)blocks_for(2 * A.n_reads, RRW_WARPS), (unsigned)n_units);
+  const int smem = 2 * RR_MAX_SYMBOLS * w * 32 * (int)sizeof(uint64_t);
+  switch (w) {
+    case 2: rr_filter_warp_kernel<2><<<grid, RRW_THREADS, smem, st>>>(A); break;
+    case 4: rr_filter_warp_kernel<4><<<grid, RRW_THREADS, smem, st>>>(A); break;
+    case 8: rr_filter_warp_kernel<8><<<grid, RRW_THREADS, smem, st>>>(A); break;
+    default: {
+      static unsigned long long smem_set = 0;  // 64 KB: above the default limit of 48 KB
+      if (const cudaError_t e = ensure_dynamic_smem(rr_filter_warp_kernel<16>, smem, &smem_set))
+        return fail(CFK_ERR_CUDA, "rr_filter_warp_kernel<16>: dynamic shared memory", e);
+      rr_filter_warp_kernel<16><<<grid, RRW_THREADS, smem, st>>>(A);
+      break;
+    }
+  }
+  CFK_CHECK_LAUNCH("rr_filter_warp_kernel", 1);
+  return CFK_OK;
+}
+
 // ---- streaming form (read_recruitment.recruit_file): raw file text in, output file text out ----------------------
 // Both copy kernels are driven by the destination: one thread writes 16 consecutive output bytes with one 16-byte store
 // and finds its source by a binary search over the sorted destination offsets, so 80-column FASTA lines and megabase
@@ -274,6 +395,49 @@ int cfk_rr_filter_units(const uint8_t* text, const int64_t* seg_off, const int64
     }
     if (n > 0)
       if (const int rc = rr_launch(nw, A, n, st)) return rc;
+  }
+  return CFK_OK;
+}
+
+/* lanes' words of rr_filter_warp_kernel for a unit of m bases: the least W with ceil(ceil(m / 64) / W) <= 32 */
+int cfk_rr_long_words(int32_t m) {
+  if (m < 1 || m > RRW_MAX_BASES) return -1;
+  const int need = (m + 63) / 64;
+  for (int w : {2, 4, 8, 16})
+    if (need <= 32 * w) return w;
+  return -1;
+}
+
+int cfk_rr_filter_long(const uint8_t* text, const int64_t* seg_off, const int64_t* seg_len, const int32_t* order, int64_t n_seg,
+                       int32_t n_units, const uint64_t* peq, const uint8_t* sym_of, const int32_t* unit_m,
+                       const int32_t* unit_threshold, int32_t exact, int32_t* out_dist, uint8_t* out_keep,
+                       cfk_stream_t stream) {
+  if (n_seg < 0 || n_seg >= (1ll << 30) || n_units < 0 || (n_units > 0 && (unit_m == nullptr || unit_threshold == nullptr)))
+    return fail(CFK_ERR_INVALID, "cfk_rr_filter_long: bad sizes");
+  if (((uintptr_t)text & 15u) != 0) return fail(CFK_ERR_INVALID, "cfk_rr_filter_long: text must be 16-byte aligned");
+  for (int32_t u = 0; u < n_units; ++u)
+    if (cfk_rr_long_words(unit_m[u]) < 0)
+      return fail(CFK_ERR_INVALID, "cfk_rr_filter_long: every unit must have 1..32768 bases");
+  if (n_seg == 0 || n_units == 0) return CFK_OK;
+  // one launch per lane-word class present (several when a class has more than RR_UNITS_PER_LAUNCH units)
+  const cudaStream_t st = (cudaStream_t)stream;
+  for (int w : {2, 4, 8, 16}) {
+    RrArgs A{text, seg_off, seg_len, order, n_seg, peq, sym_of, exact, out_dist, out_keep, {}};
+    int n = 0;
+    int64_t off = 0;
+    for (int32_t u = 0; u < n_units; ++u) {
+      const int uw = cfk_rr_long_words(unit_m[u]);
+      if (uw == w) {
+        A.unit[n++] = RrUnit{off, u * n_seg, u, unit_m[u], unit_threshold[u], 0};
+        if (n == RR_UNITS_PER_LAUNCH) {
+          if (const int rc = rr_long_launch(w, A, n, st)) return rc;
+          n = 0;
+        }
+      }
+      off += 2 * RR_MAX_SYMBOLS * 32 * uw;
+    }
+    if (n > 0)
+      if (const int rc = rr_long_launch(w, A, n, st)) return rc;
   }
   return CFK_OK;
 }

@@ -3,7 +3,9 @@ device: same command line (``rr unit.fasta reads.fasta[.gz] output.fasta edit_di
 
 rr.cpp:73-90 aligns the unit and its reverse complement against every read with edlib in HW mode (the whole unit
 against any infix of the read, k = threshold) and copies the read to the output when either alignment exists.  Here the
-two alignments of every read are bit-parallel scans on the GPU (csrc/rr_filter.cu, cfk_rr_filter).
+two alignments of every read are bit-parallel scans on the GPU (csrc/rr_filter.cu): cfk_rr_filter, one thread per read
+and strand, for units of up to 3328 bases, and cfk_rr_filter_long, one warp per read and strand, for units of up to
+32768 bases.
 
 The command line streams (recruit_file): the read file goes through in chunks of a fixed size -- a reader thread reads
 or inflates it, a native scanner (csrc/seq_scan.cpp, cfk_seq_scan) finds the records of a chunk, the device gathers
@@ -68,13 +70,50 @@ def read_sequences(path):
             yield name, seq
 
 
+MAX_SHORT_UNIT = 3328  # the longest unit of cfk_rr_filter / cfk_rr_filter_units (rr_filter_kernel<52>)
+
+
+def is_long(unit):
+    """Does the unit take cfk_rr_filter_long (the warp-per-segment kernel) rather than cfk_rr_filter?"""
+    return len(unit) > MAX_SHORT_UNIT
+
+
 def build_masks(unit):
-    """-> (peq uint64[2, S, NW], sym_of uint8[256], NW) for cfk_rr_filter."""
-    lib = _lib.load()
+    """-> (peq uint64[2, S, NW], sym_of uint8[256], NW) for cfk_rr_filter: units of 1..3328 bases (build_long_masks
+    for longer ones)."""
     m = len(unit)
-    nw = int(lib.cfk_rr_words(m))
+    nw = int(_lib.load().cfk_rr_words(m))
     if nw < 0:
         raise CfkError(f"read recruitment: the unit has {m} bases; 1..3328 are supported")
+    return _masks(unit, nw)
+
+
+def build_long_masks(unit):
+    """-> (peq uint64[2, S, W, 32], sym_of uint8[256], W) for cfk_rr_filter_long: units of 1..32768 bases.  The masks of
+    build_masks padded with zero words to 32 W, lane-minor: peq[strand, s, k, L] is word L * W + k."""
+    m = len(unit)
+    w = int(_lib.load().cfk_rr_long_words(m))
+    if w < 0:
+        raise CfkError(f"read recruitment: the unit has {m} bases; 1..32768 are supported")
+    peq, sym_of, _ = _masks(unit, 32 * w)
+    return np.ascontiguousarray(peq.reshape(2, -1, 32, w).transpose(0, 1, 3, 2)), sym_of, w
+
+
+def _job_masks(unit, long_units):
+    """The masks of a unit the streaming form filters: build_long_masks for a unit of more than 3328 bases when
+    long_units is set, build_masks otherwise (which refuses such a unit, as the streaming form always has)."""
+    if not is_long(unit):
+        return build_masks(unit)
+    if not long_units:
+        raise CfkError(f"read recruitment: the unit has {len(unit)} bases; 1..3328 are supported "
+                       "(long_units=True, which the rr and rr_multi command lines pass, takes up to 32768)")
+    return build_long_masks(unit)
+
+
+def _masks(unit, nw):
+    """The match masks and symbol table of build_masks with nw words per strand."""
+    lib = _lib.load()
+    m = len(unit)
     n_sym = int(lib.cfk_rr_max_symbols())
     symbols = sorted(set((unit + reverse_complement(unit)).encode("latin-1")))  # both strands share one symbol table
     if len(symbols) > n_sym - 1:
@@ -92,13 +131,28 @@ def build_masks(unit):
     return peq, sym_of, nw
 
 
+def _segment_plan(lens, overlap, long_unit):
+    """The device work items of reads of lengths lens (int64): read r is cut into n_seg[r] = max(1, ceil(max(lens[r] -
+    overlap, 1) / step)) segments, segment j covering bases [j step, min(j step + step + overlap, lens[r])).  step is
+    SEGMENT, or with long_unit (a unit of more than 3328 bases in the plan) at least the overlap rounded up to 16, so a
+    unit of 32 kb does not scan every base about five times.  Either way step is a multiple of 16, so a segment starts
+    on a 16-byte boundary when its read does: the kernels read the text 16 bytes at a time.
+    -> (n_seg, seg_read, start, seg_len), the last three per segment: its read, first base and length."""
+    step = max(SEGMENT, (overlap + 15) // 16 * 16) if long_unit else SEGMENT
+    n_seg = np.maximum(1, -(-np.maximum(lens - overlap, 1) // step))
+    seg_read = np.repeat(np.arange(len(lens), dtype=np.int64), n_seg)
+    start = (np.arange(seg_read.size, dtype=np.int64) - np.repeat(np.cumsum(n_seg) - n_seg, n_seg)) * step
+    return n_seg, seg_read, start, np.minimum(step + overlap, lens[seg_read] - start)
+
+
 def recruit(unit, seqs, threshold, exact=False, engine=None):
     """keep[r] (bool) for every sequence, and with exact=True the infix edit distances int32[R, 2] (unit, reverse
-    complement) of cfk_rr_filter."""
+    complement) of cfk_rr_filter, or of cfk_rr_filter_long for a unit of more than 3328 bases (up to 32768)."""
     from .engine import default_engine
     eng = engine or default_engine()
     t = eng.torch
-    peq, sym_of, _ = build_masks(unit)
+    long_unit = is_long(unit)
+    peq, sym_of, _ = build_long_masks(unit) if long_unit else build_masks(unit)
     R = len(seqs)
     keep = np.zeros(R, dtype=bool)
     dist = np.zeros((R, 2), dtype=np.int32) if exact else None
@@ -121,21 +175,22 @@ def recruit(unit, seqs, threshold, exact=False, engine=None):
         seg_read = np.arange(end - start, dtype=np.int64)
         seg_off, seg_len = offs, lens
         if not exact and threshold >= 0:
-            overlap = len(unit) + int(threshold)
-            n_seg = np.maximum(1, -(-np.maximum(lens - overlap, 1) // SEGMENT))
-            seg_read = np.repeat(seg_read, n_seg)
-            first = np.cumsum(n_seg) - n_seg
-            j = np.arange(int(n_seg.sum()), dtype=np.int64) - np.repeat(first, n_seg)
-            seg_off = offs[seg_read] + j * SEGMENT
-            seg_len = np.minimum(SEGMENT + overlap, lens[seg_read] - j * SEGMENT)
+            _, seg_read, seg_start, seg_len = _segment_plan(lens, len(unit) + int(threshold), long_unit)
+            seg_off = offs[seg_read] + seg_start
         order = np.argsort(-seg_len, kind="stable").astype(np.int32)
         n = int(seg_read.size)
         d_keep = eng._zeros(n, t.uint8)
         d_dist = eng._empty(2 * n, t.int32) if exact else None
         d_text, d_offs, d_lens, d_order = eng._to_dev(text), eng._to_dev(seg_off), eng._to_dev(seg_len), eng._to_dev(order)
+        p = eng._p
         with eng._stage("rr_filter"):
-            _lib.call("cfk_rr_filter", eng._p(d_text), eng._p(d_offs), eng._p(d_lens), eng._p(d_order), n, eng._p(d_peq),
-                      eng._p(d_sym), len(unit), int(threshold), int(bool(exact)), eng._p(d_dist), eng._p(d_keep), eng._stream())
+            if long_unit:
+                m_t = np.array([len(unit), int(threshold)], dtype=np.int32)
+                _lib.call("cfk_rr_filter_long", p(d_text), p(d_offs), p(d_lens), p(d_order), n, 1, p(d_peq), p(d_sym),
+                          m_t.ctypes.data, m_t[1:].ctypes.data, int(bool(exact)), p(d_dist), p(d_keep), eng._stream())
+            else:
+                _lib.call("cfk_rr_filter", p(d_text), p(d_offs), p(d_lens), p(d_order), n, p(d_peq), p(d_sym), len(unit),
+                          int(threshold), int(bool(exact)), p(d_dist), p(d_keep), eng._stream())
         hit = np.zeros(end - start, dtype=bool)
         np.logical_or.at(hit, seg_read, d_keep[:n].cpu().numpy().astype(bool))
         keep[start:end] = hit
@@ -303,13 +358,13 @@ def _write_in_memory(unit, read_fn, path, threshold):
     _write_in_memory_jobs(read_fn, [(unit, path, threshold)])
 
 
-def _write_in_memory_jobs(read_fn, jobs):
+def _write_in_memory_jobs(read_fn, jobs, long_units=False):
     """_write_in_memory for every (unit, path, threshold) of jobs, reading the file once.  Every unit is checked before
-    the first output is written."""
+    the first output is written (long_units: as in recruit_file_units)."""
     records = list(read_sequences(read_fn))
     if records:
         for unit, _, _ in jobs:
-            build_masks(unit)
+            _job_masks(unit, long_units)
     seqs = [seq for _, seq in records]
     for unit, path, threshold in jobs:
         keep = recruit(unit, seqs, threshold) if records else np.zeros(0, dtype=bool)
@@ -317,7 +372,8 @@ def _write_in_memory_jobs(read_fn, jobs):
             f.write("".join(f">{name}\n{seq}\n" for (name, seq), k in zip(records, keep.tolist()) if k))
 
 
-def recruit_file(unit, read_fn, output_fn, threshold, chunk_bytes=CHUNK_BYTES, engine=None, stats=None):
+def recruit_file(unit, read_fn, output_fn, threshold, chunk_bytes=CHUNK_BYTES, engine=None, stats=None,
+                 long_units=False):
     """rr's whole run, from the read file to the output file: ``>name\\nsequence\\n`` of every read of read_fn (FASTA /
     FASTQ, plain or gzip) that holds the unit or its reverse complement within `threshold` edits (threshold < 0: every
     read), in input order -- the bytes the in-memory path (read_sequences + recruit) writes, streamed in chunks of
@@ -325,8 +381,8 @@ def recruit_file(unit, read_fn, output_fn, threshold, chunk_bytes=CHUNK_BYTES, e
     file beside it, then renamed).  An input without records gives an empty file and touches neither the device nor the
     unit; otherwise an invalid unit raises before any output exists.  A chunk with a byte >= 0x80 hands the whole run to
     the in-memory path.  stats: None, or a dict that receives seconds per host stage, device seconds per stage
-    (CUDA events, "device_s") and counts."""
-    return recruit_file_units([(unit, output_fn, threshold)], read_fn, chunk_bytes, engine, stats)
+    (CUDA events, "device_s") and counts.  long_units: as in recruit_file_units."""
+    return recruit_file_units([(unit, output_fn, threshold)], read_fn, chunk_bytes, engine, stats, long_units=long_units)
 
 
 def _part_file(output_fn):
@@ -341,7 +397,7 @@ def _part_file(output_fn):
             i += 1
 
 
-def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stats=None, devices=None):
+def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stats=None, devices=None, long_units=False):
     """recruit_file for every job (unit, output_fn, threshold) of `jobs` in one pass over read_fn: the file is read,
     inflated and scanned once, the device filters every chunk for all units in one launch per unit word class, and
     each output file gets the bytes recruit_file writes for that job alone.  All outputs appear together when the run
@@ -355,7 +411,11 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
     records are dealt out in contiguous ranges of about equal bases (_split_records), each worker runs the device
     work of its range, and every output is the workers' parts of each chunk in list order -- the same bytes.
     stats: as in recruit_file, plus "job_out_bytes" (output bytes per job), "devices" (the number of workers) and
-    "device_s_per_device" (device seconds per stage of each worker; "device_s" is their sum)."""
+    "device_s_per_device" (device seconds per stage of each worker; "device_s" is their sum).
+
+    long_units: also take units of 3329..32768 bases (cfk_rr_filter_long, one warp per segment and strand; the plan's
+    segment step grows to the overlap rounded up to 16 when that exceeds SEGMENT).  Without it such a unit raises
+    CfkError, the 3328-base limit this function has always had; the rr and rr_multi command lines pass it."""
     jobs = [(unit, output_fn, int(threshold)) for unit, output_fn, threshold in jobs]
     if not jobs:
         raise ValueError("recruit_file_units: no jobs")
@@ -388,13 +448,15 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
             files.append(f)
         try:
             try:
-                _stream([(unit, threshold) for unit, _, threshold in jobs], read_fn, files, chunk_bytes, engines, st)
+                _stream([(unit, threshold) for unit, _, threshold in jobs], read_fn, files, chunk_bytes, engines, st,
+                        long_units)
             finally:
                 for f in files:
                     f.close()
         except _Fallback as e:
             st["fallback"] = str(e)
-            _write_in_memory_jobs(read_fn, [(unit, tmp, threshold) for (unit, _, threshold), tmp in zip(jobs, tmps)])
+            _write_in_memory_jobs(read_fn, [(unit, tmp, threshold) for (unit, _, threshold), tmp in zip(jobs, tmps)],
+                                  long_units)
         for tmp, (_, output_fn, _) in zip(tmps, jobs):
             os.replace(tmp, output_fn)
     except BaseException:
@@ -508,16 +570,14 @@ class _Worker:
         # in the first half)
         S, F = 0, len(run.filtered)
         if F:
-            n_seg = np.maximum(1, -(-np.maximum(seq_len - run.overlap, 1) // SEGMENT))
+            n_seg, seg_read, seg_start, seg_len = _segment_plan(seq_len, run.overlap, run.n_short < F)
             S = int(n_seg.sum())
-            seg_read = np.repeat(np.arange(R, dtype=np.int64), n_seg)
-            j = np.arange(S, dtype=np.int64) - np.repeat(np.cumsum(n_seg) - n_seg, n_seg)
             nb = 8 * (3 * S + R + 1)
             hs = self._hbuf("seg", nb)
             seg = hs.numpy()[:nb].view(np.int64)
             seg_lens = seg[S:2 * S]
-            seg[:S] = rec[seg_read, 3] + j * SEGMENT
-            seg_lens[:] = np.minimum(SEGMENT + run.overlap, seq_len[seg_read] - j * SEGMENT)
+            seg[:S] = rec[seg_read, 3] + seg_start
+            seg_lens[:] = seg_len
             seg[2 * S] = 0
             np.cumsum(n_seg, out=seg[2 * S + 1:2 * S + R + 1])
             seg[2 * S + R + 1:].view(np.int32)[:S] = np.argsort(-seg_lens, kind="stable")
@@ -540,13 +600,19 @@ class _Worker:
         c = self._mark()
         d_keep = seg_ptr = None
         if S:
-            d_keep = self._dbuf("keep", F * S)  # [unit][segment]
+            d_keep = self._dbuf("keep", F * S)  # [unit][segment]: the short units' rows, then the long units'
             d_keep[:F * S].zero_()
             base = d_seg.data_ptr()
             seg_ptr = base + 16 * S
-            _lib.call("cfk_rr_filter_units", p(d_text), base, base + 8 * S, base + 8 * (2 * S + R + 1), S, F,
-                      p(self.d_peq), p(self.d_sym), run.unit_m.ctypes.data, run.unit_threshold.ctypes.data, p(d_keep),
-                      stream)
+            args = (p(d_text), base, base + 8 * S, base + 8 * (2 * S + R + 1), S)
+            k = run.n_short
+            if k:
+                _lib.call("cfk_rr_filter_units", *args, k, p(self.d_peq), p(self.d_sym), run.unit_m.ctypes.data,
+                          run.unit_threshold.ctypes.data, p(d_keep), stream)
+            if k < F:
+                _lib.call("cfk_rr_filter_long", *args, F - k, p(self.d_peq) + 8 * run.short_words,
+                          p(self.d_sym) + 256 * k, run.unit_m[k:].ctypes.data, run.unit_threshold[k:].ctypes.data, 0,
+                          None, p(d_keep) + k * S, stream)
         d = self._mark()
         d_sizes = self._dbuf("sizes", 4 * R, torch.int32)
         d_off = self._dbuf("off", 8 * (R + 1), torch.int64)
@@ -582,7 +648,7 @@ class _Worker:
         return parts
 
 
-def _stream(jobs, read_fn, files, chunk_bytes, engines, st):
+def _stream(jobs, read_fn, files, chunk_bytes, engines, st, long_units=False):
     """recruit_file_units' pipeline: jobs = [(unit, threshold)], files[j] receives job j's output, engines() -> one
     engine per worker (called once the first record is seen).  While the workers' devices work on chunk i, the reader
     thread reads ahead, this thread scans chunk i + 1 and deals its records out, and the writer thread writes chunk
@@ -593,7 +659,9 @@ def _stream(jobs, read_fn, files, chunk_bytes, engines, st):
     import torch
     host = {"alloc": lambda n: torch.empty(n, dtype=torch.uint8)}  # pageable until the first record is seen
     # the jobs that run the filter (threshold >= 0; the others keep every read), and their units' rows in d_peq / d_sym
+    # and d_keep: the units of cfk_rr_filter_units first, then the longer ones of cfk_rr_filter_long
     filtered = [j for j, (_, threshold) in enumerate(jobs) if threshold >= 0]
+    filtered.sort(key=lambda j: is_long(jobs[j][0]))  # stable: job order within each group
     # One segment plan serves every unit.  A hit within t edits spans at most |unit| + t read bases, so it lies wholly
     # inside some segment whenever the segments overlap by at least that much; and a segment is an infix of its read,
     # so a hit inside a segment is a hit in the read.  Overlapping by the largest |unit| + t of all jobs therefore
@@ -604,6 +672,7 @@ def _stream(jobs, read_fn, files, chunk_bytes, engines, st):
         unit_m=np.array([len(jobs[j][0]) for j in filtered], dtype=np.int32),
         unit_threshold=np.array([jobs[j][1] for j in filtered], dtype=np.int32),
         overlap=max((len(jobs[j][0]) + jobs[j][1] for j in filtered), default=0),
+        n_short=sum(not is_long(jobs[j][0]) for j in filtered), short_words=0,
         timed=st["device_s"] is not None, abort=threading.Event(), writer_err=[])
     workers, writer, writer_q = [], None, queue.Queue()
 
@@ -624,11 +693,12 @@ def _stream(jobs, read_fn, files, chunk_bytes, engines, st):
 
     def start():
         nonlocal writer
-        masks = [build_masks(unit) for unit, _ in jobs]  # raises on an invalid unit, before any output
+        masks = [_job_masks(unit, long_units) for unit, _ in jobs]  # raises on an invalid unit, before any output
         peq = sym_of = None
         if filtered:
             peq = np.concatenate([masks[j][0].reshape(-1) for j in filtered]).view(np.int64)
             sym_of = np.concatenate([masks[j][1] for j in filtered])
+            run.short_words = sum(masks[j][0].size for j in filtered[:run.n_short])
         for g, eng in enumerate(engines()):
             workers.append(_Worker(g, eng, run, peq, sym_of))
         host["alloc"] = lambda n: torch.empty(n, dtype=torch.uint8, pin_memory=True)
@@ -709,8 +779,8 @@ def main(argv=None):
         threshold = int(argv[3])
     except ValueError:
         threshold = 0  # std::atoi
-    unit = next(read_sequences(unit_fn))[1]
-    recruit_file(unit, read_fn, output_fn, threshold)
+    unit = next(read_sequences(unit_fn))[1]  # 1..32768 bases (edlib's rr takes any length)
+    recruit_file(unit, read_fn, output_fn, threshold, long_units=True)
     return 0
 
 
@@ -720,7 +790,8 @@ UNITS_USAGE = ("Usage: rr_multi.py reads.fasta[.gz|.fastq] unit1.fasta output1.f
 
 def main_units(argv=None):
     """``rr_multi.py [--gpus N] reads unit1 output1 threshold1 [unit2 output2 threshold2 ...]``: what one rr run per
-    triple writes, from one pass over the read file (recruit_file_units).  Each unit is the first record of its file;
+    triple writes, from one pass over the read file (recruit_file_units).  Each unit is the first record of its file,
+    of 1..32768 bases;
     thresholds are read as main() reads them.  --gpus N runs on cuda:0 .. N-1 (devices=); without it, on one device.
     A wrong argument count, or an N that is not an integer from 1 to the number of visible devices: the usage on
     stderr, status 2."""
@@ -746,7 +817,7 @@ def main_units(argv=None):
         except ValueError:
             threshold = 0  # std::atoi, as in main()
         jobs.append((next(read_sequences(unit_fn))[1], output_fn, threshold))
-    recruit_file_units(jobs, argv[0], devices=devices)
+    recruit_file_units(jobs, argv[0], devices=devices, long_units=True)
     return 0
 
 

@@ -210,6 +210,25 @@ int cfk_rr_filter_units(const uint8_t* text, const int64_t* seg_off, const int64
                         int32_t n_units, const uint64_t* peq, const uint8_t* sym_of, const int32_t* unit_m,
                         const int32_t* unit_threshold, uint8_t* out_keep, cfk_stream_t stream);
 
+/* Units of 1..32768 bases (read_recruitment.recruit, and the streaming form with long_units, take this for units over
+ * 3328 bases): one warp per (segment, strand), the unit's 64-bit words split over the 32 lanes, W consecutive words per lane;
+ * cfk_rr_long_words(m) = the least W of {2, 4, 8, 16} with ceil(ceil(m / 64) / W) <= 32, or -1 outside 1..32768.
+ *   peq             each unit's [2][cfk_rr_max_symbols()][W][32] block, lane-minor: entry [strand][s][k][L] is word
+ *                   L * W + k of cfk_rr_filter's masks (zero past the unit), the blocks of units 0 .. U-1 one after
+ *                   another
+ *   sym_of          [U][256], one symbol table per unit
+ *   unit_m, unit_threshold   HOST int32[U]
+ *   out_dist        NULL, or [U][2 * n_seg]: as cfk_rr_filter's out_dist, per unit
+ *   out_keep        [U][n_seg], zeroed by the caller
+ * Every size and unit_m is checked before anything is launched.  One launch per W present (more for a W of more than
+ * 64 units), all on `stream`.  exact != 0 never stops early, as in cfk_rr_filter; the distances and keep bits are
+ * those of cfk_rr_filter for every unit both take. */
+int cfk_rr_long_words(int32_t m);
+int cfk_rr_filter_long(const uint8_t* text, const int64_t* seg_off, const int64_t* seg_len, const int32_t* order, int64_t n_seg,
+                       int32_t n_units, const uint64_t* peq, const uint8_t* sym_of, const int32_t* unit_m,
+                       const int32_t* unit_threshold, int32_t exact, int32_t* out_dist, uint8_t* out_keep,
+                       cfk_stream_t stream);
+
 /* ---- streaming read recruitment: read file text in, output file text out ---------------------------------------
  * cfk_seq_scan (HOST code) finds the records of one chunk of FASTA / FASTQ text exactly as read_sequences() yields them
  * (centroflye_b200/read_recruitment.py:29-55, the restatement of rr.cpp's kseq_read loop): "\n", "\r\n" and a lone "\r"
