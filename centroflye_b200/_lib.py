@@ -48,6 +48,10 @@ SIGNATURES = {
     "cfk_rr_gather": (_int, [_p, _p, _i64, _p, _i64, _p]),
     "cfk_rr_keep_sizes": (_int, [_p, _p, _p, _i64, _p, _p]),
     "cfk_rr_emit": (_int, [_p, _p, _p, _p, _i64, _i64, _p, _p]),
+    "cfk_bgzf_blocks": (_int, [_p, _i64, _p, _i64, _p]),  # host pointers
+    "cfk_bgzf_inflate": (_int, [_p, _p, _i64, _p, _p, _p]),
+    "cfk_bam_scan": (_int, [_p, _i64, _i32, _i32, _i64, _i64, _p, _i64, _p, _p]),  # host pointers
+    "cfk_rr_bam_gather": (_int, [_p, _p, _p, _i64, _p, _i64, _p]),
     "cfk_placer_best_blocks": (_int, []),
     "cfk_placer_add_read": (_int, [_p, _p, _i64, _i32, _i64, _i64, _u32, _p, _p, _i64, _p, _p, _i64, _p, _p]),
     "cfk_placer_initial_pairs": (_int, [_p, _i64, _p, _p, _i64, _p, _p]),

@@ -12,8 +12,10 @@ STREAM_SRC = os.path.join(HERE, "csrc", "docfreq_stream.cu")  # stage A, two-pha
 PLACER_SRC = os.path.join(HERE, "csrc", "placer.cu")  # read_placer scoring on the cloud CSR (row f rank 2)
 RR_SRC = os.path.join(HERE, "csrc", "rr_filter.cu")  # read recruitment pre-filter (row f rank 4)
 SCAN_SRC = os.path.join(HERE, "csrc", "seq_scan.cpp")  # host-side FASTA / FASTQ record scanner of the streaming filter
+BGZF_SRC = os.path.join(HERE, "csrc", "bgzf.cu")  # BGZF blocks inflated on the device (compressed read files)
+BAM_SCAN_SRC = os.path.join(HERE, "csrc", "bam_scan.cpp")  # host-side BGZF block finder and BAM record scanner
 COMMON_HDR = os.path.join(HERE, "csrc", "cfk_common.cuh")
-SOURCES = [SRC, STREAM_SRC, PLACER_SRC, RR_SRC, INGEST_SRC, WRITER_SRC, SCAN_SRC]
+SOURCES = [SRC, STREAM_SRC, PLACER_SRC, RR_SRC, BGZF_SRC, INGEST_SRC, WRITER_SRC, SCAN_SRC, BAM_SCAN_SRC]
 HDR = os.path.join(os.path.dirname(HERE), "include", "cfk.h")
 OUT = os.path.join(HERE, "libcfk.so")
 

@@ -293,6 +293,34 @@ __global__ void __launch_bounds__(COPY_THREADS) rr_gather_kernel(const uint8_t* 
   reinterpret_cast<uint4*>(text)[q0 >> 4] = pack16(b);
 }
 
+// text[q] = base q - rec[r][3] of BAM record r (rec = [n][4] as cfk_bam_scan writes it, bam_seq = [n][2]: offset of the
+// 4-bit SEQ in raw, reverse flag), 0 between records.  Every record starts on a 16-byte boundary, so the 16 bytes of a
+// thread belong to one record's slot.
+__global__ void __launch_bounds__(COPY_THREADS) rr_bam_gather_kernel(const uint8_t* __restrict__ raw,
+                                                                     const int64_t* __restrict__ bam_seq,
+                                                                     const int64_t* __restrict__ rec, int64_t n,
+                                                                     uint8_t* __restrict__ text, int64_t text_bytes) {
+  const int64_t q0 = ((int64_t)blockIdx.x * COPY_THREADS + threadIdx.x) * 16;
+  if (q0 >= text_bytes) return;
+  const int64_t r = last_at_or_below(rec + 3, 4, n, q0);
+  const int64_t at = q0 - rec[4 * r + 3], len = rec[4 * r + 2], src = bam_seq[2 * r];
+  const bool rev = bam_seq[2 * r + 1] != 0;
+  const char* code = rev ? "=TGKCYSBAWRDMHVN" : "=ACMGRSVTWYHKDBN";  // complement = the 4 bits reversed
+  uint8_t b[16];
+#pragma unroll
+  for (int k = 0; k < 16; ++k) {
+    const int64_t i = at + k;
+    uint8_t c = 0;
+    if (i < len) {
+      const int64_t j = rev ? len - 1 - i : i;
+      const uint8_t v = raw[src + (j >> 1)];
+      c = code[(j & 1) ? (v & 15) : (v >> 4)];
+    }
+    b[k] = c;
+  }
+  reinterpret_cast<uint4*>(text)[q0 >> 4] = pack16(b);
+}
+
 // sizes[r] = bytes of ">name\nsequence\n" when record r is kept, else 0.  A record is kept when any of its segments
 // seg_keep[seg_ptr[r] .. seg_ptr[r + 1]) hit; seg_keep == NULL keeps every record.
 __global__ void rr_keep_sizes_kernel(const uint8_t* __restrict__ seg_keep, const int64_t* __restrict__ seg_ptr,
@@ -450,6 +478,18 @@ int cfk_rr_gather(const uint8_t* raw, const int64_t* pieces, int64_t n_pieces, u
   rr_gather_kernel<<<(unsigned)blocks_for(text_bytes / 16, COPY_THREADS), COPY_THREADS, 0, (cudaStream_t)stream>>>(
       raw, pieces, n_pieces, text, text_bytes);
   CFK_CHECK_LAUNCH("rr_gather_kernel", 1);
+  return CFK_OK;
+}
+
+int cfk_rr_bam_gather(const uint8_t* raw, const int64_t* bam_seq, const int64_t* records, int64_t n_records, uint8_t* text,
+                      int64_t text_bytes, cfk_stream_t stream) {
+  if (n_records < 0 || text_bytes < 0 || (text_bytes & 15) != 0 || ((uintptr_t)text & 15u) != 0 ||
+      (text_bytes > 0 && n_records == 0))
+    return fail(CFK_ERR_INVALID, "cfk_rr_bam_gather: bad sizes, or text not 16-byte aligned");
+  if (text_bytes == 0) return CFK_OK;
+  rr_bam_gather_kernel<<<(unsigned)blocks_for(text_bytes / 16, COPY_THREADS), COPY_THREADS, 0, (cudaStream_t)stream>>>(
+      raw, bam_seq, records, n_records, text, text_bytes);
+  CFK_CHECK_LAUNCH("rr_bam_gather_kernel", 1);
   return CFK_OK;
 }
 

@@ -16,6 +16,12 @@ word class covers every unit, and each output gets the bytes recruit_file writes
 its one-job case; main_units / scripts/rr_multi.py is its command line); with devices= it deals every chunk's records
 out to several GPUs in contiguous ranges, and the outputs are the same bytes.  read_sequences() and
 recruit() are the in-memory form of the same computation, and the specification the streaming form is tested against.
+
+The read file may be FASTA / FASTQ, plain, gzip or bgzip, or unaligned BAM; nothing but its bytes tells them apart.  A
+file whose first gzip member is a BGZF block (bgzip, BAM) is inflated on the run's first device (_DeviceInflater:
+cfk_bgzf_blocks finds the blocks on the host, csrc/bgzf.cu inflates a chunk's worth at once); other gzip files are
+inflated by zlib on the reader thread.  A stream that starts with "BAM\\1" is scanned by cfk_bam_scan instead of
+cfk_seq_scan and gathered by cfk_rr_bam_gather; it yields the reads ``samtools fastq -n -F 0x900`` writes (_read_bam).
 """
 import gzip
 import os
@@ -44,10 +50,16 @@ def reverse_complement(unit):
 def read_sequences(path):
     """(name, sequence) of every FASTA / FASTQ record, plain or gzip -- what kseq_read yields: the name is the header up
     to the first whitespace, sequence lines are joined until a line starting with '>', '@' or '+'; after '+' as many
-    quality characters as the sequence has bases are skipped."""
+    quality characters as the sequence has bases are skipped.  A file whose (inflated) bytes start with "BAM\\1" is
+    unaligned BAM, read by _read_bam."""
     with open(path, "rb") as f:
         magic = f.read(2)
     opener = gzip.open if magic == b"\x1f\x8b" else open
+    with opener(path, "rb") as f:
+        bam = f.read(4) == BAM_MAGIC
+    if bam:
+        yield from _read_bam(path, opener)
+        return
     with opener(path, "rt") as f:
         line = f.readline()
         while line:
@@ -68,6 +80,52 @@ def read_sequences(path):
                     left -= len(line.rstrip("\r\n"))
                     line = f.readline()
             yield name, seq
+
+
+BAM_MAGIC = b"BAM\1"
+_BAM_PAIRS = [a + b for a in "=ACMGRSVTWYHKDBN" for b in "=ACMGRSVTWYHKDBN"]  # one SEQ byte -> its two bases
+_BAM_COMPLEMENT = str.maketrans("=ACMGRSVTWYHKDBN", "=TGKCYSBAWRDMHVN")
+
+
+def _bam_bases(packed, l_seq, reverse):
+    """The bases of a BAM SEQ field (4-bit codes, two per byte), reverse-complemented when `reverse`."""
+    seq = "".join(map(_BAM_PAIRS.__getitem__, packed))[:l_seq]
+    return seq[::-1].translate(_BAM_COMPLEMENT) if reverse else seq
+
+
+def _read_bam(path, opener):
+    """(name, sequence) of every record of an unaligned BAM file (SAM spec §4.2), read with `opener` and struct: the FASTQ
+    records ``samtools fastq -n -F 0x900`` writes -- secondary and supplementary alignments (flag & 0x900) yield
+    nothing, the name is QNAME (no /1 or /2), the sequence is SEQ over "=ACMGRSVTWYHKDBN", reverse-complemented (A-T, C-G,
+    M-K, R-Y, H-D, B-V; W, S, N and = are their own complements) when flag & 0x10 is set.  Quality, CIGAR and tags are
+    ignored.  That this is samtools' output is the intent; it has not been checked against samtools itself."""
+    import struct
+    with opener(path, "rb") as f:
+        def exact(n):
+            b = f.read(n)
+            if len(b) != n:
+                raise EOFError("the BAM file ends inside a record or its header")
+            return b
+        exact(4)
+        exact(struct.unpack("<i", exact(4))[0])  # header text
+        for _ in range(struct.unpack("<i", exact(4))[0]):  # references: name, length
+            exact(struct.unpack("<i", exact(4))[0] + 4)
+        while True:
+            head = f.read(4)
+            if not head:
+                return
+            block_size = struct.unpack("<i", head if len(head) == 4 else exact(4))[0]
+            if block_size < 32:
+                raise ValueError(f"BAM record with block_size {block_size}")
+            rec = exact(block_size)
+            l_read_name = rec[8]
+            n_cigar_op, flag, l_seq = struct.unpack_from("<HHi", rec, 12)
+            at = 32 + l_read_name + 4 * n_cigar_op
+            if l_read_name == 0 or l_seq < 0 or at + (l_seq + 1) // 2 + l_seq > block_size:
+                raise ValueError("BAM record with fields past its block_size")
+            if not flag & 0x900:
+                yield rec[32:32 + l_read_name - 1].decode("ascii"), _bam_bases(rec[at:at + (l_seq + 1) // 2], l_seq,
+                                                                                flag & 0x10)
 
 
 MAX_SHORT_UNIT = 3328  # the longest unit of cfk_rr_filter / cfk_rr_filter_units (rr_filter_kernel<52>)
@@ -207,11 +265,139 @@ _BLOCK_BYTES = 8 << 20   # the reader thread's unit of readinto / inflate; four 
 _REC_BYTES_PER_SLOT, _PIECE_BYTES_PER_SLOT = 128, 64
 
 
-def _open_binary(path):
-    """The read file as bytes, inflated when it starts with the gzip magic (like read_sequences)."""
+def _open_binary(path, inflate=None):
+    """The read file as bytes, inflated when it starts with the gzip magic (like read_sequences).  inflate: None, or
+    (device, chunk_bytes, stats) -- a file whose first member is a BGZF block is then inflated on that device
+    (_DeviceInflater; device is a callable returning a torch.device)."""
     with open(path, "rb") as f:
-        magic = f.read(2)
-    return gzip.open(path, "rb") if magic == b"\x1f\x8b" else open(path, "rb")
+        head = f.read(_BGZF_MAX_MEMBER)
+    if head[:2] != b"\x1f\x8b":
+        return open(path, "rb")
+    if inflate is not None and _bgzf_blocks(np.frombuffer(head, dtype=np.uint8), 1)[0] == 1:
+        return _DeviceInflater(path, *inflate)
+    return gzip.open(path, "rb")
+
+
+_BGZF_MAX_MEMBER = 1 << 16  # BSIZE is 16 bits: no BGZF member is larger
+_BGZF_INCOMPLETE, _BGZF_NOT_BGZF = 1, 2  # cfk_bgzf_blocks flags (include/cfk.h)
+_BGZF_STATUS = {1: "not a valid DEFLATE stream", 2: "inflated length differs from ISIZE", 3: "CRC32 mismatch"}
+
+
+def _bgzf_blocks(buf, max_blocks, rows=None):
+    """cfk_bgzf_blocks on buf (uint8 array) -> (n_blocks, consumed, inflated bytes, flags); rows: int64[max_blocks, 5]."""
+    out = np.zeros(4, dtype=np.int64)
+    if rows is None:
+        rows = np.zeros((max_blocks, 5), dtype=np.int64)
+    _lib.call("cfk_bgzf_blocks", buf.ctypes.data, buf.size, rows.ctypes.data, max_blocks, out.ctypes.data)
+    return tuple(out.tolist())
+
+
+class _DeviceInflater:
+    """A BGZF file's inflated bytes, read with readinto() like a gzip.GzipFile: cfk_bgzf_blocks finds the blocks of the
+    compressed bytes, enough of them to fill a chunk go to the device in one copy, cfk_bgzf_inflate inflates them on a
+    stream of its own, and the inflated bytes come back into a pinned buffer.  From a member that is not BGZF on
+    (or a last member cut short) the rest of the file goes to gzip.GzipFile on the host, so every file reads to the
+    bytes -- or the error -- gzip.open gives.  A block the device rejects raises gzip.BadGzipFile with its file offset.
+    stats["inflate_s"] gets the device seconds of the kernel, stats["bgzf_blocks"] the number of blocks."""
+
+    def __init__(self, path, device, chunk_bytes, stats):
+        import torch
+        self.torch, self.device, self.stats = torch, device(), stats
+        self.f = open(path, "rb")
+        self.max_blocks = max(1, chunk_bytes // _BGZF_MAX_MEMBER)
+        self.cap = self.max_blocks * _BGZF_MAX_MEMBER  # compressed bytes that always hold max_blocks blocks
+        self.buf = self.have = self.file_off = None  # compressed bytes buf[:have], from file offset file_off
+        self.out, self.at, self.n = None, 0, 0  # inflated bytes out[at:n] not yet read
+        self.tail, self.file_eof = None, False
+        self.stream = self.dev = None
+        stats.setdefault("inflate_s", 0.0)
+        stats.setdefault("bgzf_blocks", 0)
+
+    def readinto(self, view):
+        view = np.frombuffer(view, dtype=np.uint8)
+        k = 0
+        while k < view.size:
+            if self.at < self.n:
+                take = min(view.size - k, self.n - self.at)
+                view[k:k + take] = self.out[self.at:self.at + take]
+                k, self.at = k + take, self.at + take
+            elif self.tail is not None:
+                got = self.tail.readinto(view[k:])
+                if not got:
+                    break
+                k += got
+            elif not self._fill():
+                break
+        return k
+
+    def _setup(self):
+        torch = self.torch
+        torch.cuda.set_device(self.device)  # the reader thread launches on the run's first device
+        self.stream = torch.cuda.Stream(self.device)
+        pinned = lambda n: torch.empty(n, dtype=torch.uint8, pin_memory=True)  # noqa: E731
+        dev = lambda n: torch.empty(n, dtype=torch.uint8, device=self.device)  # noqa: E731
+        B = self.max_blocks
+        self.h_comp, self.h_rows = pinned(self.cap), pinned(40 * B)
+        self.h_out, self.h_status = pinned(B * _BGZF_MAX_MEMBER), pinned(4 * B)
+        self.dev = {"comp": dev(self.cap), "rows": dev(40 * B), "out": dev(B * _BGZF_MAX_MEMBER), "status": dev(4 * B)}
+        self.buf, self.have, self.file_off = self.h_comp.numpy(), 0, 0
+        self.rows = self.h_rows.numpy().view(np.int64).reshape(B, 5)
+        self.out = self.h_out.numpy()
+
+    def _fill(self):
+        """Inflates the next blocks into self.out; False at the end of the file."""
+        torch = self.torch
+        if self.dev is None:
+            self._setup()
+        while True:
+            while not self.file_eof and self.have < self.cap:  # enough compressed bytes for max_blocks blocks
+                got = self.f.readinto(memoryview(self.buf)[self.have:])
+                self.file_eof = not got
+                self.have += got
+            n, consumed, total, flags = _bgzf_blocks(self.buf[:self.have], self.max_blocks, self.rows)
+            if n or flags or consumed < self.have:
+                break
+            self.have, self.file_off = 0, self.file_off + consumed  # nothing but zero padding: skipped, read on
+            if self.file_eof:
+                return False
+        if n == 0:
+            # a member that is not BGZF, or a last member cut short: the rest of the file, from there, on the host
+            self.f.seek(self.file_off + consumed)
+            self.tail = gzip.GzipFile(fileobj=self.f, mode="rb")
+            return True
+        d = self.dev
+        status = self.h_status.numpy()[:4 * n].view(np.int32)
+        with torch.cuda.stream(self.stream):
+            d["comp"][:consumed].copy_(self.h_comp[:consumed], non_blocking=True)
+            d["rows"][:40 * n].copy_(self.h_rows[:40 * n], non_blocking=True)
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            _lib.call("cfk_bgzf_inflate", d["comp"].data_ptr(), d["rows"].data_ptr(), n, d["out"].data_ptr(),
+                      d["status"].data_ptr(), self.stream.cuda_stream)
+            b.record()
+            self.h_out[:total].copy_(d["out"][:total], non_blocking=True)
+            self.h_status[:4 * n].copy_(d["status"][:4 * n], non_blocking=True)
+        self.stream.synchronize()
+        self.stats["inflate_s"] += a.elapsed_time(b) / 1e3
+        self.stats["bgzf_blocks"] += n
+        bad = np.flatnonzero(status)
+        if bad.size:
+            i = int(bad[0])
+            start = 0 if i == 0 else int(self.rows[i - 1, 0] + self.rows[i - 1, 1] + 8)
+            while self.buf[start] == 0:  # zero padding before the member
+                start += 1
+            raise gzip.BadGzipFile(f"BGZF block at file offset {self.file_off + start}: "
+                                   f"{_BGZF_STATUS.get(int(status[i]), 'bad status')}")
+        self.at, self.n = 0, total
+        self.buf[:self.have - consumed] = self.buf[consumed:self.have]
+        self.have -= consumed
+        self.file_off += consumed
+        return True
+
+    def close(self):
+        if self.tail is not None:
+            self.tail.close()
+        self.f.close()
 
 
 class _Fallback(Exception):
@@ -222,8 +408,8 @@ class _Fallback(Exception):
 class _BlockReader:
     """Reads (or inflates) the file block by block on a thread of its own; readinto and zlib release the GIL."""
 
-    def __init__(self, path, block, depth=4):
-        self.f = _open_binary(path)
+    def __init__(self, path, block, depth=4, inflate=None):
+        self.f = _open_binary(path, inflate)
         self.block, self.seconds = block, 0.0
         self.free, self.full = queue.Queue(), queue.Queue()
         for _ in range(depth):
@@ -271,17 +457,23 @@ def _grown(store, key, nbytes, make):
     return buf
 
 
-def _scan_chunks(read_fn, chunk_bytes, host, stats):
-    """Chunks of the read file cut at record boundaries by cfk_seq_scan: yields (slot, raw, records, pieces, text_bytes)
-    where raw (uint8 tensor) holds the chunk's text, records int64[n, 4] and pieces int64[m, 3] are the scanner's tables
-    (numpy views of tensors in `host`, made by host["alloc"]).  Two slots alternate: what is yielded stays valid until
-    the next-but-one chunk is asked for.  A chunk without a complete record is doubled until it has one, so an
-    ultra-long read fits any chunk size."""
+def _scan_chunks(read_fn, chunk_bytes, host, stats, inflate_device=None):
+    """Chunks of the read file cut at record boundaries by cfk_seq_scan, or by cfk_bam_scan when the (inflated) file
+    starts with the BAM magic: yields (slot, raw, records, pieces, text_bytes, bam) where raw (uint8 tensor) holds the
+    chunk's bytes, records int64[n, 4] and pieces are the scanner's tables (numpy views of tensors in `host`, made by
+    host["alloc"]): int64[m, 3] from cfk_seq_scan, or cfk_bam_scan's bam_seq int64[n, 2] when bam is set.  Two slots
+    alternate: what is yielded stays valid until the next-but-one chunk is asked for.  A chunk without a complete
+    record is doubled until it has one, so an ultra-long read (or a BAM header) fits any chunk size; bytes before the
+    first complete record that hold none (lines outside records, the BAM header, secondary alignments) are dropped
+    instead.  inflate_device: None inflates gzip input on the host; a callable returning a torch.device inflates a
+    BGZF file on that device (_DeviceInflater)."""
     alloc = lambda key, nbytes: _grown(host, key, nbytes, host["alloc"])  # noqa: E731
-    reader = _BlockReader(read_fn, max(1 << 16, min(chunk_bytes, _BLOCK_BYTES)))
+    inflate = None if inflate_device is None else (inflate_device, chunk_bytes, stats)
+    reader = _BlockReader(read_fn, max(1 << 16, min(chunk_bytes, _BLOCK_BYTES)), inflate=inflate)
     out = np.zeros(5, dtype=np.int64)
     carry, eof, slot, table_scale = np.zeros(0, dtype=np.uint8), False, 0, 1
     blk, at, k = None, 0, 0  # the reader's block being taken apart: blk[at:k] is not in a chunk yet
+    bam, stream_off, rec_index = None, 0, 0  # BAM: raw[0]'s offset in the inflated stream, alignments before it
     try:
         while True:
             n, target = carry.size, max(chunk_bytes, carry.size)
@@ -308,13 +500,20 @@ def _scan_chunks(read_fn, chunk_bytes, host, stats):
                 max_rec = table_scale * max(64, n // _REC_BYTES_PER_SLOT)
                 max_piece = table_scale * max(64, n // _PIECE_BYTES_PER_SLOT)
                 rec = alloc((slot, "rec"), 32 * max_rec).numpy().view(np.int64)
-                piece = alloc((slot, "piece"), 24 * max_piece).numpy().view(np.int64)
                 buf = raw.numpy()
-                _lib.call("cfk_seq_scan", buf.ctypes.data, n, int(end), rec.ctypes.data, max_rec, piece.ctypes.data,
-                          max_piece, out.ctypes.data)
+                if bam is None:
+                    bam = bytes(buf[:4]) == BAM_MAGIC
+                if bam:
+                    piece = alloc((slot, "piece"), 16 * max_rec).numpy().view(np.int64)
+                    _lib.call("cfk_bam_scan", buf.ctypes.data, n, int(end), int(stream_off == 0), rec_index, stream_off,
+                              rec.ctypes.data, max_rec, piece.ctypes.data, out.ctypes.data)
+                else:
+                    piece = alloc((slot, "piece"), 24 * max_piece).numpy().view(np.int64)
+                    _lib.call("cfk_seq_scan", buf.ctypes.data, n, int(end), rec.ctypes.data, max_rec, piece.ctypes.data,
+                              max_piece, out.ctypes.data)
                 stats["assemble_s"] += t1 - t0
                 stats["scan_s"] += time.perf_counter() - t1
-                n_rec, n_piece, consumed, text_bytes, flags = out.tolist()
+                n_rec, n_piece, consumed, text_bytes, flags = out.tolist()  # BAM: n_piece = alignments consumed
                 if flags & _SCAN_NOT_ASCII:
                     raise _Fallback("a byte >= 0x80 in the read file")
                 if n_rec:
@@ -323,12 +522,20 @@ def _scan_chunks(read_fn, chunk_bytes, host, stats):
                     table_scale *= 2
                 elif end:
                     return
+                elif consumed:  # nothing to yield in buf[:consumed]: keep only the rest
+                    buf[:n - consumed] = buf[consumed:n]
+                    n -= consumed
+                    stream_off += consumed
+                    rec_index += n_piece if bam else 0
                 else:
                     target = 2 * n
-            yield slot, raw[:n], rec[:4 * n_rec].reshape(-1, 4), piece[:3 * n_piece].reshape(-1, 3), text_bytes
+            table = piece[:2 * n_rec].reshape(-1, 2) if bam else piece[:3 * n_piece].reshape(-1, 3)
+            yield slot, raw[:n], rec[:4 * n_rec].reshape(-1, 4), table, text_bytes, bam
             if end and consumed == n:
                 return
             carry, slot = buf[consumed:n], slot ^ 1
+            stream_off += consumed
+            rec_index += n_piece if bam else 0
     finally:
         stats["read_s"] += reader.seconds
         reader.close()
@@ -343,8 +550,13 @@ def scan_sequences(path, chunk_bytes=CHUNK_BYTES):
     import torch
     host = {"alloc": lambda n: torch.empty(n, dtype=torch.uint8)}
     stats = {"assemble_s": 0.0, "scan_s": 0.0, "read_s": 0.0}
-    for _, raw, rec, piece, _ in _scan_chunks(path, chunk_bytes, host, stats):
+    for _, raw, rec, piece, _, bam in _scan_chunks(path, chunk_bytes, host, stats):
         buf, p = raw.numpy(), 0
+        if bam:
+            for (name_off, name_len, seq_len, _), (src, rev) in zip(rec.tolist(), piece.tolist()):
+                yield (buf[name_off:name_off + name_len].tobytes().decode(),
+                       _bam_bases(buf[src:src + (seq_len + 1) // 2].tobytes(), seq_len, rev))
+            continue
         for name_off, name_len, seq_len, seq_dst in rec.tolist():
             parts = []
             while p < len(piece) and piece[p, 2] < seq_dst + seq_len:
@@ -375,11 +587,11 @@ def _write_in_memory_jobs(read_fn, jobs, long_units=False):
 def recruit_file(unit, read_fn, output_fn, threshold, chunk_bytes=CHUNK_BYTES, engine=None, stats=None,
                  long_units=False):
     """rr's whole run, from the read file to the output file: ``>name\\nsequence\\n`` of every read of read_fn (FASTA /
-    FASTQ, plain or gzip) that holds the unit or its reverse complement within `threshold` edits (threshold < 0: every
-    read), in input order -- the bytes the in-memory path (read_sequences + recruit) writes, streamed in chunks of
+    FASTQ, plain, gzip or bgzip, or unaligned BAM) that holds the unit or its reverse complement within `threshold`
+    edits (threshold < 0: every read), in input order -- the bytes the in-memory path (read_sequences + recruit) writes, streamed in chunks of
     about chunk_bytes.  The output appears under output_fn only when the run has finished (it is written to a temporary
     file beside it, then renamed).  An input without records gives an empty file and touches neither the device nor the
-    unit; otherwise an invalid unit raises before any output exists.  A chunk with a byte >= 0x80 hands the whole run to
+    unit, except that a BGZF file (bgzip, BAM) is inflated on the device whether it holds records or not; otherwise an invalid unit raises before any output exists.  A chunk with a byte >= 0x80 hands the whole run to
     the in-memory path.  stats: None, or a dict that receives seconds per host stage, device seconds per stage
     (CUDA events, "device_s") and counts.  long_units: as in recruit_file_units."""
     return recruit_file_units([(unit, output_fn, threshold)], read_fn, chunk_bytes, engine, stats, long_units=long_units)
@@ -402,7 +614,7 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
     inflated and scanned once, the device filters every chunk for all units in one launch per unit word class, and
     each output file gets the bytes recruit_file writes for that job alone.  All outputs appear together when the run
     has finished; on an error none is created or modified.  An input without records gives empty files and checks no
-    unit; otherwise every unit is checked, with recruit_file's errors, before any output exists.  A byte >= 0x80 hands
+    unit (a BGZF input is still inflated on the device: the first of `devices`, or the engine's); otherwise every unit is checked, with recruit_file's errors, before any output exists.  A byte >= 0x80 hands
     the whole run to the in-memory path (the file is read once, then recruit() per job).  Raises ValueError for no jobs,
     or for two jobs with the same output file.  Host and device memory follow chunk_bytes times the number of jobs.
 
@@ -426,6 +638,9 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
         def engines():
             from .engine import default_engine
             return [engine or default_engine()]
+
+        def inflate_device():
+            return engines()[0].device
         n_dev = 1
     else:
         devices = list(devices)
@@ -435,9 +650,13 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
         def engines():
             from .engine import Engine
             return [Engine(d) for d in devices]
+
+        def inflate_device():
+            import torch
+            return torch.device(devices[0])  # as Engine(devices[0]) takes it
         n_dev = len(devices)
     st = {key: 0.0 for key in ("read_s", "assemble_s", "scan_s", "plan_s", "wait_s", "write_s")}
-    st.update(chunks=0, records=0, bases=0, out_bytes=0, job_out_bytes=[0] * len(jobs), fallback=None,
+    st.update(inflate_s=0.0, bgzf_blocks=0, chunks=0, records=0, bases=0, out_bytes=0, job_out_bytes=[0] * len(jobs), fallback=None,
               devices=n_dev, device_s=None if stats is None else {},
               device_s_per_device=None if stats is None else [{} for _ in range(n_dev)])
     tmps, files = [], []
@@ -449,7 +668,7 @@ def recruit_file_units(jobs, read_fn, chunk_bytes=CHUNK_BYTES, engine=None, stat
         try:
             try:
                 _stream([(unit, threshold) for unit, _, threshold in jobs], read_fn, files, chunk_bytes, engines, st,
-                        long_units)
+                        long_units, inflate_device)
             finally:
                 for f in files:
                     f.close()
@@ -539,30 +758,37 @@ class _Worker:
         buf = _grown(self.dev, key, nbytes, lambda n: t.empty(n, dtype=t.uint8, device=self.eng.device))
         return buf.view(dtype or t.uint8)
 
-    def step(self, raw, rec, piece, text_bytes, r0, r1):
+    def step(self, raw, rec, piece, text_bytes, bam, r0, r1):
         """The device work of records r0 .. r1 - 1 of a chunk as _scan_chunks yields it: their bytes of raw and their
-        rows of rec and piece, rebased on the host, go to the device, which gathers their sequences, filters them for
-        every unit and emits every job's output; the outputs come home into this worker's output buffers.  Returns
-        the parts for the writer, [(copy-done event, job, host buffer, bytes, free queue, key)], in job order."""
+        rows of rec and piece (bam: the bam_seq rows), rebased on the host, go to the device, which gathers their
+        sequences, filters them for every unit and emits every job's output; the outputs come home into this worker's
+        output buffers.  Returns the parts for the writer, [(copy-done event, job, host buffer, bytes, free queue, key)],
+        in job order."""
         if r0 == r1:
             return []
         torch, run, p = self.torch, self.run, self.eng._p
         t0 = time.perf_counter()
         # the range's text is rec[r0, 3] .. the next record's (16-byte aligned, like every record's), its pieces are
-        # the ones placed there, and its raw bytes run from its first name to its last name or piece
+        # the ones placed there, and its raw bytes run from its first name to its last name or piece (BAM: to its
+        # last SEQ, which follows the name)
         t_lo = int(rec[r0, 3])
         t_hi = int(rec[r1, 3]) if r1 < rec.shape[0] else text_bytes
-        p0, p1 = (int(x) for x in np.searchsorted(piece[:, 2], (t_lo, t_hi)))
         lo, hi = int(rec[r0, 0]), int(rec[r1 - 1, 0] + rec[r1 - 1, 1])
-        if p1 > p0:
-            hi = max(hi, int(piece[p1 - 1, 0] + piece[p1 - 1, 1]))
-        R, P, n, text_bytes = r1 - r0, p1 - p0, hi - lo, t_hi - t_lo
+        if bam:
+            table, shift = piece[r0:r1], [lo, 0]
+            hi = max(hi, int(piece[r1 - 1, 0] + (rec[r1 - 1, 2] + 1) // 2))
+        else:
+            p0, p1 = (int(x) for x in np.searchsorted(piece[:, 2], (t_lo, t_hi)))
+            table, shift = piece[p0:p1], [lo, 0, t_lo]
+            if p1 > p0:
+                hi = max(hi, int(piece[p1 - 1, 0] + piece[p1 - 1, 1]))
+        R, P, n, text_bytes = r1 - r0, table.shape[0], hi - lo, t_hi - t_lo
         h_rec = self._hbuf("rec", 32 * R)
         rec = np.subtract(rec[r0:r1], np.array([lo, 0, 0, t_lo], dtype=np.int64),
                           out=h_rec.numpy()[:32 * R].view(np.int64).reshape(R, 4))
-        h_piece = self._hbuf("piece", 24 * P)
-        np.subtract(piece[p0:p1], np.array([lo, 0, t_lo], dtype=np.int64),
-                    out=h_piece.numpy()[:24 * P].view(np.int64).reshape(P, 3))
+        pb = table.nbytes
+        h_piece = self._hbuf("piece", pb)
+        np.subtract(table, np.array(shift, dtype=np.int64), out=h_piece.numpy()[:pb].view(np.int64).reshape(table.shape))
         seq_len = rec[:, 2]
         upper = int((rec[:, 1] + seq_len).sum()) + 3 * R
         # segments as recruit() plans them (with run.overlap); when no job has threshold >= 0 no filter runs.
@@ -587,16 +813,19 @@ class _Worker:
         d_raw[:n].copy_(raw[lo:hi], non_blocking=True)
         d_rec = self._dbuf("rec", 32 * R)
         d_rec[:32 * R].copy_(h_rec[:32 * R], non_blocking=True)
-        d_piece = self._dbuf("piece", 24 * P + 8)
+        d_piece = self._dbuf("piece", pb + 8)
         if P:
-            d_piece[:24 * P].copy_(h_piece[:24 * P], non_blocking=True)
+            d_piece[:pb].copy_(h_piece[:pb], non_blocking=True)
         if S:
             d_seg = self._dbuf("seg", nb)
             d_seg[:nb].copy_(hs[:nb], non_blocking=True)
         b = self._mark()
         stream = self.eng._stream()
         d_text = self._dbuf("text", text_bytes + 16)
-        _lib.call("cfk_rr_gather", p(d_raw), p(d_piece), P, p(d_text), text_bytes, stream)
+        if bam:
+            _lib.call("cfk_rr_bam_gather", p(d_raw), p(d_piece), p(d_rec), R, p(d_text), text_bytes, stream)
+        else:
+            _lib.call("cfk_rr_gather", p(d_raw), p(d_piece), P, p(d_text), text_bytes, stream)
         c = self._mark()
         d_keep = seg_ptr = None
         if S:
@@ -630,7 +859,15 @@ class _Worker:
             d_outs.append(d_out)
         if run.timed:
             self.events.extend((("h2d", a, b), ("gather", b, c), ("filter", c, d), ("emit", d, self._mark())))
-        totals = d_totals[:len(run.jobs)].tolist()  # the range's one size read-back
+        # the range's one size read-back: into pinned memory and an event wait, not a synchronous copy to pageable
+        # memory, which blocks the CUDA calls of other threads (the BGZF reader's) until the filter has finished
+        J = len(run.jobs)
+        h_totals = self._hbuf("totals", 8 * J)
+        h_totals[:8 * J].copy_(d_totals.view(torch.uint8)[:8 * J], non_blocking=True)
+        sized = torch.cuda.Event()
+        sized.record()
+        sized.synchronize()
+        totals = h_totals.numpy()[:8 * J].view(np.int64).tolist()
         parts = []
         for j, (total, d_out) in enumerate(zip(totals, d_outs)):
             key = self.free_out[j].get()
@@ -648,7 +885,7 @@ class _Worker:
         return parts
 
 
-def _stream(jobs, read_fn, files, chunk_bytes, engines, st, long_units=False):
+def _stream(jobs, read_fn, files, chunk_bytes, engines, st, long_units=False, inflate_device=None):
     """recruit_file_units' pipeline: jobs = [(unit, threshold)], files[j] receives job j's output, engines() -> one
     engine per worker (called once the first record is seen).  While the workers' devices work on chunk i, the reader
     thread reads ahead, this thread scans chunk i + 1 and deals its records out, and the writer thread writes chunk
@@ -719,10 +956,10 @@ def _stream(jobs, read_fn, files, chunk_bytes, engines, st, long_units=False):
                 st["job_out_bytes"][j] += nbytes
                 writer_q.put(part)
 
-    chunks = _scan_chunks(read_fn, chunk_bytes, host, st)
+    chunks = _scan_chunks(read_fn, chunk_bytes, host, st, inflate_device)
     in_flight = False
     try:
-        for slot, raw, rec, piece, text_bytes in chunks:  # scanning chunk i + 1 overlaps the devices' work on chunk i
+        for slot, raw, rec, piece, text_bytes, bam in chunks:  # scanning chunk i + 1 overlaps the devices' work on chunk i
             first = not workers
             if first:
                 start()
@@ -734,7 +971,7 @@ def _stream(jobs, read_fn, files, chunk_bytes, engines, st, long_units=False):
             st["bases"] += int(seq_len.sum())
             bounds = _split_records(seq_len, len(workers)).tolist()
             for w, r0, r1 in zip(workers, bounds[:-1], bounds[1:]):
-                w.inbox.put((raw, rec, piece, text_bytes, r0, r1))
+                w.inbox.put((raw, rec, piece, text_bytes, bam, r0, r1))
             st["chunks"] += 1
             st["plan_s"] += time.perf_counter() - t0
             if in_flight:
@@ -772,7 +1009,8 @@ def _stream(jobs, read_fn, files, chunk_bytes, engines, st, long_units=False):
 def main(argv=None):
     argv = sys.argv[1:] if argv is None else list(argv)
     if len(argv) != 4 or argv[0] == "-h":
-        print("Usage: ./rr unit.fasta reads.fasta.gz output.fasta edit_distance_threshold", end="")
+        print("Usage: ./rr unit.fasta reads.fasta.gz output.fasta edit_distance_threshold", end="")  # rr.cpp's text
+        print(RR_READS_NOTE, file=sys.stderr)
         return 0
     unit_fn, read_fn, output_fn = argv[:3]
     try:
@@ -784,13 +1022,14 @@ def main(argv=None):
     return 0
 
 
-UNITS_USAGE = ("Usage: rr_multi.py reads.fasta[.gz|.fastq] unit1.fasta output1.fasta threshold1 [unit2.fasta output2.fasta threshold2 ...]\n"
+RR_READS_NOTE = "\nreads: FASTA or FASTQ, plain, gzip or bgzip, or unaligned BAM (told apart by their bytes)"
+UNITS_USAGE = ("Usage: rr_multi.py reads.{fasta,fastq}[.gz]|reads.bam unit1.fasta output1.fasta threshold1 [unit2.fasta output2.fasta threshold2 ...]\n"
                "       --gpus N (first): deal every chunk's records over cuda:0..N-1")
 
 
 def main_units(argv=None):
     """``rr_multi.py [--gpus N] reads unit1 output1 threshold1 [unit2 output2 threshold2 ...]``: what one rr run per
-    triple writes, from one pass over the read file (recruit_file_units).  Each unit is the first record of its file,
+    triple writes, from one pass over the read file (recruit_file_units; FASTA / FASTQ, plain, gzip or bgzip, or BAM).  Each unit is the first record of its file,
     of 1..32768 bases;
     thresholds are read as main() reads them.  --gpus N runs on cuda:0 .. N-1 (devices=); without it, on one device.
     A wrong argument count, or an N that is not an integer from 1 to the number of visible devices: the usage on

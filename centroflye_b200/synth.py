@@ -232,3 +232,76 @@ def make_dataset(unit, multiplicity, div_rate, genome_seed, coverage, error_rate
                  flank_len=200000, **read_kw):
     genome, a0, alen = simulate_genome(unit, multiplicity, div_rate, genome_seed, flank_len=flank_len)
     return simulate_reads(genome, a0, alen, unit, coverage, error_rate, read_seed, **read_kw)
+
+
+# ---- compressed read files: BGZF (SAM spec §4.1) and unaligned BAM (§4.2) ---------------------------------------------
+
+BGZF_BLOCK = 65280  # input bytes per block, as bgzip and htslib write them
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+BAM_CODES = "=ACMGRSVTWYHKDBN"
+
+
+def bgzf_member(data, level=6, strategy=None, flush_at=()):
+    """One BGZF block holding `data` (at most 65536 bytes): zlib raw deflate at `level` / `strategy`, with a Z_FULL_FLUSH
+    after each offset of flush_at (several DEFLATE blocks in one member), a gzip header with the BC subfield, CRC32 and
+    ISIZE."""
+    import struct
+    import zlib
+    c = zlib.compressobj(level, zlib.DEFLATED, -15, 9, zlib.Z_DEFAULT_STRATEGY if strategy is None else strategy)
+    parts, at = [], 0
+    for cut in list(flush_at) + [len(data)]:
+        parts.append(c.compress(bytes(data[at:cut])))
+        if cut < len(data):
+            parts.append(c.flush(zlib.Z_FULL_FLUSH))
+        at = cut
+    parts.append(c.flush())
+    payload = b"".join(parts)
+    bsize = 18 + len(payload) + 8 - 1
+    if bsize > 0xffff:
+        raise ValueError("bgzf_member: the block does not compress into 64 KiB")
+    head = b"\x1f\x8b\x08\x04\x00\x00\x00\x00\x00\xff\x06\x00BC\x02\x00" + struct.pack("<H", bsize)
+    return head + payload + struct.pack("<II", zlib.crc32(data) & 0xffffffff, len(data))
+
+
+def bgzf_compress(data, level=6, strategy=None, block=BGZF_BLOCK, eof=True):
+    """`data` as BGZF: one member per `block` bytes, then the 28-byte end-of-file block."""
+    data = memoryview(bytes(data))
+    out = [bgzf_member(data[i:i + block], level, strategy) for i in range(0, len(data), block)]
+    return b"".join(out) + (BGZF_EOF if eof else b"")
+
+
+def write_bgzf(path, data, **kw):
+    with open(path, "wb") as f:
+        f.write(bgzf_compress(data, **kw))
+
+
+def bam_record(name, seq, flag=0, cigar=(), qual=None, tags=b"", ref_id=-1, pos=-1):
+    """One BAM alignment record (block_size included).  seq is text over BAM_CODES (other bytes are written as N); it is
+    stored as given, reverse-complemented or not; cigar = [(length, op index 0..8)]; qual None writes 0xff bytes."""
+    import struct
+    name_b = name.encode() + b"\0"
+    l_seq = len(seq)
+    lut = np.full(256, 15, dtype=np.uint8)
+    lut[np.frombuffer(BAM_CODES.encode(), dtype=np.uint8)] = np.arange(16, dtype=np.uint8)
+    nib = np.append(lut[np.frombuffer(seq.encode("latin-1"), dtype=np.uint8)], np.uint8(0))
+    packed = ((nib[0:l_seq:2] << 4) | nib[1:l_seq + 1:2][:(l_seq + 1) // 2]).tobytes()
+    q = b"\xff" * l_seq if qual is None else bytes(qual)
+    body = struct.pack("<iiBBHHHiiii", ref_id, pos, len(name_b), 255, 4680, len(cigar), flag, l_seq, -1, -1, 0)
+    body += name_b + b"".join(struct.pack("<I", (n << 4) | op) for n, op in cigar) + packed + q + bytes(tags)
+    return struct.pack("<i", len(body)) + body
+
+
+def bam_bytes(records, refs=(("chr1", 248956422),), text="@HD\tVN:1.6\tSO:unknown\n"):
+    """The inflated stream of a BAM file: magic, header text, references, then the records (bam_record keyword
+    dicts, or already encoded bytes)."""
+    import struct
+    out = [b"BAM\1", struct.pack("<i", len(text)), text.encode(), struct.pack("<i", len(refs))]
+    for name, length in refs:
+        out += [struct.pack("<i", len(name) + 1), name.encode() + b"\0", struct.pack("<i", length)]
+    out += [r if isinstance(r, (bytes, bytearray)) else bam_record(**r) for r in records]
+    return b"".join(out)
+
+
+def write_bam(path, records, level=6, **kw):
+    """A BAM file (bam_bytes, BGZF-compressed)."""
+    write_bgzf(path, bam_bytes(records, **kw), level=level)

@@ -265,6 +265,49 @@ int cfk_rr_keep_sizes(const uint8_t* seg_keep, const int64_t* seg_ptr, const int
 int cfk_rr_emit(const uint8_t* raw, const uint8_t* text, const int64_t* records, const int64_t* out_off, int64_t n_records,
                 int64_t max_bytes, uint8_t* out, cfk_stream_t stream);
 
+/* ---- compressed read files: BGZF blocks inflated on the device, unaligned BAM ----------------------------------
+ * cfk_bgzf_blocks (HOST code) walks the gzip members (RFC 1952 headers: FLG, the XLEN subfields searched for "BC",
+ * FNAME, FCOMMENT, FHCRC) of buf_h[0..len) and writes one row per complete BGZF block:
+ *   blocks_h [n][5]    payload offset in buf_h, payload length (the raw DEFLATE data), ISIZE, CRC32, output offset
+ *                      (the exclusive scan of ISIZE from 0);
+ *   out_h    [4]       n_blocks, consumed, inflated bytes of the rows, flags.
+ * Zero bytes between and after members are skipped.  The walk stops after max_blocks rows; before a member that ends
+ * past len (CFK_BGZF_INCOMPLETE); and before one that is not BGZF -- no "BC" subfield, an ISIZE above 65536, a header
+ * that does not fit BSIZE, or bytes that are no gzip member at all (CFK_BGZF_NOT_BGZF).  `consumed` is where it
+ * stopped.
+ *
+ * cfk_bgzf_inflate inflates the rows (offsets into comp, on the device) into out[row[4] ..] and writes status[i]:
+ * CFK_BGZF_OK, CFK_BGZF_BAD_STREAM (not a DEFLATE stream that ends with the payload, or a back-reference before the
+ * block's start), CFK_BGZF_BAD_LENGTH (the stream yields more or fewer than ISIZE bytes) or CFK_BGZF_BAD_CRC.  All of
+ * RFC 1951; every member starts with an empty window.  ISIZE must be at most 65536.
+ *
+ * cfk_bam_scan (HOST code) finds the records of one chunk of inflated BAM (SAM spec §4.2).  With `header` the chunk
+ * starts at the stream's beginning and the header (magic, text, references) is skipped first; if it is not complete
+ * nothing is consumed.  Secondary and supplementary alignments (flag & 0x900) are consumed and yield nothing.  It
+ * writes, for every other complete record,
+ *   records_h [n][4]   as cfk_seq_scan's: name offset in buf_h, name length, l_seq, 16-byte aligned text offset;
+ *   bam_seq_h [n][2]   offset in buf_h of the 4-bit SEQ, 1 if the record is reverse-complemented (flag & 0x10);
+ *   out_h     [5]      n_records, records consumed (every alignment), consumed, text_bytes, flags (CFK_SCAN_FULL).
+ * Every record is validated (block_size, l_read_name, l_seq, fields within block_size, a NUL-terminated name of
+ * '!'..'~'); an invalid record, or at_eof with a record or header cut off, fails naming the record's index
+ * (first_index + records before it) and its offset in the inflated stream (stream_offset + offset in buf_h).
+ *
+ * cfk_rr_bam_gather writes the text cfk_rr_gather writes for FASTA / FASTQ: record r's SEQ decoded through
+ * "=ACMGRSVTWYHKDBN" (reversed and complemented where flagged) at records[r][3], 0 elsewhere. */
+#define CFK_BGZF_INCOMPLETE 1
+#define CFK_BGZF_NOT_BGZF 2
+#define CFK_BGZF_OK 0
+#define CFK_BGZF_BAD_STREAM 1
+#define CFK_BGZF_BAD_LENGTH 2
+#define CFK_BGZF_BAD_CRC 3
+int cfk_bgzf_blocks(const uint8_t* buf_h, int64_t len, int64_t* blocks_h, int64_t max_blocks, int64_t* out_h);
+int cfk_bgzf_inflate(const uint8_t* comp, const int64_t* blocks, int64_t n_blocks, uint8_t* out, int32_t* status,
+                     cfk_stream_t stream);
+int cfk_bam_scan(const uint8_t* buf_h, int64_t len, int32_t at_eof, int32_t header, int64_t first_index,
+                 int64_t stream_offset, int64_t* records_h, int64_t max_records, int64_t* bam_seq_h, int64_t* out_h);
+int cfk_rr_bam_gather(const uint8_t* raw, const int64_t* bam_seq, const int64_t* records, int64_t n_records, uint8_t* text,
+                      int64_t text_bytes, cfk_stream_t stream);
+
 /* ---- read_placer scoring on the cloud CSR (SURVEY.md §8f rank 2) --------------------------------
  * Replaces the data structures of ReadPlacer.add_reads, scripts/read_placer.py:42-94, and of CloudContig.add_read /
  * update_mapping_scores, scripts/cloud_contig.py:26-41,87-95; the greedy loop (one read per iteration) stays on the
